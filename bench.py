@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the batched satellite environment step on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): RK4 satellite env-steps/sec on synthetic random orbits and actions. A "step" is
 one pass of the hot path over one batch: one fused env step in rk4 mode (clip/gate/impulse, S RK4+J2
@@ -17,6 +17,10 @@ per-GPU batch on every rank (weak scaling; envs are independent, no data-path co
 2048-step horizon.
 
 One JSON line on stdout (rank 0). See DESIGN.md "Measurement" for every field.
+
+--dump-outputs DIR writes what rank 0's last timed step returned to its caller: obs.npy (next observations, fp32,
+[envs, 18]), reward.npy (fp64), done.npy (0 / 1 as fp32) and ret_std.npy (std of the discounted returns, fp64). The
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -78,7 +82,11 @@ def parse():
     ap.add_argument("--config4", action="store_true", help="also run BASELINE config 4 at N=1 (1 048 576 envs on one GPU); "
                                                            "always run for N>1 (1 048 576 / N envs per GPU, T=256)")
     ap.add_argument("--no-config4", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (rank 0) as DIR/<name>.npy; "
+                                                           "bench_outputs/ in the tree is git-ignored")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup_requested = args.warmup
     if args.gpus >= 8 and "--ppo-horizon" not in " ".join(sys.argv):
         args.ppo_horizon = 2048                  # config 5 proper: 2048-step x 65 536-env rollout on 8 GPUs (8192 envs/GPU)
@@ -420,6 +428,32 @@ def run_config4(args, rank, world, dev, torch, dist, eng):
     return out
 
 
+DUMP_MAX_BYTES = 64_000_000
+
+
+def _float_array(t):
+    a = t.cpu().numpy()
+    return a if a.dtype in (np.float32, np.float64) else a.astype(np.float32)
+
+
+def dump_outputs(path, per_env, extra):
+    """Writes a step's outputs as path/<name>.npy, float64 arrays as they are and everything else as float32, so that two
+    builds can be compared output for output. When the per-env arrays exceed DUMP_MAX_BYTES, every one of them is cut to
+    the same seeded sample of rows and the sampled row indices are written as rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    per_env = {k: _float_array(v) for k, v in per_env.items()}
+    extra = {k: _float_array(v) for k, v in extra.items()}
+    n = len(next(iter(per_env.values())))
+    row_bytes = sum(a.nbytes // n for a in per_env.values())
+    if row_bytes * n > DUMP_MAX_BYTES:
+        keep = (DUMP_MAX_BYTES - 1_000_000) // (row_bytes + 8)      # 8 B per row for rows.npy, 1 MB for the rest
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        per_env = {k: a[rows] for k, a in per_env.items()}
+        extra["rows"] = rows.astype(np.float64)
+    for k, a in {**per_env, **extra}.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def bind_to_gpu_numa_node(local_rank):
     """Multi-GPU runs: pin this rank (and therefore its first-touch pinned host buffers) to the CPUs NVML reports as local
     to its GPU, so the e2e path's PCIe traffic does not cross the socket interconnect. Returns the CPU count or None."""
@@ -515,6 +549,10 @@ def run_ours(args, rank, world, local_rank):
         ev[i][1].record()
     barrier()
     wall = time.perf_counter() - wall0
+    if args.dump_outputs and rank == 0:                             # before the sections below reuse the ring slots
+        k = (args.warmup + args.steps - 1) % RING
+        dump_outputs(args.dump_outputs, {"obs": buf_obs[k], "reward": buf_rew[k], "done": buf_done[k]},
+                     {"ret_std": buf_rstd[k:k + 1]})
     total_ms = sum(a.elapsed_time(b) for a, b in ev)
     t_all = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if world > 1:

@@ -103,7 +103,7 @@ def test_rk4_argument_errors(eng):
 def test_env_cw_bit_identical_to_reference_rollouts(golden, eng, scen):
     """N=1 env driven by the reference's recorded action stream: obs, reward, done, danger-zone count,
     fuel and distance must be IDENTICAL to the reference env (north star: rewards/dones identical)."""
-    g = golden("env_golden.npz")
+    g = {**golden("env_golden.npz"), **golden("env_capt_golden.npz")}
     T = len(g[f"{scen}_reward"])
     env = eng.EnvBatch(1, mode="cw", flag=int(g[f"{scen}_flag"]), d_capture=float(g[f"{scen}_d_capture"]),
                        max_episode_steps=int(g[f"{scen}_max_episode_steps"]), auto_reset=True, stm=g["stm100_columns"])

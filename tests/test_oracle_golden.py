@@ -86,7 +86,7 @@ def test_cw_matrix_matches_reference(golden, oracle):
 
 @pytest.mark.parametrize("scen", ["cfg1", "long", "capt", "flag1"])
 def test_env_rollout_bit_identical(golden, oracle, scen):
-    g = golden("env_golden.npz")
+    g = {**golden("env_golden.npz"), **golden("env_capt_golden.npz")}
     env = oracle.Env(d_capture=float(g[f"{scen}_d_capture"]), max_episode_steps=int(g[f"{scen}_max_episode_steps"]),
                      M=g["stm100_columns"])
     flag = int(g[f"{scen}_flag"])

@@ -300,7 +300,8 @@ enum { SAT_PPO_OFF_W1 = 0, SAT_PPO_OFF_B1 = 4608, SAT_PPO_OFF_W2 = 4864, SAT_PPO
 typedef struct SatPpoNet {
     float* params;      /* flat parameters (SAT_PPO_OFF_*), updated in place by sat_ppo_adam; 16-byte aligned */
     float* packed;      /* SAT_ACTOR_PACKED_FLOATS kernel image of params (what sat_actor_sample reads); rewritten by sat_ppo_adam */
-    float* grads;       /* flat gradient, same layout, SAT_PPO_PARAM_FLOATS + 1 floats: the last one is the minibatch loss */
+    float* grads;       /* flat gradient, same layout, SAT_PPO_PARAM_FLOATS + 1 floats: the last one is the minibatch loss
+                           (SAT_PPO_GRAD_FLOATS_STATS for sat_ppo_actor_grad_stats) */
     float* exp_avg;     /* Adam first moment, flat */
     float* exp_avg_sq;  /* Adam second moment, flat */
     float* workspace;   /* sat_ppo_workspace_floats(mb) floats, may be shared by the two networks of one agent */
@@ -336,6 +337,35 @@ int sat_ppo_adam(const SatPpoNet* net, const float* lr, float beta1, float beta2
 int sat_ppo_adam_peers(const SatPpoNet* net, const float* lr, float beta1, float beta2, float eps, float max_grad_norm,
                        float grad_scale, int64_t* step, const float* const* peer_grads, int world, int64_t offset_floats,
                        void* stream);
+
+/* Training diagnostics of the fused step. sat_ppo_actor_grad_stats computes exactly the gradient and loss of
+ * sat_ppo_actor_grad (bit-identical grads[0 .. n]) and also writes the minibatch means of four per-row terms to the tail
+ * grads[n + 2 .. n + 6), n = SAT_PPO_PARAM_FLOATS(3): -min(surr1, surr2), the entropy, the approximate KL
+ * (ratio - 1) - log ratio, and the fraction of rows with |ratio - 1| > epsilon. net->grads must then hold
+ * SAT_PPO_GRAD_FLOATS_STATS(3) floats. Because the tail sits in the gradient buffer, an all-reduce of those floats (or the
+ * peer read of sat_ppo_adam_peers_stats) carries the diagnostics with the gradient, and every rank sees the same sums.
+ * sat_ppo_adam_stats / sat_ppo_adam_peers_stats do exactly the step of sat_ppo_adam / sat_ppo_adam_peers (bit-identical
+ * parameters and moments) and, before it, ADD one minibatch to the device fp64 record [SAT_PPO_STATS_DOUBLES]: the loss
+ * slot grads[n] and (actor only: heads == 3) the four tail terms, each times grad_scale (the global minibatch means after an
+ * all-reduce), the pre-clip gradient norm, the clip coefficient and a count of 1. The caller zeroes the record; per-epoch
+ * means are sum / count. */
+#define SAT_PPO_GRAD_FLOATS_STATS(heads) (SAT_PPO_PARAM_FLOATS(heads) + 6)
+#define SAT_PPO_STAT_LOSS 0        /* minibatch loss: actor surrogate - entropy_coef * entropy, or the critic's MSE */
+#define SAT_PPO_STAT_SURROGATE 1   /* actor: mean of -min(ratio * adv, clamp(ratio, 1 - eps, 1 + eps) * adv) */
+#define SAT_PPO_STAT_ENTROPY 2     /* actor: mean entropy of the Gaussian policy (summed over the action dimensions) */
+#define SAT_PPO_STAT_APPROX_KL 3   /* actor: mean of (ratio - 1) - log ratio, evaluated as expm1(log ratio) - log ratio */
+#define SAT_PPO_STAT_CLIP_FRAC 4   /* actor: fraction of rows with |ratio - 1| > epsilon */
+#define SAT_PPO_STAT_GRAD_NORM 5   /* global gradient norm before clipping (what clip_grad_norm_ returns) */
+#define SAT_PPO_STAT_CLIP_COEF 6   /* gradient scale applied by the clip: min(max_norm / (norm + 1e-6), 1), 1 without clip */
+#define SAT_PPO_STAT_COUNT 7       /* number of minibatches added */
+#define SAT_PPO_STATS_DOUBLES 8
+int sat_ppo_actor_grad_stats(const SatPpoNet* net, const float* s, const float* a, const float* old_logp, const float* adv,
+                             const int64_t* index, int64_t mb, float epsilon, float entropy_coef, void* stream);
+int sat_ppo_adam_stats(const SatPpoNet* net, const float* lr, float beta1, float beta2, float eps, float max_grad_norm,
+                       float grad_scale, int64_t* step, double* record, void* stream);
+int sat_ppo_adam_peers_stats(const SatPpoNet* net, const float* lr, float beta1, float beta2, float eps, float max_grad_norm,
+                             float grad_scale, int64_t* step, const float* const* peer_grads, int world, int64_t offset_floats,
+                             double* record, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Measurement helpers (bench.py): dependent-free DFMA / FFMA chains to measure the FP64 / FP32

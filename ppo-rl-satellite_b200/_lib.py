@@ -58,6 +58,17 @@ def ppo_param_floats(heads: int) -> int:
     return 70656 + 257 * heads + (3 if heads == 3 else 0)
 
 
+def ppo_grad_floats_stats(heads: int) -> int:
+    """SAT_PPO_GRAD_FLOATS_STATS: flat gradient, loss slot, one spare float and the four-float diagnostics tail"""
+    return ppo_param_floats(heads) + 6
+
+
+# fp64 record of sat_ppo_adam_stats (SAT_PPO_STAT_*): sums over the minibatches added, COUNT of them
+(PPO_STAT_LOSS, PPO_STAT_SURROGATE, PPO_STAT_ENTROPY, PPO_STAT_APPROX_KL, PPO_STAT_CLIP_FRAC, PPO_STAT_GRAD_NORM,
+ PPO_STAT_CLIP_COEF, PPO_STAT_COUNT) = range(8)
+PPO_STATS_DOUBLES = 8
+
+
 _P, _I64, _I32, _D, _F, _U64 = C.c_void_p, C.c_int64, C.c_int, C.c_double, C.c_float, C.c_uint64
 SIGNATURES = {
     "sat_abi_version": (C.c_int, []),
@@ -74,6 +85,9 @@ SIGNATURES = {
     "sat_ppo_critic_grad": (C.c_int, [_P, _P, _P, _P, _I64, _P]),
     "sat_ppo_adam": (C.c_int, [_P, _P, _F, _F, _F, _F, _F, _P, _P]),
     "sat_ppo_adam_peers": (C.c_int, [_P, _P, _F, _F, _F, _F, _F, _P, _P, _I32, _I64, _P]),
+    "sat_ppo_actor_grad_stats": (C.c_int, [_P, _P, _P, _P, _P, _P, _I64, _F, _F, _P]),
+    "sat_ppo_adam_stats": (C.c_int, [_P, _P, _F, _F, _F, _F, _F, _P, _P, _P]),
+    "sat_ppo_adam_peers_stats": (C.c_int, [_P, _P, _F, _F, _F, _F, _F, _P, _P, _I32, _I64, _P, _P]),
     "sat_reachable_domain": (C.c_int, [_P, _P, _I64, _I32, _I32, _D, _P, _P, _P, _P]),
     "sat_orbital_elements": (C.c_int, [_P, _I64, _D, _P, _P, _P]),
     "sat_state_from_elements": (C.c_int, [_P, _I64, _D, _P, _P]),

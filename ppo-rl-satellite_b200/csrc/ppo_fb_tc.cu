@@ -46,7 +46,9 @@ constexpr int OFF_B1P = SM_W3T + HID * 16;       // b1 in layer-1 accumulator co
 constexpr int OFF_BAR = OFF_B1P + HID * 4;
 constexpr int OFF_TMEM = OFF_BAR + 24 * 8;
 constexpr int FB_SMEM = OFF_TMEM + 16 + 1024;
-static_assert(FB_SMEM <= 227 * 1024, "shared memory budget");
+constexpr int OFF_STAT = OFF_TMEM + 16;          // stats instantiation only: per-warp partial sums of the diagnostics [4][4]
+constexpr int FB_SMEM_STATS = FB_SMEM + 4 * 4 * 4;
+static_assert(FB_SMEM_STATS <= 227 * 1024, "shared memory budget");
 
 // image: chunk 0 = W1 (as in actor_tc.cu), chunks 1..8 = W2 forward (n = output unit j, k = input unit), chunks 9..16 = W2
 // backward (n = input unit i, k = output unit j in the permuted order: position kk = 8 p + jj of chunk kc is j = 64 p + 8 kc + jj)
@@ -146,14 +148,17 @@ __device__ __forceinline__ void scale_by_act_grad(const float* __restrict__ gwar
     }
 }
 
-template <bool CRITIC, bool TANH>
+// STATS (actor only): the row threads also reduce the per-row diagnostics (surrogate, entropy, approximate KL, clipped), each
+// scaled by inv_n like the loss, into part_stat [tile][8] (the first four entries)
+template <bool CRITIC, bool TANH, bool STATS>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 ppo_fb_tc_kernel(const float* __restrict__ packed, const unsigned char* __restrict__ image, float max_action,
                  const float* __restrict__ s, const float* __restrict__ a, const float* __restrict__ old_logp,
                  const float* __restrict__ adv, const float* __restrict__ v_target, const int64_t* __restrict__ index,
                  int64_t n, float inv_n, float epsilon, float entropy_coef,
                  float* __restrict__ h1g, float* __restrict__ dz2b, float* __restrict__ dz1g, float* __restrict__ xs,
-                 float* __restrict__ part_head, float* __restrict__ part_scal, int64_t mp) {
+                 float* __restrict__ part_head, float* __restrict__ part_scal, int64_t mp, float* __restrict__ part_stat) {
+    static_assert(!(STATS && CRITIC), "the critic has no per-row diagnostics beyond its loss");
     extern __shared__ unsigned char smem_dyn[];
     unsigned char* sm = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
     float* stg = reinterpret_cast<float*>(sm + OFF_STG);
@@ -376,6 +381,7 @@ ppo_fb_tc_kernel(const float* __restrict__ packed, const unsigned char* __restri
                     pre[k] = ((q[(0 * TM + r) * 4] + q[(1 * TM + r) * 4]) + q[(2 * TM + r) * 4]) + q[(3 * TM + r) * 4];
                 }
                 float d3[3] = {0.0f, 0.0f, 0.0f}, dls[3] = {0.0f, 0.0f, 0.0f}, loss = 0.0f;
+                [[maybe_unused]] float stat[4] = {0.0f, 0.0f, 0.0f, 0.0f};
                 if (live) {
                     if (CRITIC) {
                         const float v = pre[0] + __ldg(packed + OFF_B3);
@@ -410,6 +416,13 @@ ppo_fb_tc_kernel(const float* __restrict__ packed, const unsigned char* __restri
                             d3[k] = gs * diff * iv * max_action * (1.0f - th[k] * th[k]);
                             dls[k] = gs * (diff * diff * iv - 1.0f) - entropy_coef * inv_n;
                         }
+                        if constexpr (STATS) {
+                            // approximate KL (ratio - 1) - log ratio as expm1 - lsum: (expf(lsum) - 1) - lsum cancels in fp32
+                            stat[0] = -fminf(surr1, surr2) * inv_n;
+                            stat[1] = ent * inv_n;
+                            stat[2] = (expm1f(lsum) - lsum) * inv_n;
+                            stat[3] = fabsf(ratio - 1.0f) > epsilon ? inv_n : 0.0f;
+                        }
                     }
                 }
                 dz3s[r] = make_float4(d3[0], d3[1], d3[2], 0.0f);
@@ -422,10 +435,27 @@ ppo_fb_tc_kernel(const float* __restrict__ packed, const unsigned char* __restri
                 if (lane == 0)
 #pragma unroll
                     for (int k = 0; k < 8; ++k) scal[warp * 8 + k] = rs[k];
+                if constexpr (STATS) {
+                    float* statw = reinterpret_cast<float*>(sm + OFF_STAT);
+#pragma unroll
+                    for (int k = 0; k < 4; ++k)
+#pragma unroll
+                        for (int off = 16; off; off >>= 1) stat[k] += __shfl_xor_sync(0xffffffffu, stat[k], off);
+                    if (lane == 0)
+#pragma unroll
+                        for (int k = 0; k < 4; ++k) statw[warp * 4 + k] = stat[k];
+                }
             }
             asm volatile("bar.sync 1, %0;" ::"n"(TC_COMPUTE) : "memory");
             FB_TRACE(t * 16 + 6);
             if (tid < 8) part_scal[(int64_t)tile * 8 + tid] = ((scal[tid] + scal[8 + tid]) + scal[16 + tid]) + scal[24 + tid];
+            if constexpr (STATS) {
+                const float* statw = reinterpret_cast<const float*>(sm + OFF_STAT);
+                if (tid >= 8 && tid < 12) {
+                    const int k = tid - 8;
+                    part_stat[(int64_t)tile * 8 + k] = ((statw[k] + statw[4 + k]) + statw[8 + k]) + statw[12 + k];
+                }
+            }
             // ---------------- dz2 = (dz3 W3) act'(h2): eight operand chunks of the backward product (K order permuted), the
             // per-tile column sums of dW3 = dz3^T h2 and db2 = sum dz2, dz2 to HBM
             {
@@ -497,8 +527,8 @@ ppo_fb_tc_kernel(const float* __restrict__ packed, const unsigned char* __restri
 }
 
 template <typename K>
-int set_smem(K kernel) {
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FB_SMEM);
+int set_smem(K kernel, int bytes) {
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
     return e == cudaSuccess ? SAT_OK : (int)e;
 }
 
@@ -511,8 +541,9 @@ extern "C" int sat_debug_fb_tc_trace(unsigned long long* out) { return (int)cuda
 int ppo_fb_tc_launch(bool critic, bool use_tanh, const float* packed, unsigned char* image, float max_action, const float* s,
                      const float* a, const float* old_logp, const float* adv, const float* v_target, const int64_t* index,
                      int64_t n, float inv_n, float epsilon, float entropy_coef, float* h1g, float* dz2b, float* dz1g, float* xs,
-                     float* part_head, float* part_scal, int64_t mp, cudaStream_t stream) {
+                     float* part_head, float* part_scal, int64_t mp, float* part_stat, cudaStream_t stream) {
     if (mp % TM) return SAT_ERR_SIZE;
+    if (part_stat && critic) return SAT_ERR_SIZE;
     static int sm_count[64] = {0};
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
@@ -533,16 +564,18 @@ int ppo_fb_tc_launch(bool critic, bool use_tanh, const float* packed, unsigned c
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;     // overlap the kernel's prologue with the pack kernel
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
-#define SAT_FB_LAUNCH(C, T)                                                                                                    \
+#define SAT_FB_LAUNCH(C, T, S)                                                                                                 \
     do {                                                                                                                       \
-        int rc = set_smem(ppo_fb_tc_kernel<C, T>);                                                                            \
+        cfg.dynamicSmemBytes = S ? FB_SMEM_STATS : FB_SMEM;                                                                    \
+        int rc = set_smem(ppo_fb_tc_kernel<C, T, S>, (int)cfg.dynamicSmemBytes);                                              \
         if (rc) return rc;                                                                                                     \
-        e = cudaLaunchKernelEx(&cfg, ppo_fb_tc_kernel<C, T>, packed, (const unsigned char*)image, max_action, s, a, old_logp, adv, v_target,    \
-                               index, n, inv_n, epsilon, entropy_coef, h1g, dz2b, dz1g, xs, part_head, part_scal, mp);          \
+        e = cudaLaunchKernelEx(&cfg, ppo_fb_tc_kernel<C, T, S>, packed, (const unsigned char*)image, max_action, s, a, old_logp, adv, v_target, \
+                               index, n, inv_n, epsilon, entropy_coef, h1g, dz2b, dz1g, xs, part_head, part_scal, mp, part_stat); \
         if (e != cudaSuccess) return (int)e;                                                                                   \
     } while (0)
-    if (critic) { if (use_tanh) SAT_FB_LAUNCH(true, true); else SAT_FB_LAUNCH(true, false); }
-    else { if (use_tanh) SAT_FB_LAUNCH(false, true); else SAT_FB_LAUNCH(false, false); }
+    if (critic) { if (use_tanh) SAT_FB_LAUNCH(true, true, false); else SAT_FB_LAUNCH(true, false, false); }
+    else if (part_stat) { if (use_tanh) SAT_FB_LAUNCH(false, true, true); else SAT_FB_LAUNCH(false, false, true); }
+    else { if (use_tanh) SAT_FB_LAUNCH(false, true, false); else SAT_FB_LAUNCH(false, false, false); }
 #undef SAT_FB_LAUNCH
     e = cudaGetLastError();
     return e == cudaSuccess ? SAT_OK : (int)e;

@@ -19,6 +19,11 @@
 //   colsum_kernel     deterministic sum of the per-CTA / per-slab partials into the flat gradient.
 //   ppo_adam_kernel   one 8-CTA cluster: gradient norm through distributed shared memory, clip, Adam, and the packed
 //                     (transposed) weight image for the next forward.
+// The *_stats entry points run the STATS instantiations of the forward/backward and Adam kernels: the actor's row threads also
+// reduce the per-row diagnostics (surrogate, entropy, approximate KL, clipped) into part_stat, one more colsum launch writes them
+// to grads[n + 2 .. n + 6) (so the gradient exchange carries them), and the Adam kernel adds the global minibatch means, the
+// gradient norm and the clip coefficient to a caller-owned fp64 record. Gradients and parameters are bit-identical to the
+// default kernels'.
 #include <cooperative_groups.h>
 #include "mlp_tile.cuh"
 #include "ppo_fb_tc.cuh"
@@ -38,7 +43,7 @@ __host__ __device__ inline int off_b3(int heads) { return SAT_PPO_OFF_W3 + heads
 __host__ __device__ inline int param_floats(int heads) { return SAT_PPO_PARAM_FLOATS(heads); }
 
 struct Workspace {
-    float *h1, *dz2b, *dz1, *xs, *part_head, *part_scal, *part_w2, *part_w1, *part_b1;
+    float *h1, *dz2b, *dz1, *xs, *part_head, *part_scal, *part_w2, *part_w1, *part_b1, *part_stat;
     unsigned char* tc_image;         // the tensor-core forward/backward kernel's split, swizzled weight operands
     int64_t mp, tiles;
 };
@@ -46,7 +51,7 @@ constexpr int64_t MP_ALIGN = 128;    // rows are padded to the tensor-core kerne
 __host__ inline int64_t ws_floats(int64_t mb) {
     const int64_t mp = (mb + MP_ALIGN - 1) / MP_ALIGN * MP_ALIGN, tiles = mp / M;
     return mp * HID * 3 + mp * XS_LD + tiles * 4 * HID + tiles * 8 + (int64_t)W2_SLABS * HID * HID +
-           (int64_t)W1_SLABS * (HID * IN + HID) + SAT_PPO_TC_IMAGE_BYTES / 4 + 64;
+           (int64_t)W1_SLABS * (HID * IN + HID) + SAT_PPO_TC_IMAGE_BYTES / 4 + 64 + tiles * 8;
 }
 __host__ inline Workspace ws_carve(float* base, int64_t mb) {
     Workspace w;
@@ -62,6 +67,7 @@ __host__ inline Workspace ws_carve(float* base, int64_t mb) {
     w.part_w1 = p; p += (int64_t)W1_SLABS * HID * IN;
     w.part_b1 = p; p += (int64_t)W1_SLABS * HID;
     w.tc_image = reinterpret_cast<unsigned char*>(p + ((64 - ((p - base) & 63)) & 63));     // 256-byte aligned (base is 16-byte aligned)
+    w.part_stat = base + ws_floats(mb) - w.tiles * 8;                                        // [tiles][8], the last region
     return w;
 }
 
@@ -77,6 +83,9 @@ struct __align__(128) FbSmem {
     uint64_t bar_misc;
 };
 static_assert(NWARPS * 4 * HID * 4 <= NSTAGE * KT * HID * 4, "reduction scratch must fit in the stage region");
+struct __align__(128) FbSmemStats : FbSmem {
+    float stat[2][4];                // per-warp partial sums of the diagnostics (STATS instantiation)
+};
 
 __device__ __forceinline__ float act_grad(float h, int use_tanh) { return use_tanh ? 1.0f - h * h : (h > 0.0f ? 1.0f : 0.0f); }
 __device__ __forceinline__ float& acc_ref(float2 (&acc)[RT][NP], int i, int c, int q) {
@@ -90,14 +99,17 @@ __device__ __forceinline__ void acc_zero(float2 (&acc)[RT][NP]) {
         for (int j = 0; j < NP; ++j) acc[i][j] = make_float2(0.0f, 0.0f);
 }
 
-template <bool CRITIC>
+// STATS (actor only): the row threads also reduce the per-row diagnostics (surrogate, entropy, approximate KL, clipped), each
+// scaled by inv_n like the loss, into part_stat [tile][8] (the first four entries)
+template <bool CRITIC, bool STATS>
 __global__ void __launch_bounds__(THREADS, 2)
 ppo_fb_kernel(const float* __restrict__ packed, const float* __restrict__ w2, int use_tanh, float max_action,
               const float* __restrict__ s, const float* __restrict__ a, const float* __restrict__ old_logp,
               const float* __restrict__ adv, const float* __restrict__ v_target, const int64_t* __restrict__ index,
               int64_t n, float inv_n, float epsilon, float entropy_coef,
               float* __restrict__ h1g, float* __restrict__ dz2b, float* __restrict__ dz1g, float* __restrict__ xs,
-              float* __restrict__ part_head, float* __restrict__ part_scal, int64_t mp) {
+              float* __restrict__ part_head, float* __restrict__ part_scal, int64_t mp, float* __restrict__ part_stat) {
+    static_assert(!(STATS && CRITIC), "the critic has no per-row diagnostics beyond its loss");
     extern __shared__ __align__(128) unsigned char smem_raw[];
     FbSmem& sm = *reinterpret_cast<FbSmem*>(smem_raw);
     const int tid = threadIdx.x, tx = tid % TXN, ty = tid / TXN, warp = tid >> 5;
@@ -225,6 +237,7 @@ ppo_fb_kernel(const float* __restrict__ packed, const float* __restrict__ w2, in
     if (tid < M) {
         const int64_t g = row0 + tid;
         float d3[3] = {0.0f, 0.0f, 0.0f}, dls[3] = {0.0f, 0.0f, 0.0f}, loss = 0.0f;
+        [[maybe_unused]] float stat[4] = {0.0f, 0.0f, 0.0f, 0.0f};
         if (g < n) {
             const int64_t src = index ? index[g] : g;
             if (CRITIC) {
@@ -260,6 +273,13 @@ ppo_fb_kernel(const float* __restrict__ packed, const float* __restrict__ w2, in
                     d3[k] = gs * diff * iv * max_action * (1.0f - th[k] * th[k]);
                     dls[k] = gs * (diff * diff * iv - 1.0f) - entropy_coef * inv_n;
                 }
+                if constexpr (STATS) {
+                    // approximate KL (ratio - 1) - log ratio as expm1 - lsum: (expf(lsum) - 1) - lsum cancels in fp32
+                    stat[0] = -fminf(surr1, surr2) * inv_n;
+                    stat[1] = ent * inv_n;
+                    stat[2] = (expm1f(lsum) - lsum) * inv_n;
+                    stat[3] = fabsf(ratio - 1.0f) > epsilon ? inv_n : 0.0f;
+                }
             }
         }
 #pragma unroll
@@ -273,9 +293,22 @@ ppo_fb_kernel(const float* __restrict__ packed, const float* __restrict__ w2, in
         if ((tid & 31) == 0)
 #pragma unroll
             for (int k = 0; k < 8; ++k) sm.red[warp][k] = red[k];
+        if constexpr (STATS) {
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+#pragma unroll
+                for (int off = 16; off; off >>= 1) stat[k] += __shfl_xor_sync(0xffffffffu, stat[k], off);
+            if ((tid & 31) == 0)
+#pragma unroll
+                for (int k = 0; k < 4; ++k) reinterpret_cast<FbSmemStats*>(smem_raw)->stat[warp][k] = stat[k];
+        }
     }
     __syncthreads();
     if (tid < 8) part_scal[(int64_t)blockIdx.x * 8 + tid] = sm.red[0][tid] + sm.red[1][tid];
+    if constexpr (STATS) {
+        const FbSmemStats& sst = *reinterpret_cast<const FbSmemStats*>(smem_raw);
+        if (tid >= 8 && tid < 12) part_stat[(int64_t)blockIdx.x * 8 + tid - 8] = sst.stat[0][tid - 8] + sst.stat[1][tid - 8];
+    }
 
     // ---------------- dz2 = (dz3 W3) act'(h2) in place; per-CTA partial sums of dW3 (rows 0..heads-1) and db2 (row 3)
     {
@@ -548,11 +581,15 @@ __device__ __forceinline__ int packed_index(int i, int heads) {
     return OFF_LS + (i - b3 - heads);
 }
 
+// STATS: before the update, thread 0 adds the minibatch's global means (loss slot grads[total] and, for the actor, the
+// diagnostics tail grads[total + 2 ..]; summed over the peers in rank order on the peer path, times grad_scale), the pre-clip
+// gradient norm, the clip coefficient and a count of 1 to record[SAT_PPO_STATS_DOUBLES] (fp64)
+template <bool STATS>
 __global__ void __cluster_dims__(ADAM_CTAS, 1, 1) __launch_bounds__(ADAM_THREADS)
 ppo_adam_kernel(float* __restrict__ params, float* __restrict__ packed, const float* __restrict__ grads,
                 float* __restrict__ exp_avg, float* __restrict__ exp_avg_sq, int heads, const float* __restrict__ lr_ptr,
                 float beta1, float beta2, float eps, float max_norm, float grad_scale, int64_t* __restrict__ step_ptr,
-                const float* const* __restrict__ peers, int world, int64_t peer_off) {
+                const float* const* __restrict__ peers, int world, int64_t peer_off, double* __restrict__ record) {
     cg::cluster_group cluster = cg::this_cluster();
     __shared__ float warp_sums[32];
     __shared__ float cta_sum;
@@ -593,6 +630,26 @@ ppo_adam_kernel(float* __restrict__ params, float* __restrict__ packed, const fl
     cluster.sync();                                           // nobody leaves (or bumps the step) while peers still read
     float coef = 1.0f;
     if (max_norm > 0.0f) coef = fminf(max_norm / (sqrtf(sumsq) + 1e-6f), 1.0f);               // clip_grad_norm_ (:229, :238)
+    if constexpr (STATS) {
+        if (gtid == 0) {
+            auto slot = [&](int k) {
+                float v = 0.0f;
+                if (peers) { for (int r = 0; r < world; ++r) v += __ldcg(peers[r] + peer_off + total + k); }
+                else v = grads[total + k];
+                return (double)(v * grad_scale);
+            };
+            record[SAT_PPO_STAT_LOSS] += slot(0);
+            if (heads == 3) {
+                record[SAT_PPO_STAT_SURROGATE] += slot(2);
+                record[SAT_PPO_STAT_ENTROPY] += slot(3);
+                record[SAT_PPO_STAT_APPROX_KL] += slot(4);
+                record[SAT_PPO_STAT_CLIP_FRAC] += slot(5);
+            }
+            record[SAT_PPO_STAT_GRAD_NORM] += (double)sqrtf(sumsq);
+            record[SAT_PPO_STAT_CLIP_COEF] += (double)coef;
+            record[SAT_PPO_STAT_COUNT] += 1.0;
+        }
+    }
     const float lr = *lr_ptr;
     const float bc1 = 1.0f - powf(beta1, (float)step), bc2 = 1.0f - powf(beta2, (float)step);
     const float step_size = lr / bc1, bc2_sqrt = sqrtf(bc2);
@@ -685,6 +742,60 @@ inline bool ppo_tc_enabled() {
     return g_ppo_tc != 0;
 }
 
+// the per-tile diagnostics -> grads[n + 2 .. n + 6), the tail the gradient exchange carries with the gradient
+int sum_stats(const SatPpoNet* net, const Workspace& w, cudaStream_t stream, int64_t head_tiles) {
+    SumPlan plan;
+    plan.g[0] = SumGroup{w.part_stat, 8, (int)head_tiles, 4, param_floats(net->heads) + 2, 0};
+    plan.groups = 1;
+    colsum_kernel<<<1, 1024, 0, stream>>>(plan, net->grads);
+    return launch_status();
+}
+
+template <bool STATS>
+int actor_grad(const SatPpoNet* net, const float* s, const float* a, const float* old_logp, const float* adv,
+               const int64_t* index, int64_t mb, float epsilon, float entropy_coef, cudaStream_t stream) {
+    int rc = check_net(net);
+    if (rc) return rc;
+    if (!s || !a || !old_logp || !adv) return SAT_ERR_NULL;
+    if (net->heads != 3 || mb <= 0) return SAT_ERR_SIZE;
+    rc = set_smem(ppo_fb_kernel<false, STATS>, STATS ? sizeof(FbSmemStats) : sizeof(FbSmem));
+    if (rc) return rc;
+    const Workspace w = ws_carve(net->workspace, mb);
+    float* part_stat = STATS ? w.part_stat : nullptr;
+    if (ppo_tc_enabled()) {
+        rc = ppo_fb_tc_launch(false, net->use_tanh != 0, net->packed, w.tc_image, net->max_action, s, a, old_logp, adv, nullptr, index, mb,
+                              1.0f / (float)mb, epsilon, entropy_coef, w.h1, w.dz2b, w.dz1, w.xs, w.part_head, w.part_scal, w.mp,
+                              part_stat, stream);
+        if (rc) return rc;
+        rc = finish_grads(net, w, stream, w.mp / MP_ALIGN, true);
+        if (rc || !STATS) return rc;
+        return sum_stats(net, w, stream, w.mp / MP_ALIGN);
+    }
+    ppo_fb_kernel<false, STATS><<<(unsigned)w.tiles, THREADS, STATS ? sizeof(FbSmemStats) : sizeof(FbSmem), stream>>>(
+        net->packed, net->params + SAT_PPO_OFF_W2, net->use_tanh, net->max_action, s, a, old_logp, adv, nullptr, index, mb,
+        1.0f / (float)mb, epsilon, entropy_coef, w.h1, w.dz2b, w.dz1, w.xs, w.part_head, w.part_scal, w.mp, part_stat);
+    rc = launch_status();
+    if (rc) return rc;
+    rc = finish_grads(net, w, stream, w.tiles, false);
+    if (rc || !STATS) return rc;
+    return sum_stats(net, w, stream, w.tiles);
+}
+
+template <bool STATS>
+int adam(const SatPpoNet* net, const float* lr, float beta1, float beta2, float eps, float max_grad_norm, float grad_scale,
+         int64_t* step, bool peer_path, const float* const* peer_grads, int world, int64_t offset_floats, double* record,
+         cudaStream_t stream) {
+    int rc = check_net(net);
+    if (rc) return rc;
+    if (!lr || !step || (peer_path && !peer_grads) || (STATS && !record)) return SAT_ERR_NULL;
+    if (peer_path && (world < 1 || world > 64 || offset_floats < 0)) return SAT_ERR_SIZE;
+    ppo_adam_kernel<STATS><<<ADAM_CTAS, ADAM_THREADS, 0, stream>>>(net->params, net->packed, net->grads, net->exp_avg,
+                                                                  net->exp_avg_sq, net->heads, lr, beta1, beta2, eps,
+                                                                  max_grad_norm, grad_scale, step, peer_grads, world,
+                                                                  offset_floats, record);
+    return launch_status();
+}
+
 }  // namespace
 
 extern "C" {
@@ -707,26 +818,12 @@ int sat_ppo_pack(const SatPpoNet* net, void* stream) {
 
 int sat_ppo_actor_grad(const SatPpoNet* net, const float* s, const float* a, const float* old_logp, const float* adv,
                        const int64_t* index, int64_t mb, float epsilon, float entropy_coef, void* stream) {
-    int rc = check_net(net);
-    if (rc) return rc;
-    if (!s || !a || !old_logp || !adv) return SAT_ERR_NULL;
-    if (net->heads != 3 || mb <= 0) return SAT_ERR_SIZE;
-    rc = set_smem(ppo_fb_kernel<false>, sizeof(FbSmem));
-    if (rc) return rc;
-    const Workspace w = ws_carve(net->workspace, mb);
-    if (ppo_tc_enabled()) {
-        rc = ppo_fb_tc_launch(false, net->use_tanh != 0, net->packed, w.tc_image, net->max_action, s, a, old_logp, adv, nullptr, index, mb,
-                              1.0f / (float)mb, epsilon, entropy_coef, w.h1, w.dz2b, w.dz1, w.xs, w.part_head, w.part_scal, w.mp,
-                              (cudaStream_t)stream);
-        if (rc) return rc;
-        return finish_grads(net, w, (cudaStream_t)stream, w.mp / MP_ALIGN, true);
-    }
-    ppo_fb_kernel<false><<<(unsigned)w.tiles, THREADS, sizeof(FbSmem), (cudaStream_t)stream>>>(
-        net->packed, net->params + SAT_PPO_OFF_W2, net->use_tanh, net->max_action, s, a, old_logp, adv, nullptr, index, mb,
-        1.0f / (float)mb, epsilon, entropy_coef, w.h1, w.dz2b, w.dz1, w.xs, w.part_head, w.part_scal, w.mp);
-    rc = launch_status();
-    if (rc) return rc;
-    return finish_grads(net, w, (cudaStream_t)stream, w.tiles, false);
+    return actor_grad<false>(net, s, a, old_logp, adv, index, mb, epsilon, entropy_coef, (cudaStream_t)stream);
+}
+
+int sat_ppo_actor_grad_stats(const SatPpoNet* net, const float* s, const float* a, const float* old_logp, const float* adv,
+                             const int64_t* index, int64_t mb, float epsilon, float entropy_coef, void* stream) {
+    return actor_grad<true>(net, s, a, old_logp, adv, index, mb, epsilon, entropy_coef, (cudaStream_t)stream);
 }
 
 int sat_ppo_critic_grad(const SatPpoNet* net, const float* s, const float* v_target, const int64_t* index, int64_t mb,
@@ -735,19 +832,19 @@ int sat_ppo_critic_grad(const SatPpoNet* net, const float* s, const float* v_tar
     if (rc) return rc;
     if (!s || !v_target) return SAT_ERR_NULL;
     if (net->heads != 1 || mb <= 0) return SAT_ERR_SIZE;
-    rc = set_smem(ppo_fb_kernel<true>, sizeof(FbSmem));
+    rc = set_smem(ppo_fb_kernel<true, false>, sizeof(FbSmem));
     if (rc) return rc;
     const Workspace w = ws_carve(net->workspace, mb);
     if (ppo_tc_enabled()) {
         rc = ppo_fb_tc_launch(true, net->use_tanh != 0, net->packed, w.tc_image, 0.0f, s, nullptr, nullptr, nullptr, v_target, index, mb,
                               1.0f / (float)mb, 0.0f, 0.0f, w.h1, w.dz2b, w.dz1, w.xs, w.part_head, w.part_scal, w.mp,
-                              (cudaStream_t)stream);
+                              nullptr, (cudaStream_t)stream);
         if (rc) return rc;
         return finish_grads(net, w, (cudaStream_t)stream, w.mp / MP_ALIGN, true);
     }
-    ppo_fb_kernel<true><<<(unsigned)w.tiles, THREADS, sizeof(FbSmem), (cudaStream_t)stream>>>(
+    ppo_fb_kernel<true, false><<<(unsigned)w.tiles, THREADS, sizeof(FbSmem), (cudaStream_t)stream>>>(
         net->packed, net->params + SAT_PPO_OFF_W2, net->use_tanh, 0.0f, s, nullptr, nullptr, nullptr, v_target, index, mb,
-        1.0f / (float)mb, 0.0f, 0.0f, w.h1, w.dz2b, w.dz1, w.xs, w.part_head, w.part_scal, w.mp);
+        1.0f / (float)mb, 0.0f, 0.0f, w.h1, w.dz2b, w.dz1, w.xs, w.part_head, w.part_scal, w.mp, nullptr);
     rc = launch_status();
     if (rc) return rc;
     return finish_grads(net, w, (cudaStream_t)stream, w.tiles, false);
@@ -755,27 +852,26 @@ int sat_ppo_critic_grad(const SatPpoNet* net, const float* s, const float* v_tar
 
 int sat_ppo_adam(const SatPpoNet* net, const float* lr, float beta1, float beta2, float eps, float max_grad_norm,
                  float grad_scale, int64_t* step, void* stream) {
-    int rc = check_net(net);
-    if (rc) return rc;
-    if (!lr || !step) return SAT_ERR_NULL;
-    ppo_adam_kernel<<<ADAM_CTAS, ADAM_THREADS, 0, (cudaStream_t)stream>>>(net->params, net->packed, net->grads, net->exp_avg,
-                                                                         net->exp_avg_sq, net->heads, lr, beta1, beta2, eps,
-                                                                         max_grad_norm, grad_scale, step, nullptr, 1, 0);
-    return launch_status();
+    return adam<false>(net, lr, beta1, beta2, eps, max_grad_norm, grad_scale, step, false, nullptr, 1, 0, nullptr, (cudaStream_t)stream);
+}
+
+int sat_ppo_adam_stats(const SatPpoNet* net, const float* lr, float beta1, float beta2, float eps, float max_grad_norm,
+                       float grad_scale, int64_t* step, double* record, void* stream) {
+    return adam<true>(net, lr, beta1, beta2, eps, max_grad_norm, grad_scale, step, false, nullptr, 1, 0, record, (cudaStream_t)stream);
 }
 
 int sat_ppo_adam_peers(const SatPpoNet* net, const float* lr, float beta1, float beta2, float eps, float max_grad_norm,
                        float grad_scale, int64_t* step, const float* const* peer_grads, int world, int64_t offset_floats,
                        void* stream) {
-    int rc = check_net(net);
-    if (rc) return rc;
-    if (!lr || !step || !peer_grads) return SAT_ERR_NULL;
-    if (world < 1 || world > 64 || offset_floats < 0) return SAT_ERR_SIZE;
-    ppo_adam_kernel<<<ADAM_CTAS, ADAM_THREADS, 0, (cudaStream_t)stream>>>(net->params, net->packed, net->grads, net->exp_avg,
-                                                                         net->exp_avg_sq, net->heads, lr, beta1, beta2, eps,
-                                                                         max_grad_norm, grad_scale, step, peer_grads, world,
-                                                                         offset_floats);
-    return launch_status();
+    return adam<false>(net, lr, beta1, beta2, eps, max_grad_norm, grad_scale, step, true, peer_grads, world, offset_floats, nullptr,
+                       (cudaStream_t)stream);
+}
+
+int sat_ppo_adam_peers_stats(const SatPpoNet* net, const float* lr, float beta1, float beta2, float eps, float max_grad_norm,
+                             float grad_scale, int64_t* step, const float* const* peer_grads, int world, int64_t offset_floats,
+                             double* record, void* stream) {
+    return adam<true>(net, lr, beta1, beta2, eps, max_grad_norm, grad_scale, step, true, peer_grads, world, offset_floats, record,
+                      (cudaStream_t)stream);
 }
 
 }  // extern "C"

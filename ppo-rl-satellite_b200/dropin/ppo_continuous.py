@@ -22,6 +22,7 @@ try:
     from ._boot import engine as _eng
 except ImportError:
     from _boot import engine as _eng
+_L = _eng.L
 
 
 def orthogonal_init(layer, gain=1.0):
@@ -103,6 +104,52 @@ def allreduce_grads_(module, group=None):
         off += g.numel()
 
 
+_FROM_ARGS = object()
+
+
+class PpoUpdateStats:
+    """Training diagnostics of one PPO_continuous.optimize call.
+
+    `records` is an fp64 tensor [K][2][PPO_STATS_DOUBLES] (layout _lib.PPO_STAT_*) on the training device: for every epoch and
+    network (0 actor, 1 critic) the sums over that epoch's minibatches of the global minibatch means, with COUNT the number of
+    minibatches. Nothing is read back until as_dict(), except one fp64 per epoch when target_kl is set."""
+
+    def __init__(self, records, minibatches: int, target_kl=None):
+        self.records, self.minibatches, self.target_kl = records, int(minibatches), target_kl
+        self.epochs_run, self.early_stopped = 0, False
+        self.extra = {}                 # further device scalars reported by as_dict(), e.g. explained_variance
+
+    def end_epoch(self, e: int) -> bool:
+        """Called once epoch e is enqueued on the current stream; True when the remaining epochs must not run: the mean over
+        epoch e's minibatches of the global approximate KL is above target_kl (one fp64 read, synchronising the stream)."""
+        self.epochs_run = e + 1
+        if self.target_kl is None or e + 1 >= self.records.shape[0]:
+            return False
+        kl = float(self.records[e, 0, _L.PPO_STAT_APPROX_KL].item()) / self.minibatches
+        self.early_stopped = kl > self.target_kl
+        return self.early_stopped
+
+    def as_dict(self) -> dict:
+        """Means over all minibatches that ran (one device synchronisation)."""
+        names = sorted(self.extra)
+        flat = torch.cat([self.records.reshape(-1)] + [self.extra[k].reshape(1).to(self.records) for k in names]).cpu()
+        rec = flat[:self.records.numel()].view(self.records.shape)[:self.epochs_run]
+        act, cri = rec.sum(0)
+        n = _L.PPO_STAT_COUNT
+
+        def mean(r, k):
+            return float(r[k] / r[n]) if r[n] > 0 else float("nan")
+        out = {"policy_loss": mean(act, _L.PPO_STAT_SURROGATE), "entropy": mean(act, _L.PPO_STAT_ENTROPY),
+               "approx_kl": mean(act, _L.PPO_STAT_APPROX_KL), "clip_fraction": mean(act, _L.PPO_STAT_CLIP_FRAC),
+               "value_loss": mean(cri, _L.PPO_STAT_LOSS), "actor_grad_norm": mean(act, _L.PPO_STAT_GRAD_NORM),
+               "critic_grad_norm": mean(cri, _L.PPO_STAT_GRAD_NORM), "epochs_run": self.epochs_run,
+               "early_stopped": self.early_stopped,
+               "approx_kl_per_epoch": [mean(r[0], _L.PPO_STAT_APPROX_KL) for r in rec]}
+        for i, k in enumerate(names):
+            out[k] = float(flat[self.records.numel() + i])
+        return out
+
+
 class PPO_continuous:
     def __init__(self, args, agent_idx, device="cuda", seed=0, fused_update=True):
         if getattr(args, "policy_dist", "Gaussian") != "Gaussian":
@@ -114,6 +161,8 @@ class PPO_continuous:
         self.gamma, self.lamda, self.epsilon, self.K_epochs = args.gamma, args.lamda, args.epsilon, args.K_epochs
         self.entropy_coef, self.set_adam_eps = args.entropy_coef, args.set_adam_eps
         self.use_grad_clip, self.use_lr_decay, self.use_adv_norm = args.use_grad_clip, args.use_lr_decay, args.use_adv_norm
+        self.target_kl = getattr(args, "target_kl", None)
+        self.last_update_stats = None
         self.actor = Actor_Gaussian(args, agent_idx).to(self.device)
         self.critic = Critic(args, agent_idx).to(self.device)
         eps = dict(eps=1e-5) if self.set_adam_eps else {}
@@ -122,6 +171,7 @@ class PPO_continuous:
         self.optimizer_actor = torch.optim.Adam(self.actor.parameters(), lr=torch.tensor(float(self.lr_a), device=self.device), **eps, **cap)
         self.optimizer_critic = torch.optim.Adam(self.critic.parameters(), lr=torch.tensor(float(self.lr_c), device=self.device), **eps, **cap)
         self._graph = None
+        self._stats_acc = None
         self._fused = None
         self.fused_update = bool(fused_update)        # update(): fused CUDA minibatch step instead of autograd + torch Adam
         self._use_tanh = bool(args.use_tanh)
@@ -208,9 +258,11 @@ class PPO_continuous:
             raise ValueError(f"PPO update with unequal per-rank batches (min {-int(t[1])}, max {int(t[0])} samples): shard the envs "
                              f"evenly (n_total % world == 0) or trim the rollout to a common size")
 
-    def _optimize_fused(self, s, a, a_logprob, adv, v_target, mb, group):
+    def _optimize_fused(self, s, a, a_logprob, adv, v_target, mb, group, out=None):
         """The actor chain and the critic chain are independent (ppo_continuous.py:216-239 shares only s[index]), so each
-        runs on its own stream: one network's short kernels (partial sums, Adam) hide under the other's GEMM kernels."""
+        runs on its own stream: one network's short kernels (partial sums, Adam) hide under the other's GEMM kernels.
+        out (PpoUpdateStats): the stats variants of the kernels add every minibatch to out.records; the diagnostics ride in the
+        gradient buffer's tail, so the same exchange makes them global."""
         dist = torch.distributed
         if group is False:                            # explicit "no gradient exchange" (single-rank use inside a job)
             world, group = 1, None
@@ -228,23 +280,29 @@ class PPO_continuous:
         clip = 0.5 if self.use_grad_clip else 0.0
         main = torch.cuda.current_stream(self.device)
         sa, sc = f["streams"]
-        for _ in range(self.K_epochs):
+        stats = out is not None
+        for e in range(self.K_epochs):
             perm = torch.randperm(B, device=s.device)
             sa.wait_stream(main); sc.wait_stream(main)
             perm.record_stream(sa); perm.record_stream(sc)
+            rec_a, rec_c = (out.records[e, 0], out.records[e, 1]) if stats else (None, None)
             for lo in range(0, B, mb):
                 m = min(mb, B - lo)
                 index = perm.data_ptr() + 8 * lo
                 with torch.cuda.stream(sa):
-                    na.actor_grad(s, a, a_logprob, adv, index, m, self.epsilon, self.entropy_coef)
+                    na.actor_grad(s, a, a_logprob, adv, index, m, self.epsilon, self.entropy_coef, stats=stats)
                     if world > 1 and not peers:
-                        dist.all_reduce(na.grads, group=group)
-                    na.adam(clip, 1.0 / world)
+                        dist.all_reduce(na.grads_stats if stats else na.grads, group=group)
+                    na.adam(clip, 1.0 / world, record=rec_a)
                 with torch.cuda.stream(sc):
                     nc.critic_grad(s, v_target, index, m)
                     if world > 1 and not peers:
                         dist.all_reduce(nc.grads, group=group)
-                    nc.adam(clip, 1.0 / world)
+                    nc.adam(clip, 1.0 / world, record=rec_c)
+            if stats:
+                with torch.cuda.stream(sa):
+                    if out.end_epoch(e):
+                        break
         main.wait_stream(sa); main.wait_stream(sc)
         self._dirty = False                           # the Adam kernel rewrites the packed weight images itself
 
@@ -278,12 +336,13 @@ class PPO_continuous:
             adv, v_target = adv.view(-1, 1), v_target.view(-1, 1)
             if self.use_adv_norm:
                 _eng.adv_normalize_(adv, group=False)
-        self.optimize(s, a, a_logprob, adv, v_target, fused=self.fused_update)
+        self.last_update_stats = self.optimize(s, a, a_logprob, adv, v_target, fused=self.fused_update)
         if self.use_lr_decay:
             self.lr_decay(total_steps)
 
-    def _minibatch_step(self, s, a, a_logprob, adv, v_target, group):
-        """one clipped-PPO actor step + one critic step on a minibatch (ppo_continuous.py:216-239)"""
+    def _minibatch_step(self, s, a, a_logprob, adv, v_target, group, acc=None):
+        """one clipped-PPO actor step + one critic step on a minibatch (ppo_continuous.py:216-239); acc: fp64 [2][8] device
+        accumulator the minibatch's statistics are added to (PpoUpdateStats layout)"""
         dist_now = self.actor.get_dist(s)
         dist_entropy = dist_now.entropy().sum(1, keepdim=True)
         a_logprob_now = dist_now.log_prob(a)
@@ -294,8 +353,11 @@ class PPO_continuous:
         self.optimizer_actor.zero_grad(set_to_none=False)
         actor_loss.mean().backward()
         allreduce_grads_(self.actor, group)
+        norms = []
         if self.use_grad_clip:
-            torch.nn.utils.clip_grad_norm_(self.actor.parameters(), 0.5)
+            norms.append(torch.nn.utils.clip_grad_norm_(self.actor.parameters(), 0.5))
+        elif acc is not None:
+            norms.append(torch.nn.utils.get_total_norm([p.grad for p in self.actor.parameters()]))
         self.optimizer_actor.step()
         v_s = self.critic(s)
         critic_loss = F.mse_loss(v_target, v_s)
@@ -303,18 +365,29 @@ class PPO_continuous:
         critic_loss.backward()
         allreduce_grads_(self.critic, group)
         if self.use_grad_clip:
-            torch.nn.utils.clip_grad_norm_(self.critic.parameters(), 0.5)
+            norms.append(torch.nn.utils.clip_grad_norm_(self.critic.parameters(), 0.5))
+        elif acc is not None:
+            norms.append(torch.nn.utils.get_total_norm([p.grad for p in self.critic.parameters()]))
         self.optimizer_critic.step()
+        if acc is not None:
+            with torch.no_grad():
+                log_ratio = a_logprob_now.sum(1, keepdim=True) - a_logprob.sum(1, keepdim=True)
+                one, zero = critic_loss.new_ones(()), critic_loss.new_zeros(())
+                coef = [torch.clamp(0.5 / (nm + 1e-6), max=1.0) if self.use_grad_clip else one for nm in norms]
+                acc[0] += torch.stack([actor_loss.mean(), (-torch.min(surr1, surr2)).mean(), dist_entropy.mean(),
+                                       (torch.expm1(log_ratio) - log_ratio).mean(),
+                                       ((ratios - 1.0).abs() > self.epsilon).float().mean(), norms[0], coef[0], one]).double()
+                acc[1] += torch.stack([critic_loss, zero, zero, zero, zero, norms[1], coef[1], one]).double()
 
-    def _graph_for(self, tensors, mb, group):
+    def _graph_for(self, tensors, mb, group, acc=None):
         """CUDA graph of (gather minibatch by a static index buffer -> _minibatch_step), keyed by the buffer addresses"""
-        key = (tuple(t.data_ptr() for t in tensors), tuple(t.shape for t in tensors), mb)
+        key = (tuple(t.data_ptr() for t in tensors), tuple(t.shape for t in tensors), mb, acc is not None)
         if self._graph is not None and self._graph["key"] == key:
             return self._graph
         idx = torch.zeros(mb, dtype=torch.long, device=self.device)
 
         def body():
-            self._minibatch_step(*(t.index_select(0, idx) for t in tensors), group)
+            self._minibatch_step(*(t.index_select(0, idx) for t in tensors), group, acc)
         # warm-up on a side stream (allocator, cuBLAS handles, lazily created Adam state), then capture; weights and
         # optimiser state are restored IN PLACE afterwards so the captured addresses stay valid
         params = list(self.actor.parameters()) + list(self.critic.parameters())
@@ -342,30 +415,53 @@ class PPO_continuous:
                                 v.copy_(snap[p][k])
                             else:
                                 v.zero_()             # state created during the warm-up: back to a fresh optimiser
+            if acc is not None:
+                acc.zero_()
         self._graph = {"key": key, "graph": g, "idx": idx}
         return self._graph
 
-    def optimize(self, s, a, a_logprob, adv, v_target, mini_batch_size=None, group=None, use_graph=False, fused=False):
+    def optimize(self, s, a, a_logprob, adv, v_target, mini_batch_size=None, group=None, use_graph=False, fused=False,
+                 stats=False, target_kl=_FROM_ARGS):
         """K epochs of clipped-PPO minibatch steps (ppo_continuous.py:213-239) on device tensors.
         fused: the hand-written forward/backward/Adam kernels (own Adam moments, independent of the torch optimisers);
-        use_graph: replay one captured CUDA graph of the PyTorch step per minibatch (static buffers, full minibatches only)."""
+        use_graph: replay one captured CUDA graph of the PyTorch step per minibatch (static buffers, full minibatches only).
+        stats: return a PpoUpdateStats (policy / value loss, entropy, approximate KL, clip fraction, gradient norms) with the
+        same keys on every path; otherwise None, unless target_kl is set.
+        target_kl (default: args.target_kl, else None): early stop at epoch granularity. After each epoch the mean over its
+        minibatches of the global approximate KL is read back (one fp64, the only added host synchronisation); above
+        target_kl, the remaining epochs of both networks do not run. Unlike SB3's per-minibatch 1.5 x target_kl test, the
+        epoch that crossed the target completes, which keeps the actor / critic streams overlapped within the epoch."""
         B = s.shape[0]
         mb = mini_batch_size or self.mini_batch_size
+        if target_kl is _FROM_ARGS:
+            target_kl = self.target_kl
+        out = None
+        if stats or target_kl is not None:
+            out = PpoUpdateStats(torch.zeros((self.K_epochs, 2, _L.PPO_STATS_DOUBLES), dtype=torch.float64, device=s.device),
+                                 -(-B // mb), target_kl)
         if fused:
-            return self._optimize_fused(s, a, a_logprob, adv, v_target, mb, group)
+            self._optimize_fused(s, a, a_logprob, adv, v_target, mb, group, out)
+            return out
         dist = torch.distributed
-        if group is not False and dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+        multi = group is not False and dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
+        if multi:
             self._require_equal_batches(B, group, self.device)
+        acc = None
+        if out is not None:                               # static accumulator: a captured graph adds into it
+            if self._stats_acc is None or self._stats_acc.device != s.device:
+                self._stats_acc = torch.zeros((2, _L.PPO_STATS_DOUBLES), dtype=torch.float64, device=s.device)
+            acc = self._stats_acc
+            acc.zero_()
         tensors = (s, a, a_logprob, adv, v_target)
         graph = None
         if use_graph and B >= mb:
             try:
-                graph = self._graph_for(tensors, mb, group)
+                graph = self._graph_for(tensors, mb, group, acc)
             except Exception as exc:                      # capture not possible here: stay eager, say so once
                 import warnings
                 warnings.warn(f"CUDA-graph capture of the PPO step failed ({exc!r}); running eagerly")
                 graph = None
-        for _ in range(self.K_epochs):
+        for e in range(self.K_epochs):
             perm = torch.randperm(B, device=s.device)
             for lo in range(0, B, mb):
                 index = perm[lo:lo + mb]
@@ -373,8 +469,17 @@ class PPO_continuous:
                     graph["idx"].copy_(index)
                     graph["graph"].replay()
                 else:
-                    self._minibatch_step(*(t[index] for t in tensors), group)
+                    self._minibatch_step(*(t[index] for t in tensors), group, acc)
+            if out is not None:
+                if multi:                                 # per-rank minibatch means -> global means, the same on every rank
+                    dist.all_reduce(acc, group=group)
+                    acc /= dist.get_world_size(group)
+                out.records[e].copy_(acc)
+                acc.zero_()
+                if out.end_epoch(e):
+                    break
         self._dirty = True
+        return out
 
     def lr_decay(self, total_steps):
         lr_a_now = self.lr_a * (1 - total_steps / self.max_train_steps)

@@ -580,8 +580,11 @@ class PpoFusedNet:
         dev = next(module.parameters()).device
         self.device = dev
         self.params = torch.zeros(self.n + 2, dtype=torch.float32, device=dev)
-        self.grads = torch.zeros(self.n + 2, dtype=torch.float32, device=dev)        # [n] = minibatch loss
-        self._own_grads = self.grads
+        # [n] = minibatch loss, [n + 2, n + 6) = the actor's diagnostics (stats variant); `grads` is the first n + 2 floats,
+        # what the gradient exchange carries with stats off, `grads_stats` the whole buffer
+        self.n_stats = L.ppo_grad_floats_stats(self.heads)
+        self._own_grads = torch.zeros(self.n_stats, dtype=torch.float32, device=dev)
+        self._set_grads(self._own_grads)
         self.exp_avg = torch.zeros(self.n + 2, dtype=torch.float32, device=dev)
         self.exp_avg_sq = torch.zeros(self.n + 2, dtype=torch.float32, device=dev)
         self.step = torch.zeros(1, dtype=torch.int64, device=dev)
@@ -603,15 +606,13 @@ class PpoFusedNet:
         import torch.distributed._symmetric_memory as symm
         torch = self.torch
         g = group if group is not None else dist.group.WORLD
-        stride = _round_up(self.n + 2, 64)
+        stride = _round_up(self.n_stats, 64)
         buf = symm.empty(2 * stride, dtype=torch.float32, device=self.device)
         hdl = symm.rendezvous(buf, g.group_name)
         buf.zero_()
         self._peer = {"buf": buf, "hdl": hdl, "stride": stride, "parity": 0, "world": int(hdl.world_size),
                       "ptrs": int(hdl.buffer_ptrs_dev)}
-        self.grads = buf[:self.n + 2]
-        if self.net is not None:
-            self.net.grads = self.grads.data_ptr()
+        self._set_grads(buf[:self.n_stats])
         hdl.barrier()
         return self
 
@@ -619,10 +620,14 @@ class PpoFusedNet:
         """back to a private gradient buffer (used when the symmetric-memory rendezvous did not succeed on EVERY rank)"""
         if self._peer is not None or self.grads.data_ptr() != self._own_grads.data_ptr():
             self._peer = None
-            self.grads = self._own_grads
-            if self.net is not None:
-                self.net.grads = self.grads.data_ptr()
+            self._set_grads(self._own_grads)
         return self
+
+    def _set_grads(self, buf):
+        self.grads_stats = buf
+        self.grads = buf[:self.n + 2]
+        if getattr(self, "net", None) is not None:
+            self.net.grads = self.grads.data_ptr()
 
     def _slices(self):
         names = self.CRITIC_NAMES if self.critic else self.ACTOR_NAMES
@@ -667,31 +672,42 @@ class PpoFusedNet:
                                  None if self.critic else b + 4 * (o3 + 257 * self.heads), self.packed.data_ptr(),
                                  18, 256, self.heads, self.use_tanh, self.max_action)
 
-    def actor_grad(self, s, a, old_logp, adv, index, mb, epsilon, entropy_coef):
-        L.check(self.lib.sat_ppo_actor_grad(C.byref(self.net), L.ptr(s), L.ptr(a), L.ptr(old_logp), L.ptr(adv), index, mb,
-                                            float(epsilon), float(entropy_coef), L.stream_ptr()), "sat_ppo_actor_grad")
+    def actor_grad(self, s, a, old_logp, adv, index, mb, epsilon, entropy_coef, stats=False):
+        """stats: also the minibatch's diagnostics in grads_stats[n + 2:] (sat_ppo_actor_grad_stats; same gradient bits)"""
+        fn, name = (self.lib.sat_ppo_actor_grad_stats, "sat_ppo_actor_grad_stats") if stats else (self.lib.sat_ppo_actor_grad, "sat_ppo_actor_grad")
+        L.check(fn(C.byref(self.net), L.ptr(s), L.ptr(a), L.ptr(old_logp), L.ptr(adv), index, mb, float(epsilon),
+                   float(entropy_coef), L.stream_ptr()), name)
 
     def critic_grad(self, s, v_target, index, mb):
         L.check(self.lib.sat_ppo_critic_grad(C.byref(self.net), L.ptr(s), L.ptr(v_target), index, mb, L.stream_ptr()),
                 "sat_ppo_critic_grad")
 
-    def adam(self, max_grad_norm: float, grad_scale: float = 1.0):
+    def adam(self, max_grad_norm: float, grad_scale: float = 1.0, record=None):
+        """record: fp64 device tensor [PPO_STATS_DOUBLES] the step adds this minibatch's global statistics to
+        (sat_ppo_adam_stats; same parameter bits)"""
         pr = self._peer
+        args = (C.byref(self.net), L.ptr(self.lr), self.betas[0], self.betas[1], self.eps, float(max_grad_norm),
+                float(grad_scale), L.ptr(self.step))
+        if record is not None and (record.dtype != self.torch.float64 or record.numel() != L.PPO_STATS_DOUBLES):
+            raise L.SatError(f"record must be {L.PPO_STATS_DOUBLES} fp64 values")
         if pr is None:
-            L.check(self.lib.sat_ppo_adam(C.byref(self.net), L.ptr(self.lr), self.betas[0], self.betas[1], self.eps,
-                                          float(max_grad_norm), float(grad_scale), L.ptr(self.step), L.stream_ptr()), "sat_ppo_adam")
+            if record is None:
+                L.check(self.lib.sat_ppo_adam(*args, L.stream_ptr()), "sat_ppo_adam")
+            else:
+                L.check(self.lib.sat_ppo_adam_stats(*args, L.ptr(record), L.stream_ptr()), "sat_ppo_adam_stats")
             return
         # every rank's gradient kernels for this step are stream-ordered before its barrier; a rank can run at most one
         # step ahead of the slowest (the next barrier holds it), hence the two alternating halves of the buffer
         pr["hdl"].barrier()
         off = pr["parity"] * pr["stride"]
-        L.check(self.lib.sat_ppo_adam_peers(C.byref(self.net), L.ptr(self.lr), self.betas[0], self.betas[1], self.eps,
-                                            float(max_grad_norm), float(grad_scale), L.ptr(self.step), pr["ptrs"], pr["world"],
-                                            off, L.stream_ptr()), "sat_ppo_adam_peers")
+        if record is None:
+            L.check(self.lib.sat_ppo_adam_peers(*args, pr["ptrs"], pr["world"], off, L.stream_ptr()), "sat_ppo_adam_peers")
+        else:
+            L.check(self.lib.sat_ppo_adam_peers_stats(*args, pr["ptrs"], pr["world"], off, L.ptr(record), L.stream_ptr()),
+                    "sat_ppo_adam_peers_stats")
         pr["parity"] ^= 1
         off = pr["parity"] * pr["stride"]
-        self.grads = pr["buf"][off:off + self.n + 2]
-        self.net.grads = self.grads.data_ptr()
+        self._set_grads(pr["buf"][off:off + self.n_stats])
 
     def state_dict(self):
         return {"exp_avg": self.exp_avg.clone(), "exp_avg_sq": self.exp_avg_sq.clone(), "step": self.step.clone()}

@@ -47,6 +47,7 @@ class VectorTrainer:
         self.row_offset = rank * env.n
         self.seed = seed
         self.t_global = 0
+        self.explained_variance = None
         if self.obs_stats is not None:
             self.obs_stats.update_normalize(env.observe())          # statistics of the initial observations
         self.learner_is_pursuer = env.params.flag == 0
@@ -83,29 +84,47 @@ class VectorTrainer:
             x = (x - self.obs_stats.mean) / (self.obs_stats.std + 1e-8)
         buf.obs[self.T] = x.float()
 
-    def compute_advantages(self, group=None):
+    def compute_advantages(self, group=None, explained_variance=False):
+        """explained_variance: also set self.explained_variance (device fp64 scalar) = 1 - Var(adv) / Var(v_target) over the
+        rollout (all ranks of `group`), taken before the advantage normalisation; v_target - values == adv, so this is the
+        rollout-level explained variance of the critic"""
         buf, ag = self.buf, self.agent
         T, n = self.T, self.env.n
         ag.critic_kernel.value(buf.obs.view(-1, 18), out=buf.values.view(-1))
         r32 = buf.rew64.float()
         r_scale = (1.0 / (buf.ret_std + 1e-8)).float() if self.ret_stats is not None else None
         eng.gae_time_major(r32, buf.values, buf.done, ag.gamma, ag.lamda, r_scale=r_scale, adv=buf.adv, v_target=buf.v_target)
+        if explained_variance:
+            m = torch.stack([eng.adv_moments(buf.adv), eng.adv_moments(buf.v_target)])      # [2][sum, sum of squares, count]
+            dist = torch.distributed
+            if group is not False and dist.is_available() and dist.is_initialized():
+                pg = None if group in (None, True) else group
+                if dist.get_world_size(pg) > 1:
+                    dist.all_reduce(m, group=pg)
+            var = m[:, 1] / m[:, 2] - (m[:, 0] / m[:, 2]) ** 2
+            self.explained_variance = 1.0 - var[0] / var[1]
         if ag.use_adv_norm:
             eng.adv_normalize_(buf.adv, group=group)
         return buf.adv, buf.v_target
 
-    def update(self, mini_batch_size: int, total_steps: int = 0, group=None, use_graph: bool = True, fused: bool = True):
+    def update(self, mini_batch_size: int, total_steps: int = 0, group=None, use_graph: bool = True, fused: bool = True,
+               stats: bool = False):
         """fused: hand-written forward/backward/Adam kernels (csrc/ppo_update.cu); otherwise the PyTorch step, replayed as
-        a CUDA graph when use_graph."""
+        a CUDA graph when use_graph. Returns what the agent's optimize() returns: a PpoUpdateStats when stats (it then also
+        reports explained_variance) or the agent's target_kl is set, else None."""
         buf, ag = self.buf, self.agent
-        adv, v_target = self.compute_advantages(group)
+        adv, v_target = self.compute_advantages(group, explained_variance=stats)
         B = self.T * self.env.n
-        ag.optimize(buf.obs[:self.T].reshape(B, 18), buf.act.reshape(B, 3), buf.logp.reshape(B, 3), adv.reshape(B, 1),
-                    v_target.reshape(B, 1), mini_batch_size=mini_batch_size, group=group, use_graph=use_graph, fused=fused)
+        out = ag.optimize(buf.obs[:self.T].reshape(B, 18), buf.act.reshape(B, 3), buf.logp.reshape(B, 3), adv.reshape(B, 1),
+                          v_target.reshape(B, 1), mini_batch_size=mini_batch_size, group=group, use_graph=use_graph, fused=fused,
+                          stats=stats)
+        if stats:
+            out.extra["explained_variance"] = self.explained_variance
         if ag.use_lr_decay:
             ag.lr_decay(total_steps)
         if ag._dirty:
             ag.sync_kernels()
+        return out
 
 
     # ---- full-run checkpoint: env SoA state, running normalisers, Philox counter, networks + optimisers
@@ -148,19 +167,23 @@ class SelfPlay:
         self.trainers = {0: VectorTrainer(env, pursuer, evader, T, rank=rank, seed=seed, **kw),
                          1: VectorTrainer(env, evader, pursuer, T, rank=rank, seed=seed + 1, **kw)}
 
-    def run_phase(self, flag: int, iterations: int, group=None, use_graph: bool = True, fused: bool = True, callback=None):
+    def run_phase(self, flag: int, iterations: int, group=None, use_graph: bool = True, fused: bool = True, callback=None,
+                  stats: bool = False):
+        """stats: each iteration's record also carries the update's training diagnostics (PpoUpdateStats.as_dict keys and
+        explained_variance)"""
         env, tr = self.env, self.trainers[flag]
         env.reset(flag=flag)                                   # reset(Flag) for every env; fuel / dis / dz persist (Q2)
         tr.learner_is_pursuer = flag == 0
         out = []
         for it in range(iterations):
             tr.collect()
-            stats = {"flag": flag, "iteration": it, "mean_reward": float(tr.buf.rew64.mean()),
-                     "episodes_finished": int(tr.buf.done.sum())}
-            tr.update(self.mb, total_steps=it, group=group, use_graph=use_graph, fused=fused)
-            out.append(stats)
+            record = {"flag": flag, "iteration": it, "mean_reward": float(tr.buf.rew64.mean()),
+                      "episodes_finished": int(tr.buf.done.sum())}
+            upd = tr.update(self.mb, total_steps=it, group=group, use_graph=use_graph, fused=fused, stats=stats)
+            record = dict(record, **upd.as_dict()) if stats else record
+            out.append(record)
             if callback is not None:
-                callback(stats)
+                callback(record)
         return out
 
     def run(self, rounds: int, iterations_per_phase: int, **kw):

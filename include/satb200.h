@@ -273,10 +273,30 @@ int sat_cw_propagate(double* x, int64_t n, int64_t ld, const double* stm_host, v
 int sat_cw_ode_rk45(double* x, int64_t n, int64_t ld, double t_bound, double w2, double w3, double wz,
                     double rtol, double atol, int32_t* status_out, void* stream);
 /* calculate_orbital_elements(miu, R0, V0) (satellite_function.py:161-255): rv [n][6] -> (a,e,i,omega,Omega,f) [n][6];
- * kind_out [n] = 6, or 0 for the circular / parabolic element sets (which this library does not produce). */
+ * kind_out [n] = 6, or 0 (elements_out unspecified) for the circular / parabolic element sets: sat_orbital_elements_all
+ * returns those. */
 int sat_orbital_elements(const double* rv, int64_t n, double miu, double* elements_out, int32_t* kind_out, void* stream);
 /* calculate_state_information(data, miu) (satellite_function.py:257-315), six-element form: -> rv [n][6]. */
 int sat_state_from_elements(const double* elements, int64_t n, double miu, double* rv_out, void* stream);
+/* calculate_orbital_elements on every branch: elements_out [n][6] holds the list the reference returns, zero-padded, and
+ * kind_out [n] its length, which names the branch (SAT_ELEM_KIND_*):
+ *   SAT_ELEM_KIND_GENERAL   6: columns 0-5 = a, e, i, omega, Omega, f   (energy != 0 and e != 0: elliptic / hyperbolic;
+ *                              the same bits as sat_orbital_elements)
+ *   SAT_ELEM_KIND_PARABOLIC 5: columns 0-4 = p, i, omega, Omega, f      (energy == 0 exactly; column 5 = 0)
+ *   SAT_ELEM_KIND_CIRCULAR  4: columns 0-3 = a, i, u, Omega             (e == 0 exactly; u = argument of latitude, NaN for
+ *                              an equatorial orbit as in the reference; columns 4-5 = 0)
+ * Bit-identical to the reference's arithmetic on every branch (the host libm's acos and pow, csrc/glibm.cuh). */
+#define SAT_ELEM_KIND_GENERAL 6
+#define SAT_ELEM_KIND_PARABOLIC 5
+#define SAT_ELEM_KIND_CIRCULAR 4
+int sat_orbital_elements_all(const double* rv, int64_t n, double miu, double* elements_out, int32_t* kind_out,
+                             void* stream);
+/* calculate_state_information(data, miu) for n element sets of n_el elements each, elements [n][n_el] -> rv [n][6]:
+ *   n_el = 6: (a, e, i, omega, Omega, f), exactly sat_state_from_elements;
+ *   n_el = 5: (p, i, omega, Omega, f), the parabolic form (e = 1);
+ *   n_el = 4: (a, i, u, Omega), the circular form (e = 0).
+ * The 5- and 4-element forms use the host libm's sin, cos and pow (csrc/glibm.cuh). Any other n_el: SAT_ERR_SIZE. */
+int sat_state_from_elements_n(const double* elements, int64_t n, int n_el, double miu, double* rv_out, void* stream);
 
 /* Reachable-domain sweep (SURVEY.md s8 f.3). Replaces Reachable_Domain() of single_pluse_model/RD_single_pulse.py:40-148
  * (N1 = 1) for n pursuer states given as elements [n][6] = (a, e, i, omega, Omega, f) and delta_max [n]: for each of the

@@ -68,6 +68,9 @@ def ppo_grad_floats_stats(heads: int) -> int:
  PPO_STAT_CLIP_COEF, PPO_STAT_COUNT) = range(8)
 PPO_STATS_DOUBLES = 8
 
+# kind codes of sat_orbital_elements_all (SAT_ELEM_KIND_*): the number of elements the reference returns on each branch
+ELEM_KIND_GENERAL, ELEM_KIND_PARABOLIC, ELEM_KIND_CIRCULAR = 6, 5, 4
+
 
 _P, _I64, _I32, _D, _F, _U64 = C.c_void_p, C.c_int64, C.c_int, C.c_double, C.c_float, C.c_uint64
 SIGNATURES = {
@@ -91,6 +94,8 @@ SIGNATURES = {
     "sat_reachable_domain": (C.c_int, [_P, _P, _I64, _I32, _I32, _D, _P, _P, _P, _P]),
     "sat_orbital_elements": (C.c_int, [_P, _I64, _D, _P, _P, _P]),
     "sat_state_from_elements": (C.c_int, [_P, _I64, _D, _P, _P]),
+    "sat_orbital_elements_all": (C.c_int, [_P, _I64, _D, _P, _P, _P]),
+    "sat_state_from_elements_n": (C.c_int, [_P, _I64, _I32, _D, _P, _P]),
     "sat_workspace_bytes": (_I64, [_I64]),
     "sat_env_default_params": (None, [C.POINTER(SatEnvParams)]),
     "sat_env_init": (C.c_int, [C.POINTER(SatEnvState), _D, _D, C.POINTER(SatEnvParams), _P]),

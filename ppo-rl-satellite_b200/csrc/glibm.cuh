@@ -1,4 +1,4 @@
-// glibm.cuh -- sin / cos / acos / atan / pow(x, 2) with the SAME BITS as the host libm the reference runs on.
+// glibm.cuh -- sin / cos / acos / atan / pow(x, 2) / pow(x, 0.5) with the SAME BITS as the host libm the reference runs on.
 //
 // Why this exists (DESIGN.md s3, VERDICT r01 item 1): the reference's danger-zone count
 // (environment.py:317-332 -> satellite_function.py:161-255, :317-373, :462-565) is an integer that depends on the last
@@ -13,7 +13,7 @@
 //   s_sin.c   __sin / __cos   (do_sin, do_cos, TAYLOR_SIN, reduce_sincos; |x| < 105414350, above that -> NaN here)
 //   e_asin.c  __ieee754_acos  (all ranges)
 //   s_atan.c  __atan          (all ranges)
-//   e_pow.c   __pow           (log_inline + exp_inline, for y == 2.0 only; |x| outside [2^-369, 2^369] -> x*x here)
+//   e_pow.c   __pow           (log_inline + exp_inline, for y == 2.0 and y == 0.5; y == 2: |x| outside [2^-369, 2^369] -> x*x here)
 // in the variant the ifunc resolvers select on every FMA-capable x86-64 host (__sin_fma, __cos_fma, __atan_fma,
 // __ieee754_acos_fma, __pow_fma): those are the generic sources compiled with -mfma, i.e. with GCC's contraction of
 // a*b+c into fused operations.  Which operations are fused was read off the machine code of the libm in this image;
@@ -341,7 +341,7 @@ GLIBM_FN double atan(double x) {
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// e_pow.c: pow(x, 2.0)  (python / numpy scalar `x ** 2`)
+// e_pow.c: pow(x, 2.0)  (python / numpy scalar `x ** 2`) and pow(x, 0.5)
 // ---------------------------------------------------------------------------------------------------------------
 namespace k {
 constexpr double LN2HI = 0x1.62e42fefa3800p-1, LN2LO = 0x1.ef35793c76730p-45;
@@ -351,12 +351,9 @@ constexpr double INVLN2N = 0x1.71547652b82fep+7, SHIFT = 0x1.8p52, NEGLN2HIN = -
 constexpr double C2 = 0x1.ffffffffffdbdp-2, C3 = 0x1.555555555543cp-3, C4 = 0x1.55555cf172b91p-5, C5 = 0x1.1111167a4d017p-7;
 }  // namespace k
 
-GLIBM_FN double pow2(double x) {
-    uint64_t ix = bits_(x) & 0x7fffffffffffffffull;                          // y = 2 is an even integer: sign of x is dropped
-    uint32_t topx = (uint32_t)(ix >> 52);
-    if (topx == 0x7ffu || ix == 0ull) return mul_(x, x);                     // 0, inf, nan
-    if (topx == 0u) { ix = (bits_(mul_(dbl_(ix), 0x1p52)) & 0x7fffffffffffffffull) - (52ull << 52); topx = (uint32_t)(ix >> 52) & 0x7ffu; }
-    if (topx < 0x3ffu - 369u || topx > 0x3ffu + 369u) return mul_(x, x);     // result near over/underflow: not restated
+// log_inline + exp_inline of e_pow.c for y = 2 or 0.5: ix is the bit pattern of a positive normal x whose |y log x| stays
+// below 512, so neither of exp_inline's special cases is reached
+GLIBM_FN double pow_core(uint64_t ix, double y) {
     // log_inline
     const uint64_t tmp = ix - 0x3fe6955500000000ull;
     const int i = (int)((tmp >> 45) & 0x7f);
@@ -380,9 +377,9 @@ GLIBM_FN double pow2(double x) {
     const double lo = fma_(ar3, pp, add_(add_(add_(lo1, lo2), lo3), lo4));
     const double lhi = add_(hi, lo);
     const double llo = add_(sub_(hi, lhi), lo);
-    // pow: ehi + elo = y log(x), y = 2
-    const double ehi = mul_(2.0, lhi);
-    const double elo = fma_(2.0, llo, fma_(lhi, 2.0, neg_(ehi)));
+    // pow: ehi + elo = y log(x)
+    const double ehi = mul_(y, lhi);
+    const double elo = fma_(y, llo, fma_(lhi, y, neg_(ehi)));
     // exp_inline
     const uint32_t abstop = (uint32_t)(bits_(ehi) >> 52) & 0x7ffu;
     if (abstop < 0x3c9u) return add_(1.0, ehi);                              // |y log x| < 2^-54
@@ -401,6 +398,25 @@ GLIBM_FN double pow2(double x) {
     return fma_(tmp2, scale, scale);
 }
 
+GLIBM_FN double pow2(double x) {
+    uint64_t ix = bits_(x) & 0x7fffffffffffffffull;                          // y = 2 is an even integer: sign of x is dropped
+    uint32_t topx = (uint32_t)(ix >> 52);
+    if (topx == 0x7ffu || ix == 0ull) return mul_(x, x);                     // 0, inf, nan
+    if (topx == 0u) { ix = (bits_(mul_(dbl_(ix), 0x1p52)) & 0x7fffffffffffffffull) - (52ull << 52); topx = (uint32_t)(ix >> 52) & 0x7ffu; }
+    if (topx < 0x3ffu - 369u || topx > 0x3ffu + 369u) return mul_(x, x);     // result near over/underflow: not restated
+    return pow_core(ix, 2.0);
+}
+
+// pow(x, 0.5) (python `x ** 0.5`; not sqrt(x): glibc's pow is not correctly rounded). |0.5 log x| < 373 for every positive
+// double, so all of them are restated.
+GLIBM_FN double pow_half(double x) {
+    uint64_t ix = bits_(x);
+    if (2 * ix - 1 >= 2 * 0x7ff0000000000000ull - 1) return mul_(x, x);     // +-0, +-inf, nan (e_pow.c zeroinfnan)
+    if (ix >> 63) return nan_();                                             // finite x < 0: invalid
+    if ((ix >> 52) == 0u) ix = (bits_(mul_(x, 0x1p52)) & 0x7fffffffffffffffull) - (52ull << 52);   // subnormal
+    return pow_core(ix, 0.5);
+}
+
 #if defined(__CUDACC__)
 // Out-of-line copies for straight-line device code with many call sites (orbital elements, danger-zone set-up): one
 // body per function keeps the kernel inside the instruction cache (inlined everywhere the danger-zone kernel grew to
@@ -411,6 +427,7 @@ static __device__ __noinline__ double cos(double x) { return glibm::cos(x); }
 static __device__ __noinline__ double acos(double x) { return glibm::acos(x); }
 static __device__ __noinline__ double atan(double x) { return glibm::atan(x); }
 static __device__ __noinline__ double pow2(double x) { return glibm::pow2(x); }
+static __device__ __noinline__ double pow_half(double x) { return glibm::pow_half(x); }
 }  // namespace call
 #endif
 

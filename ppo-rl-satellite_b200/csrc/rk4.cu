@@ -144,6 +144,44 @@ __global__ void state_info_kernel(const double* __restrict__ el, int64_t n, doub
     rv[idx * 6 + 5] = s * (si * (cu + e * co));
 }
 
+// calculate_orbital_elements on every branch: the reference's list, zero-padded to 6 columns, and its length as the kind
+__global__ void elements_all_kernel(const double* __restrict__ rv, int64_t n, double miu, double* __restrict__ out,
+                                    int32_t* __restrict__ kind) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    double R[3] = {rv[i * 6], rv[i * 6 + 1], rv[i * 6 + 2]}, V[3] = {rv[i * 6 + 3], rv[i * 6 + 4], rv[i * 6 + 5]};
+    Elements el = {0, 0, 0, 0, 0, 0};
+    kind[i] = orbital_elements<true, true>(miu, R, V, el);
+    out[i * 6] = el.a; out[i * 6 + 1] = el.e; out[i * 6 + 2] = el.i;
+    out[i * 6 + 3] = el.omega; out[i * 6 + 4] = el.Omega; out[i * 6 + 5] = el.f;
+}
+
+// calculate_state_information (satellite_function.py:287-315), the forms the parabolic and circular branches return:
+//   NEL = 5: [p, i, omega, Omega, f], e = 1;   NEL = 4: [a, i, u, Omega], e = 0, p = a, omega = 0, f = u.
+// Both run the six-element form's tail (:303-315) with the host libm's sin, cos and pow (glibm.cuh), so they are
+// bit-identical to the reference's arithmetic.
+template <int NEL>
+__global__ void state_info_form_kernel(const double* __restrict__ el, int64_t n, double miu, double* __restrict__ rv) {
+    const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= n) return;
+    const double* d = el + idx * NEL;
+    double p, e, i, omega, Omega, f, u;
+    if constexpr (NEL == 5) { p = d[0]; i = d[1]; omega = d[2]; Omega = d[3]; f = d[4]; e = 1.0; u = omega + f; }
+    else { p = d[0]; i = d[1]; u = d[2]; Omega = d[3]; e = 0.0; omega = 0.0; f = u; }
+    const double2 scO = glibm::call::sincos(Omega), scu = glibm::call::sincos(u), sci = glibm::call::sincos(i);
+    const double2 sco = (NEL == 5) ? glibm::call::sincos(omega) : make_double2(0.0, 1.0);
+    const double cf = (NEL == 5) ? glibm::call::cos(f) : scu.y;
+    const double sO = scO.x, cO = scO.y, su = scu.x, cu = scu.y, si = sci.x, ci = sci.y, so = sco.x, co = sco.y;
+    const double k = p / (1.0 + e * cf);                                  // :303
+    rv[idx * 6 + 0] = k * (cO * cu - sO * su * ci);
+    rv[idx * 6 + 1] = k * (sO * cu + cO * su * ci);
+    rv[idx * 6 + 2] = k * (si * su);
+    const double s = glibm::call::pow_half(miu / p);                     // :309
+    rv[idx * 6 + 3] = s * (-cO * (su + e * so) - sO * (cu + e * co) * ci);
+    rv[idx * 6 + 4] = s * (-sO * (su + e * so) + cO * (cu + e * co) * ci);
+    rv[idx * 6 + 5] = s * (si * (cu + e * co));
+}
+
 // packed FFMA2 (fma.rn.f32x2) chain: the fp32 issue-rate ceiling of sm_100
 __global__ void peak_ffma2_kernel(float* sink, int iters) {
     float2 a[8];
@@ -236,6 +274,24 @@ int sat_state_from_elements(const double* elements, int64_t n, double miu, doubl
     if (!elements || !rv_out) return SAT_ERR_NULL;
     if (n <= 0) return SAT_ERR_SIZE;
     state_info_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(elements, n, miu, rv_out);
+    return launch_status();
+}
+
+int sat_orbital_elements_all(const double* rv, int64_t n, double miu, double* elements_out, int32_t* kind_out,
+                             void* stream) {
+    if (!rv || !elements_out || !kind_out) return SAT_ERR_NULL;
+    if (n <= 0) return SAT_ERR_SIZE;
+    elements_all_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(rv, n, miu, elements_out, kind_out);
+    return launch_status();
+}
+
+int sat_state_from_elements_n(const double* elements, int64_t n, int n_el, double miu, double* rv_out, void* stream) {
+    if (n_el == 6) return sat_state_from_elements(elements, n, miu, rv_out, stream);
+    if (!elements || !rv_out) return SAT_ERR_NULL;
+    if (n <= 0 || (n_el != 5 && n_el != 4)) return SAT_ERR_SIZE;
+    const unsigned blocks = (unsigned)((n + 127) / 128);
+    if (n_el == 5) state_info_form_kernel<5><<<blocks, 128, 0, (cudaStream_t)stream>>>(elements, n, miu, rv_out);
+    else state_info_form_kernel<4><<<blocks, 128, 0, (cudaStream_t)stream>>>(elements, n, miu, rv_out);
     return launch_status();
 }
 

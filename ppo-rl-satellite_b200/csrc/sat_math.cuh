@@ -163,13 +163,17 @@ struct Lm {
 };
 
 // ------------------------------------------------------------------------------------------
-// orbital elements, satellite_function.py:161-255 (six-element branch; returns false for the
-// circular / parabolic branches, for which the reference's danger-zone code raises)
+// orbital elements, satellite_function.py:161-255. The reference returns a list whose length gives the branch:
+//   6: [a, e, i, omega, Omega, f]   energy != 0, e != 0 (elliptic or hyperbolic)
+//   5: [p, i, omega, Omega, f]      energy == 0 (parabolic, :186-190, :247-253)
+//   4: [a, i, u, Omega]             e == 0 (circular, :212, :223-227)
+// ALL = false (the danger-zone path; the reference's danger-zone code raises on the last two): returns 6, or 0 for the
+// parabolic / circular branches. ALL = true: returns the length and writes the list into el's fields in order.
 // ------------------------------------------------------------------------------------------
 struct Elements { double a, e, i, omega, Omega, f; };
 
-template <bool EXACT = true>
-SAT_DEV bool orbital_elements(double miu, const double R0[3], const double V0[3], Elements& el) {
+template <bool EXACT = true, bool ALL = false>
+SAT_DEV int orbital_elements(double miu, const double R0[3], const double V0[3], Elements& el) {
     double r_norm = norm3(R0), v_norm = norm3(V0);                       // :183-184
     double r_dot_v = dot3(R0, V0);                                       // :185
     double v2 = Lm<EXACT>::pow2(v_norm);                                     // v_norm ** 2 (:186, :193)
@@ -183,7 +187,9 @@ SAT_DEV bool orbital_elements(double miu, const double R0[3], const double V0[3]
     double h = norm3(H);                                                 // :199
     N[0] = -H[1]; N[1] = H[0]; N[2] = 0.0;                               // :206 cross([0,0,1], H)
     double n = norm3(N);                                                 // :208
-    if (energy == 0.0 || e == 0.0) return false;
+    if constexpr (!ALL) {
+        if (energy == 0.0 || e == 0.0) return 0;
+    }
     el.a = 1.0 / fabs(energy);                                           // :188
     el.e = e;
     el.i = Lm<EXACT>::acos(H[2] / h);                                               // :210
@@ -196,7 +202,17 @@ SAT_DEV bool orbital_elements(double miu, const double R0[3], const double V0[3]
     double f = Lm<EXACT>::acos(dot3(E, R0) / e / r_norm);                           // :242
     if (r_dot_v < 0.0) f = kTwoPi - f;
     el.f = f;
-    return true;
+    if constexpr (ALL) {
+        // e == 0: the reference leaves omega and f at 0 (above they are acos of 0 / 0) and computes u instead (:223-227)
+        if (e == 0.0) {
+            el.omega = 0.0; el.f = 0.0;
+            double u = Lm<EXACT>::acos(dot3(N, R0) / n / r_norm);                  // :225
+            if (R0[2] < 0.0) u = kTwoPi - u;
+            if (energy != 0.0) { el = {el.a, el.i, u, el.Omega, 0.0, 0.0}; return 4; }
+        }
+        if (energy == 0.0) { el = {Lm<EXACT>::pow2(h) / miu, el.i, el.omega, el.Omega, el.f, 0.0}; return 5; }   // p (:201)
+    }
+    return 6;
 }
 
 // ------------------------------------------------------------------------------------------

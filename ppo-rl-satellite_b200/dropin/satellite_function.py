@@ -2,7 +2,7 @@
 
 Clohessy_Wiltshire.State_transition_matrix, Time_window_of_danger_zone.{calculate_orbital_elements,
 calculate_state_information, calculate_number_of_hanger_area} run as CUDA kernels (batch of one, or batched when
-given arrays with a leading axis). Numerical_calculation_method.numerical_calculation (the RK45 propagator the env has
+given arrays with a leading axis); the first two cover every branch and element-set form of the reference. Numerical_calculation_method.numerical_calculation (the RK45 propagator the env has
 commented out) is a per-state adaptive kernel. Out of scope (never called by the env or the driver, SURVEY.md s2): the
 time-window sweep, Lagrange propagation, Danger_index_and_TW_matching_index.
 """
@@ -68,28 +68,17 @@ class Time_window_of_danger_zone:
 
     @staticmethod
     def calculate_orbital_elements(miu, R0, V0):
-        """satellite_function.py:161-255 -> [a, e, i, omega, Omega, f] (six-element branch)."""
-        import torch
-        rv = _dev(np.concatenate([np.asarray(R0, dtype=np.float64), np.asarray(V0, dtype=np.float64)]).reshape(1, 6))
-        out = torch.empty((1, 6), dtype=torch.float64, device="cuda")
-        kind = torch.empty(1, dtype=torch.int32, device="cuda")
-        _L.check(_L.load().sat_orbital_elements(rv.data_ptr(), 1, float(miu), out.data_ptr(), kind.data_ptr(),
-                                                _L.stream_ptr()), "sat_orbital_elements")
-        if int(kind[0]) != 6:
-            raise NotImplementedError("circular / parabolic element sets are not produced by the CUDA path")
-        return [float(v) for v in out.cpu().numpy()[0]]
+        """satellite_function.py:161-255 -> [a, e, i, omega, Omega, f]; on the parabolic branch (energy == 0)
+        [p, i, omega, Omega, f], on the circular branch (e == 0) [a, i, u, Omega]."""
+        rv = np.concatenate([np.asarray(R0, dtype=np.float64), np.asarray(V0, dtype=np.float64)]).reshape(1, 6)
+        out, kind = orbital_elements_batch(miu, rv)
+        return [float(v) for v in out[0, :int(kind[0])]]
 
     @staticmethod
     def calculate_state_information(data, miu=3.986e14):
-        """satellite_function.py:257-315 (six-element form) -> (Coordinate[3], V[3])."""
-        import torch
-        if len(data) != 6:
-            raise NotImplementedError("only the six-element form is on the CUDA path")
-        el = _dev(np.asarray(data, dtype=np.float64).reshape(1, 6))
-        out = torch.empty((1, 6), dtype=torch.float64, device="cuda")
-        _L.check(_L.load().sat_state_from_elements(el.data_ptr(), 1, float(miu), out.data_ptr(), _L.stream_ptr()),
-                 "sat_state_from_elements")
-        o = out.cpu().numpy()[0]
+        """satellite_function.py:257-315 -> (Coordinate[3], V[3]) from [a, e, i, omega, Omega, f], [p, i, omega, Omega, f]
+        or [a, i, u, Omega]."""
+        o = state_information_batch(np.asarray(data, dtype=np.float64).reshape(1, -1), miu=miu)[0]
         return o[:3].copy(), o[3:].copy()
 
     def calculate_number_of_hanger_area(self):
@@ -136,20 +125,24 @@ class Numerical_calculation_method:
 
 
 def orbital_elements_batch(miu, rv):
-    """rv: [n, 6] array (R, V) -> elements [n, 6], kind [n] (batched helper, CUDA)."""
+    """rv: [n, 6] array (R, V) -> elements [n, 6], kind [n] (batched helper, CUDA). Row k holds the list
+    calculate_orbital_elements returns, zero-padded; kind[k] is its length: 6, 5 (parabolic) or 4 (circular)."""
     import torch
     rv = _dev(rv)
     out = torch.empty_like(rv)
     kind = torch.empty(rv.shape[0], dtype=torch.int32, device="cuda")
-    _L.check(_L.load().sat_orbital_elements(rv.data_ptr(), rv.shape[0], float(miu), out.data_ptr(), kind.data_ptr(),
-                                            _L.stream_ptr()), "sat_orbital_elements")
+    _L.check(_L.load().sat_orbital_elements_all(rv.data_ptr(), rv.shape[0], float(miu), out.data_ptr(), kind.data_ptr(),
+                                                _L.stream_ptr()), "sat_orbital_elements_all")
     return out.cpu().numpy(), kind.cpu().numpy()
 
 
 def state_information_batch(el, miu=3.986e14):
+    """el: [n, 6], [n, 5] or [n, 4] element sets (the forms calculate_state_information takes) -> [n, 6] (R, V)."""
     import torch
     el = _dev(el)
-    out = torch.empty_like(el)
-    _L.check(_L.load().sat_state_from_elements(el.data_ptr(), el.shape[0], float(miu), out.data_ptr(), _L.stream_ptr()),
-             "sat_state_from_elements")
+    if el.dim() != 2 or el.shape[1] not in (6, 5, 4):
+        raise ValueError(f"element sets must be [n, 6], [n, 5] or [n, 4], got {tuple(el.shape)}")
+    out = torch.empty((el.shape[0], 6), dtype=torch.float64, device="cuda")
+    _L.check(_L.load().sat_state_from_elements_n(el.data_ptr(), el.shape[0], el.shape[1], float(miu), out.data_ptr(),
+                                                 _L.stream_ptr()), "sat_state_from_elements_n")
     return out.cpu().numpy()

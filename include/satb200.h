@@ -59,7 +59,8 @@ enum { SAT_COL_P = 0, SAT_COL_PV = 3, SAT_COL_E = 6, SAT_COL_EV = 9,
 enum { SAT_ICOL_DZ = 0, SAT_ICOL_COUNT = 1, SAT_ICOL_INTSTATE = 2, SAT_ICOL_ERR = 3, SAT_ISTATE_COLS = 4 };
 
 typedef struct {
-    double*  state;    /* [SAT_STATE_COLS][ld] fp64: P(3) Pv(3) E(3) Ev(3) fuel_c fuel_t dis R(discounted return) */
+    double*  state;    /* [SAT_STATE_COLS][ld] fp64: P(3) Pv(3) E(3) Ev(3) fuel_c fuel_t dis R(discounted return);
+                        * [SAT_STATE_COLS_STARTS][ld] with the per-env start columns (below) */
     int32_t* istate;   /* [SAT_ISTATE_COLS][ld]: dangerous_zone, episode step count, int_state (Q1), err */
     int64_t  n;        /* number of environments */
     int64_t  ld;       /* column stride (elements), >= n, even */
@@ -72,7 +73,9 @@ typedef struct {
     int32_t mode;               /* SAT_MODE_CW: the shipped env (CW STM); SAT_MODE_RK4: S RK4 substeps (inertial) */
     int32_t flag;               /* 0 pursuer training (environment.py:83-179), 1 evader training (:181-255) */
     int32_t max_episode_steps;  /* environment.py:46 */
-    int32_t auto_reset;         /* 1: envs that finish are reset in the same launch (batched contract) */
+    int32_t auto_reset;         /* 0: none; SAT_RESET_STARTS (2): envs that finish are reset to their start columns in the
+                                 * same launch (needs a SAT_STATE_COLS_STARTS-column state buffer); any other non-zero
+                                 * value: reset to reset_p / reset_e in the same launch (batched contract) */
     int32_t action_dtype;       /* SAT_ACT_F32 / SAT_ACT_F64; layout [n][3] */
     int32_t substeps;           /* rk4 mode: RK4 substeps per env step */
     int32_t skip_danger_zone;   /* 1: do not evaluate the danger-zone count (keeps it at its stale value) */
@@ -102,6 +105,25 @@ int sat_env_init(const SatEnvState* st, double fuel_c, double fuel_t, const SatE
 /* reset(Flag) (environment.py:66-79) for envs whose mask byte is non-zero (mask NULL = all).
  * fuel / dis / dangerous_zone persist exactly as in the reference (they are never reset there). */
 int sat_env_reset(const SatEnvState* st, const uint8_t* mask, const SatEnvParams* p, void* stream);
+/* Per-env start states. A state buffer of SAT_STATE_COLS_STARTS columns holds in columns SAT_COL_START .. +11 each env's
+ * NEXT start, in the order of columns 0..11 (P, Pv, E, Ev, CW frame, metres and m/s). With auto_reset == SAT_RESET_STARTS,
+ * sat_env_step / sat_env_step_timed / sat_env_step_host reset a finished env to its start columns: kinematics from the
+ * columns, count = 0 and int_state = 0 (a float start has no int64 truncation, Q1); fuel, dis, dangerous_zone persist and
+ * the discounted return resets on done, as in the default reset. The step does not redraw the starts: call
+ * sat_env_draw_starts with the step's done mask afterwards. The columns are ordinary device memory: a caller who wants
+ * another distribution writes them directly. */
+enum { SAT_COL_START = 16, SAT_STATE_COLS_STARTS = 28 };
+#define SAT_RESET_STARTS 2
+/* draw the next start of every env whose mask byte is non-zero (mask NULL = all) into the start columns, uniform in the
+ * box lo_host[c] <= x <= hi_host[c] (lo == hi fixes a column). lo_host / hi_host: [12] host arrays copied into the launch.
+ * Keyed by (seed, row_offset + env index, draw) only: Philox4x32-10, key (uint32)seed, (uint32)(seed >> 32) ^ 0x53434E31,
+ * counter (g_lo, g_hi, draw, j) for j = 0..5; block j's (c0, c1) and (c2, c3) give columns 2j and 2j + 1 as
+ * u = ((c_a << 32 | c_b) >> 11) * 2^-53 and x = min(lo + (hi - lo) * u, hi), each operation rounded, x = lo when lo == hi.
+ * NULL bounds: SAT_ERR_NULL; lo > hi, a non-finite bound or box width, row_offset < 0: SAT_ERR_SIZE. */
+int sat_env_draw_starts(const SatEnvState* st, const uint8_t* mask, const double* lo_host, const double* hi_host,
+                        uint64_t seed, uint32_t draw, int64_t row_offset, void* stream);
+/* reset() to the start columns for the masked envs (mask NULL = all): kinematics, count = 0, int_state = 0 */
+int sat_env_reset_starts(const SatEnvState* st, const uint8_t* mask, void* stream);
 /* observation of the current state: [n][18] = [P-E, Pv-Ev, P, Pv, E, Ev] (environment.py:76-77) */
 int sat_env_observe(const SatEnvState* st, float* obs_f32, double* obs_f64, void* stream);
 /* The fp32 observation the policy networks are fed: rebuilt from the fp64 state (environment.py:76-77) and, when obs_stats !=

@@ -15,6 +15,9 @@ LIB_PATH = os.path.join(_HERE, "lib", "libsatb200.so")
 SAT_STATE_COLS = 16
 SAT_ISTATE_COLS = 4
 COL_P, COL_PV, COL_E, COL_EV, COL_FUEL_C, COL_FUEL_T, COL_DIS, COL_RET = 0, 3, 6, 9, 12, 13, 14, 15
+# per-env start states: SAT_STATE_COLS_STARTS-column buffers hold each env's next start in columns COL_START .. +11
+COL_START, SAT_STATE_COLS_STARTS = 16, 28
+RESET_STARTS = 2                  # SatEnvParams.auto_reset value: reset finished envs to their start columns
 ICOL_DZ, ICOL_COUNT, ICOL_INTSTATE, ICOL_ERR = 0, 1, 2, 3
 MODE_CW, MODE_RK4 = 0, 1
 ACT_F32, ACT_F64 = 0, 1
@@ -72,7 +75,7 @@ PPO_STATS_DOUBLES = 8
 ELEM_KIND_GENERAL, ELEM_KIND_PARABOLIC, ELEM_KIND_CIRCULAR = 6, 5, 4
 
 
-_P, _I64, _I32, _D, _F, _U64 = C.c_void_p, C.c_int64, C.c_int, C.c_double, C.c_float, C.c_uint64
+_P, _I64, _I32, _D, _F, _U64, _U32 = C.c_void_p, C.c_int64, C.c_int, C.c_double, C.c_float, C.c_uint64, C.c_uint32
 SIGNATURES = {
     "sat_abi_version": (C.c_int, []),
     "sat_strerror": (C.c_char_p, [C.c_int]),
@@ -100,6 +103,9 @@ SIGNATURES = {
     "sat_env_default_params": (None, [C.POINTER(SatEnvParams)]),
     "sat_env_init": (C.c_int, [C.POINTER(SatEnvState), _D, _D, C.POINTER(SatEnvParams), _P]),
     "sat_env_reset": (C.c_int, [C.POINTER(SatEnvState), _P, C.POINTER(SatEnvParams), _P]),
+    "sat_env_draw_starts": (C.c_int, [C.POINTER(SatEnvState), _P, C.POINTER(C.c_double), C.POINTER(C.c_double), _U64, _U32,
+                                      _I64, _P]),
+    "sat_env_reset_starts": (C.c_int, [C.POINTER(SatEnvState), _P, _P]),
     "sat_env_observe": (C.c_int, [C.POINTER(SatEnvState), _P, _P, _P]),
     "sat_env_observe_norm": (C.c_int, [C.POINTER(SatEnvState), _P, _P, _P]),
     "sat_env_step": (C.c_int, [C.POINTER(SatEnvState), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,

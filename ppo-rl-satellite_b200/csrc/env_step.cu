@@ -130,7 +130,8 @@ SAT_DEV void propagate_rk4(const SatEnvParams& p, Lane& L) {
 // OBS = true (host-buffer path): the kernel also writes the step's NEXT observation (after the auto reset) to obs_early.
 // The observation depends only on the propagated state and the terminal checks, not on the danger-zone solve of kernel
 // B, so its device-to-host copy can run on a copy engine underneath kernel B.
-template <typename ActT, bool OBS>
+// STARTS (auto_reset == SAT_RESET_STARTS, OBS only): the post-reset observation comes from the env's start columns.
+template <typename ActT, bool OBS, bool STARTS = false>
 __global__ void __launch_bounds__(kFrontBlock, 14)
 env_front_rk4_kernel(const SatEnvState st, const ActT* __restrict__ pa, const ActT* __restrict__ ea,
                      double* __restrict__ dis_prev_out, float* __restrict__ obs_early,
@@ -181,8 +182,19 @@ env_front_rk4_kernel(const SatEnvState st, const ActT* __restrict__ pa, const Ac
         const int count_new = st.istate[SAT_ICOL_COUNT * st.ld + e] + 1;
         const bool done = (dis <= p.d_capture) || (count_new >= p.max_episode_steps);
         if (done && p.auto_reset) {
+            if (STARTS) {
+                // each lane loads the start columns itself: the lanes of one env agree on `done`, a warp does not
+                const int64_t ld = st.ld;
+                const double* __restrict__ Sst = st.state + SAT_COL_START * ld;
 #pragma unroll
-            for (int k = 0; k < 3; ++k) { P[k] = p.reset_p[k]; E[k] = p.reset_e[k]; Pv[k] = 0.0; Ev[k] = 0.0; }
+                for (int k = 0; k < 3; ++k) {
+                    P[k] = Sst[(SAT_COL_P + k) * ld + e]; Pv[k] = Sst[(SAT_COL_PV + k) * ld + e];
+                    E[k] = Sst[(SAT_COL_E + k) * ld + e]; Ev[k] = Sst[(SAT_COL_EV + k) * ld + e];
+                }
+            } else {
+#pragma unroll
+                for (int k = 0; k < 3; ++k) { P[k] = p.reset_p[k]; E[k] = p.reset_e[k]; Pv[k] = 0.0; Ev[k] = 0.0; }
+            }
         }
         if (valid) {
             float* o = obs_early + e * kObs + craft * 9;
@@ -271,8 +283,11 @@ SAT_DEV void queue_run(SolveQueue& q) {
 // back half of step(): exchange, distance, terminal checks, danger zone, reward, observation, statistics
 // partials, auto-reset. environment.py:130-179 / :212-255, :317-343, :346-396.
 // FUSED = true: front half in the same kernel (cw mode, where propagation is one 6x6 product).
+// STARTS = true (auto_reset == SAT_RESET_STARTS): a reset puts the env at its start columns (SAT_COL_START..+11) with
+// int_state = 0 instead of at reset_p / reset_e with int_state = 1. The two lanes of an env agree on reset_now but the
+// lanes of a warp do not, so nothing in the reset branches exchanges across lanes: each lane loads the columns it needs.
 // ---------------------------------------------------------------------------------------------
-template <bool FUSED, typename ActT, int MINB, bool EXACT>
+template <bool FUSED, typename ActT, int MINB, bool EXACT, bool STARTS = false>
 __global__ void __launch_bounds__(kBlock, MINB)
 env_step_kernel(const SatEnvState st, const ActT* __restrict__ pa, const ActT* __restrict__ ea,
                 const int32_t* __restrict__ count_override, float* __restrict__ obs_f32,
@@ -338,10 +353,23 @@ env_step_kernel(const SatEnvState st, const ActT* __restrict__ pa, const ActT* _
     const int rows = (int)(rem < kEnvsPerBlock ? rem : kEnvsPerBlock);
     {
         double Po[3], Pvo[3], Eo[3], Evo[3];
+        if (STARTS) {
 #pragma unroll
-        for (int k = 0; k < 3; ++k) {
-            Po[k] = reset_now ? p.reset_p[k] : P[k];  Pvo[k] = reset_now ? 0.0 : Pv[k];
-            Eo[k] = reset_now ? p.reset_e[k] : E[k];  Evo[k] = reset_now ? 0.0 : Ev[k];
+            for (int k = 0; k < 3; ++k) { Po[k] = P[k]; Pvo[k] = Pv[k]; Eo[k] = E[k]; Evo[k] = Ev[k]; }
+            if (reset_now) {
+                const double* __restrict__ Sst = S + SAT_COL_START * ld;
+#pragma unroll
+                for (int k = 0; k < 3; ++k) {
+                    Po[k] = Sst[(SAT_COL_P + k) * ld + e];  Pvo[k] = Sst[(SAT_COL_PV + k) * ld + e];
+                    Eo[k] = Sst[(SAT_COL_E + k) * ld + e];  Evo[k] = Sst[(SAT_COL_EV + k) * ld + e];
+                }
+            }
+        } else {
+#pragma unroll
+            for (int k = 0; k < 3; ++k) {
+                Po[k] = reset_now ? p.reset_p[k] : P[k];  Pvo[k] = reset_now ? 0.0 : Pv[k];
+                Eo[k] = reset_now ? p.reset_e[k] : E[k];  Evo[k] = reset_now ? 0.0 : Ev[k];
+            }
         }
         if (craft == 0) {
 #pragma unroll
@@ -436,7 +464,16 @@ env_step_kernel(const SatEnvState st, const ActT* __restrict__ pa, const ActT* _
 
     // ---------------- auto reset (environment.py:66-79; fuel/dis/dangerous_zone persist, Q2)
     int int_state_new = 0, count_store = count_new;
-    if (reset_now) {
+    if (STARTS) {
+        // reset to the env's start: the lane's own craft from the start columns (re-read rather than kept live across
+        // the danger-zone solve). Starts are floats, so no int64 truncation follows (int_state = 0).
+        if (reset_now) {
+            const double* __restrict__ Sst = S + (SAT_COL_START + craft * 6) * ld;
+#pragma unroll
+            for (int k = 0; k < 3; ++k) { L.r[k] = Sst[k * ld + e]; L.v[k] = Sst[(3 + k) * ld + e]; }
+            count_store = 0;
+        }
+    } else if (reset_now) {
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
             P[k] = p.reset_p[k]; E[k] = p.reset_e[k]; Pv[k] = 0.0; Ev[k] = 0.0;
@@ -685,6 +722,54 @@ __global__ void env_init_kernel(const SatEnvState st, double fuel_c, double fuel
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// per-env start states (SAT_STATE_COLS_STARTS-column buffers): reset to the start columns, and the draw of the next starts
+// ---------------------------------------------------------------------------------------------
+// reset() to the start: kinematics from columns SAT_COL_START..+11, count = 0, int_state = 0; fuel / dis / dangerous_zone /
+// the discounted return persist, as in env_init_kernel's reset form
+__global__ void env_reset_starts_kernel(const SatEnvState st, const uint8_t* __restrict__ mask) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= st.n) return;
+    if (mask && !mask[e]) return;
+    const int64_t ld = st.ld;
+#pragma unroll
+    for (int c = 0; c < 12; ++c) st.state[c * ld + e] = st.state[(SAT_COL_START + c) * ld + e];
+    st.istate[SAT_ICOL_INTSTATE * ld + e] = 0;
+    st.istate[SAT_ICOL_COUNT * ld + e] = 0;
+}
+
+struct StartBox { double lo[12], hi[12]; };
+
+// Uniform draw in the box, keyed by (seed, global env id, draw index) only, so that a sharded batch and a resumed run
+// draw the same starts. Philox4x32-10 with key (seed_lo, seed_hi ^ "SCN1") - never the actor noise's key for the same
+// seed - and counter (g_lo, g_hi, draw, j): block j gives columns 2j (from c0:c1) and 2j + 1 (from c2:c3), each a 53-bit
+// uniform u in [0, 1). Value lo + (hi - lo) * u with each operation rounded (-fmad=false), capped at hi; lo where lo == hi.
+__global__ void env_draw_starts_kernel(const SatEnvState st, const uint8_t* __restrict__ mask, const StartBox box,
+                                       uint64_t seed, uint32_t draw, int64_t row_offset) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= st.n) return;
+    if (mask && !mask[e]) return;
+    const int64_t ld = st.ld;
+    const uint64_t g = (uint64_t)(row_offset + e);
+    const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32) ^ 0x53434E31u;
+    double* __restrict__ out = st.state + SAT_COL_START * ld + e;
+#pragma unroll
+    for (int j = 0; j < 6; ++j) {
+        uint32_t c[4] = {(uint32_t)g, (uint32_t)(g >> 32), draw, (uint32_t)j};
+        philox4x32_10(c, k0, k1);
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+            const int col = 2 * j + h;
+            const uint64_t bits = (((uint64_t)c[2 * h] << 32) | c[2 * h + 1]) >> 11;
+            const double u = (double)bits * 0x1p-53;
+            const double lo = box.lo[col], hi = box.hi[col];
+            double v = __dadd_rn(lo, __dmul_rn(__dsub_rn(hi, lo), u));
+            v = v > hi ? hi : v;
+            out[col * ld] = lo < hi ? v : lo;
+        }
+    }
+}
+
 __global__ void env_observe_kernel(const SatEnvState st, float* __restrict__ obs_f32, double* __restrict__ obs_f64) {
     // one thread per (env, obs element): reads are column-coalesced per element class, writes fully coalesced
     const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -835,6 +920,33 @@ int sat_env_reset(const SatEnvState* st, const uint8_t* mask, const SatEnvParams
     return launch_status();
 }
 
+int sat_env_draw_starts(const SatEnvState* st, const uint8_t* mask, const double* lo_host, const double* hi_host,
+                        uint64_t seed, uint32_t draw, int64_t row_offset, void* stream) {
+    int rc = check_state(st);
+    if (rc) return rc;
+    if (!lo_host || !hi_host) return SAT_ERR_NULL;
+    if (row_offset < 0) return SAT_ERR_SIZE;
+    StartBox box;
+    for (int c = 0; c < 12; ++c) {
+        const double lo = lo_host[c], hi = hi_host[c];
+        if (!std::isfinite(lo) || !std::isfinite(hi) || !(lo <= hi) || !std::isfinite(hi - lo)) return SAT_ERR_SIZE;
+        box.lo[c] = lo; box.hi[c] = hi;
+    }
+    const int threads = 256;
+    const unsigned blocks = (unsigned)((st->n + threads - 1) / threads);
+    env_draw_starts_kernel<<<blocks, threads, 0, (cudaStream_t)stream>>>(*st, mask, box, seed, draw, row_offset);
+    return launch_status();
+}
+
+int sat_env_reset_starts(const SatEnvState* st, const uint8_t* mask, void* stream) {
+    int rc = check_state(st);
+    if (rc) return rc;
+    const int threads = 256;
+    const unsigned blocks = (unsigned)((st->n + threads - 1) / threads);
+    env_reset_starts_kernel<<<blocks, threads, 0, (cudaStream_t)stream>>>(*st, mask);
+    return launch_status();
+}
+
 int sat_env_observe_norm(const SatEnvState* st, const double* obs_stats, float* obs_f32, void* stream) {
     int rc = check_state(st);
     if (rc) return rc;
@@ -882,11 +994,18 @@ int env_step_impl(const SatEnvState* st, const void* pa, const void* ea, const i
     double* dis_prev = ws ? (double*)(ws + ws_disprev_offset()) : nullptr;
     double* partials = want_stats ? (double*)(ws + ws_partials_offset(n)) : nullptr;
     if (ev) cudaEventRecord(ev[0], s);
-    // exact host-libm arithmetic in the danger-zone path (default) or libdevice (SatEnvParams.fast_libm)
+    // exact host-libm arithmetic in the danger-zone path (default) or libdevice (SatEnvParams.fast_libm); resets to the
+    // reference's literals or (auto_reset == SAT_RESET_STARTS) to each env's start columns
+    const bool starts = p->auto_reset == SAT_RESET_STARTS;
 #define SAT_LAUNCH_FINISH(FUSED, T, ...)                                                                                   \
     do {                                                                                                                   \
-        if (p->fast_libm) env_step_kernel<FUSED, T, kFinishMinBlocks, false><<<(unsigned)nblocks, kBlock, 0, s>>>(__VA_ARGS__); \
-        else env_step_kernel<FUSED, T, kFinishMinBlocks, true><<<(unsigned)nblocks, kBlock, 0, s>>>(__VA_ARGS__);          \
+        if (starts) {                                                                                                      \
+            if (p->fast_libm) env_step_kernel<FUSED, T, kFinishMinBlocks, false, true><<<(unsigned)nblocks, kBlock, 0, s>>>(__VA_ARGS__); \
+            else env_step_kernel<FUSED, T, kFinishMinBlocks, true, true><<<(unsigned)nblocks, kBlock, 0, s>>>(__VA_ARGS__); \
+        } else {                                                                                                           \
+            if (p->fast_libm) env_step_kernel<FUSED, T, kFinishMinBlocks, false><<<(unsigned)nblocks, kBlock, 0, s>>>(__VA_ARGS__); \
+            else env_step_kernel<FUSED, T, kFinishMinBlocks, true><<<(unsigned)nblocks, kBlock, 0, s>>>(__VA_ARGS__);      \
+        }                                                                                                                  \
     } while (0)
     if (p->mode == SAT_MODE_CW) {
         // one fused kernel: the propagation is a 6x6 product
@@ -902,8 +1021,12 @@ int env_step_impl(const SatEnvState* st, const void* pa, const void* ea, const i
         const int64_t fblocks = (2 * n + kFrontBlock - 1) / kFrontBlock;
         if (obs_early && (count_override || p->action_dtype != SAT_ACT_F32 || !pa_copy || !ea_copy)) return SAT_ERR_MODE;
         if (obs_early) {
-            env_front_rk4_kernel<float, true><<<(unsigned)fblocks, kFrontBlock, 0, s>>>(*st, (const float*)pa, (const float*)ea,
-                                                                                       dis_prev, obs_early, pa_copy, ea_copy, *p);
+            if (starts)
+                env_front_rk4_kernel<float, true, true><<<(unsigned)fblocks, kFrontBlock, 0, s>>>(
+                    *st, (const float*)pa, (const float*)ea, dis_prev, obs_early, pa_copy, ea_copy, *p);
+            else
+                env_front_rk4_kernel<float, true><<<(unsigned)fblocks, kFrontBlock, 0, s>>>(*st, (const float*)pa, (const float*)ea,
+                                                                                           dis_prev, obs_early, pa_copy, ea_copy, *p);
             if (front_done) cudaEventRecord(front_done, s);
             SAT_LAUNCH_FINISH(false, float, *st, pa_copy, ea_copy,
                 count_override, obs_f32, obs_f64, term_obs_f64, reward, done, dis_prev, partials, ticket, *p);

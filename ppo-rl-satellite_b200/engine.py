@@ -137,6 +137,13 @@ class EnvBatch:
     mode "cw": the env as shipped (CW STM, environment.py:117-121) -> bit-level parity target.
     mode "rk4": propagation by `substeps` RK4 steps of size h of the inertial two-body+J2 ODE
     (north-star production path; relative<->inertial by the reference's translation, environment.py:334-343).
+
+    start_box=(lo, hi), two length-12 sequences over (P, Pv, E, Ev) in the CW frame (metres, m/s): starts mode. Every env
+    owns a start, drawn on the device uniformly in lo <= x <= hi (lo == hi fixes a column) and keyed by (start_seed,
+    row_offset + env index, draw index) only, so a sharded batch or a resumed run draws the same starts. Every reset of an
+    env, manual or automatic, puts its kinematics at its start (count 0, int_state 0; fuel / dis / dangerous_zone persist)
+    and then draws its next one. `starts` is the [12, n] view of the next starts. start_box=None: the reference's reset
+    literals for every env.
     """
 
     def __init__(self, n: int, mode: str = "cw", flag: int = 0, d_capture: float = 100000.0,
@@ -144,13 +151,18 @@ class EnvBatch:
                  max_episode_steps: int = 1000, auto_reset: bool = True, substeps: int = 100, h: float = 1.0,
                  j2: float = J2, gamma: float = 0.99, skip_danger_zone: bool = False, t_step: float = 100.0,
                  fast_libm: bool = False,
-                 stm: np.ndarray | None = None, device="cuda"):
+                 stm: np.ndarray | None = None, device="cuda", start_box=None, start_seed: int = 0, row_offset: int = 0):
         torch = L.require_cuda()
         self.torch = torch
         self.lib = L.load()
         self.n = int(n)
         self.device = torch.device(device)
-        self.state, self._state_buf = alloc_soa(L.SAT_STATE_COLS, self.n, torch.float64, self.device)
+        self.start_box = None if start_box is None else _start_box(start_box)
+        self.start_seed, self.row_offset, self.start_draws = int(start_seed) & (2 ** 64 - 1), int(row_offset), 0
+        if self.row_offset < 0:
+            raise L.SatError("row_offset must be >= 0")
+        cols = L.SAT_STATE_COLS if self.start_box is None else L.SAT_STATE_COLS_STARTS
+        self.state, self._state_buf = alloc_soa(cols, self.n, torch.float64, self.device)
         self.istate, self._istate_buf = alloc_soa(L.SAT_ISTATE_COLS, self.n, torch.int32, self.device)
         self.ld = self._state_buf.shape[1]
         self.st = L.SatEnvState(self._state_buf.data_ptr(), self._istate_buf.data_ptr(), self.n, self.ld)
@@ -158,7 +170,7 @@ class EnvBatch:
         p.mode = {"cw": L.MODE_CW, "rk4": L.MODE_RK4}[mode]
         p.flag = int(flag)
         p.max_episode_steps = int(max_episode_steps)
-        p.auto_reset = int(bool(auto_reset))
+        p.auto_reset = (1 if self.start_box is None else L.RESET_STARTS) if auto_reset else 0
         p.substeps = int(substeps)
         p.skip_danger_zone = int(bool(skip_danger_zone))
         p.fast_libm = int(bool(fast_libm))        # False: exact host-libm arithmetic in the danger-zone count (bit parity)
@@ -186,17 +198,49 @@ class EnvBatch:
         self.params.d_capture = float(v)
 
     def init(self):
-        """constructor state + reset() (environment.py:26-62, 66-79)."""
+        """constructor state + reset() (environment.py:26-62, 66-79). Starts mode: then every env's first start is drawn,
+        the envs are reset to it, and every env's next start is drawn."""
         L.guard_device(self.device)
         L.check(self.lib.sat_env_init(C.byref(self.st), self._fuel0[0], self._fuel0[1], C.byref(self.params),
                                       L.stream_ptr()), "sat_env_init")
+        if self.start_box is not None:
+            self.draw_starts()
+            L.check(self.lib.sat_env_reset_starts(C.byref(self.st), None, L.stream_ptr()), "sat_env_reset_starts")
+            self.draw_starts()
 
     def reset(self, mask=None, flag=None):
-        """reset(Flag) for the masked envs (uint8 CUDA tensor) or all; fuel/dis/dangerous_zone persist (Q2)."""
+        """reset(Flag) for the masked envs (uint8 CUDA tensor) or all; fuel/dis/dangerous_zone persist (Q2).
+        Starts mode: the masked envs go to their starts (count 0, int_state 0), then their next starts are drawn."""
         if flag is not None:
             self.params.flag = int(flag)
+        if self.start_box is not None:
+            L.check(self.lib.sat_env_reset_starts(C.byref(self.st), L.ptr(mask), L.stream_ptr()), "sat_env_reset_starts")
+            self.draw_starts(mask)
+            return
         L.check(self.lib.sat_env_reset(C.byref(self.st), L.ptr(mask), C.byref(self.params), L.stream_ptr()),
                 "sat_env_reset")
+
+    def draw_starts(self, mask=None):
+        """draw the next start of the masked envs (uint8 CUDA tensor; None = all) into the start columns; one draw index
+        (start_draws) per call"""
+        if self.start_box is None:
+            raise L.SatError("draw_starts needs a batch built with start_box")
+        L.guard_device(self.device)
+        lo, hi = self.start_box
+        L.check(self.lib.sat_env_draw_starts(C.byref(self.st), L.ptr(mask), (C.c_double * 12)(*lo), (C.c_double * 12)(*hi),
+                                             self.start_seed, self.start_draws & 0xFFFFFFFF, self.row_offset,
+                                             L.stream_ptr()), "sat_env_draw_starts")
+        self.start_draws += 1
+
+    @property
+    def starts(self):
+        """[12, n] view of every env's next start (columns P, Pv, E, Ev); None without start_box"""
+        return None if self.start_box is None else self.state[L.COL_START:L.COL_START + 12]
+
+    def _redraw_after_step(self, done):
+        # the step reset its finished envs to their starts (same launch); they now need their next ones
+        if self.start_box is not None and self.params.auto_reset == L.RESET_STARTS:
+            self.draw_starts(done)
 
     def observe(self, dtype=None):
         torch = self.torch
@@ -224,6 +268,7 @@ class EnvBatch:
                                       L.ptr(ret_stats.buf) if ret_stats is not None else None,
                                       L.ptr(ret_std_out), self.workspace.data_ptr(), C.byref(self.params),
                                       L.stream_ptr()), "sat_env_step")
+        self._redraw_after_step(done)
         return reward, done
 
     def step_timed(self, pa, ea, reward=None, done=None, obs_stats: RunningStats | None = None,
@@ -232,13 +277,14 @@ class EnvBatch:
         between the launches on the launching stream (bench.py's per-kernel roofline)."""
         self.params.action_dtype = L.ACT_F32 if pa.dtype == self.torch.float32 else L.ACT_F64
         ms = (C.c_float * 3)()
+        done = self.done if done is None else done
         L.check(self.lib.sat_env_step_timed(C.byref(self.st), L.ptr(pa), L.ptr(ea), None, None, None, None,
-                                            L.ptr(self.reward if reward is None else reward),
-                                            L.ptr(self.done if done is None else done),
+                                            L.ptr(self.reward if reward is None else reward), L.ptr(done),
                                             L.ptr(obs_stats.buf) if obs_stats is not None else None,
                                             L.ptr(ret_stats.buf) if ret_stats is not None else None, None,
                                             self.workspace.data_ptr(), C.byref(self.params), L.stream_ptr(), ms),
                 "sat_env_step_timed")
+        self._redraw_after_step(done)
         return float(ms[0]), float(ms[1]), float(ms[2])
 
     # -- host-buffer form: the reference-facing call with numpy in / numpy out (e2e path)
@@ -285,6 +331,9 @@ class EnvBatch:
                                            hb["dio"].data_ptr(), C.byref(self.params), L.stream_ptr(),
                                            hb["streams"][0].cuda_stream, chunks),
                 "sat_env_step_host")
+        if self.start_box is not None and self.params.auto_reset == L.RESET_STARTS:
+            self.done.copy_(hb["done"])                      # the step synchronised: done_h is final
+            self._redraw_after_step(self.done)
         return obs_h, rew_h, done_h
 
     def step_host_single(self, pa_np: np.ndarray, ea_np: np.ndarray):
@@ -304,12 +353,20 @@ class EnvBatch:
         p = self.params
         return {"n": self.n, "mode": self.mode, "state": self.state.detach().cpu().clone(),
                 "istate": self.istate.detach().cpu().clone(),
+                "start_box": self.start_box, "start_seed": self.start_seed, "row_offset": self.row_offset,
+                "start_draws": self.start_draws,
                 "params": {k: (list(getattr(p, k)) if hasattr(getattr(p, k), "__len__") else getattr(p, k))
                            for k, _t in p._fields_}}
 
     def load_state_dict(self, sd):
         if int(sd["n"]) != self.n or sd["mode"] != self.mode:
             raise L.SatError("checkpoint is for a different batch size / propagation mode")
+        if (sd.get("start_box") is None) != (self.start_box is None):
+            raise L.SatError("checkpoint is for a batch %s start_box" % ("without" if self.start_box is not None else "with"))
+        if self.start_box is not None:
+            self.start_box = _start_box(sd["start_box"])
+            self.start_seed, self.row_offset = int(sd["start_seed"]), int(sd["row_offset"])
+            self.start_draws = int(sd["start_draws"])
         self.state.copy_(sd["state"].to(self.device))
         self.istate.copy_(sd["istate"].to(self.device))
         for k, v in sd["params"].items():
@@ -356,6 +413,21 @@ class EnvBatch:
     @property
     def err(self):
         return self.istate[L.ICOL_ERR]
+
+
+def _start_box(box):
+    """(lo, hi) -> two 12-tuples of floats, lo <= hi, all finite"""
+    try:
+        lo, hi = box
+        lo, hi = tuple(float(x) for x in np.asarray(lo, dtype=np.float64).ravel()), \
+            tuple(float(x) for x in np.asarray(hi, dtype=np.float64).ravel())
+    except (TypeError, ValueError) as exc:
+        raise L.SatError("start_box must be (lo, hi), two sequences of 12 numbers") from exc
+    if len(lo) != 12 or len(hi) != 12:
+        raise L.SatError("start_box must be (lo, hi), two sequences of 12 numbers (P, Pv, E, Ev)")
+    if not all(math.isfinite(a) and math.isfinite(b) and a <= b and math.isfinite(b - a) for a, b in zip(lo, hi)):
+        raise L.SatError("start_box needs finite bounds with lo <= hi")
+    return lo, hi
 
 
 def danger_zone_count(rv, dv, u=MU_M, debug=False):

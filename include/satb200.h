@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define SATB200_ABI_VERSION 1
+#define SATB200_ABI_VERSION 2
 
 #define SAT_OK          0
 #define SAT_ERR_NULL   -1   /* required pointer is NULL */
@@ -180,16 +180,18 @@ int sat_fsolve_pfai(const double* dvm, const double* theta, const double* v1x, c
 #define SAT_LIBM_SINCOS_C 6
 int sat_libm_eval(int fn, const double* x, double* y, int64_t n, void* stream);
 
-/* host-buffer form of step(): actions from (pinned) host memory, obs_f32/reward/done to host memory, synchronised
- * before returning. d_io is a caller-provided device staging buffer of sat_env_step_host_bytes(n) bytes.
- * With aux_stream != NULL and chunks > 1 (<= 16) the batch is cut into env ranges that alternate between `stream` and
- * `aux_stream`, so the H2D copies, the kernels and the D2H copies of different ranges overlap.
- * chunks == 0 selects the zero-copy form: when all five host buffers are pinned (UVA-mapped) they are passed to the
- * kernels directly and results stream to host memory while the kernels run (falls back to staged copies otherwise). */
+/* host-buffer form of step(): fp32 actions from host memory, obs_f32/reward/done to host memory, synchronised before
+ * returning. d_io is a caller-provided device buffer of sat_env_step_host_bytes(n) bytes. The inputs select the form:
+ *   - all five host buffers pinned (UVA-mapped), rk4 mode and aux_stream != NULL: kernel A reads the actions from host
+ *     memory and writes the next observation to d_io, from where a copy engine moves it to obs_host on aux_stream while
+ *     kernel B runs on `stream` and writes reward / done straight to host memory;
+ *   - all five pinned, any other case (cw mode, or aux_stream == NULL): zero-copy on `stream`, the kernels read the
+ *     actions from and write the results to the host buffers directly;
+ *   - otherwise (pageable memory): staged copies on `stream`: H2D of the actions to d_io, the step, D2H of the results. */
 int64_t sat_env_step_host_bytes(int64_t n);
 int sat_env_step_host(const SatEnvState* st, const float* pa_host, const float* ea_host,
                       float* obs_host, double* reward_host, uint8_t* done_host, void* d_io,
-                      const SatEnvParams* p, void* stream, void* aux_stream, int chunks);
+                      const SatEnvParams* p, void* stream, void* aux_stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Normalisation. Replaces RunningMeanStd.update / Normalization.__call__ (normalization.py:19-43)

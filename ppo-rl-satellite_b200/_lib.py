@@ -116,7 +116,7 @@ SIGNATURES = {
     "sat_fsolve_pfai": (C.c_int, [_P, _P, _P, _P, _P, _P, _I64, _D, _P, _P, _P]),
     "sat_libm_eval": (C.c_int, [_I32, _P, _P, _I64, _P]),
     "sat_env_step_host_bytes": (_I64, [_I64]),
-    "sat_env_step_host": (C.c_int, [C.POINTER(SatEnvState), _P, _P, _P, _P, _P, _P, C.POINTER(SatEnvParams), _P, _P, _I32]),
+    "sat_env_step_host": (C.c_int, [C.POINTER(SatEnvState), _P, _P, _P, _P, _P, _P, C.POINTER(SatEnvParams), _P, _P]),
     "sat_norm_update": (C.c_int, [_P, _P, _I64, _I32, _I32, _P, _P, _P, _P]),
     "sat_actor_pack": (C.c_int, [C.POINTER(SatActorWeights), _P, _P]),
     "sat_actor_sample": (C.c_int, [C.POINTER(SatActorWeights), _P, C.POINTER(SatEnvState), _P, _I64, _I64,
@@ -154,7 +154,7 @@ def load():
             fn = getattr(lib, name)     # AttributeError if the .so does not export a declared symbol
             fn.restype = res
             fn.argtypes = args
-        if lib.sat_abi_version() != 1:
+        if lib.sat_abi_version() != 2:
             raise ImportError("libsatb200.so ABI version mismatch")
         _lib = lib
     return _lib

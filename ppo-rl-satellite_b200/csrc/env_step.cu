@@ -1054,6 +1054,30 @@ int env_step_impl(const SatEnvState* st, const void* pa, const void* ea, const i
     if (ev) cudaEventRecord(ev[3], s);
     return rc;
 }
+
+// d_io of sat_env_step_host: pa | ea (fp32 [n][3] each) | obs fp32 [n][18] | reward fp64 [n] | done u8 [n] | the env
+// step's workspace, each region 256-byte aligned; `bytes` is the size of the whole buffer
+struct HostIo {
+    float *pa, *ea, *obs;
+    double* reward;
+    uint8_t* done;
+    void* ws;
+    int64_t bytes;
+};
+inline HostIo host_io_carve(void* d_io, int64_t n) {
+    const uintptr_t base = (uintptr_t)d_io;
+    int64_t off = 0;
+    auto take = [&](int64_t b) { const uintptr_t p = base + (uintptr_t)off; off += (b + 255) / 256 * 256; return p; };
+    HostIo io;
+    io.pa = (float*)take(n * 12);
+    io.ea = (float*)take(n * 12);
+    io.obs = (float*)take(n * 72);
+    io.reward = (double*)take(n * 8);
+    io.done = (uint8_t*)take(n);
+    io.ws = (void*)(base + (uintptr_t)off);
+    io.bytes = off + sat_workspace_bytes(n);
+    return io;
+}
 }  // namespace
 
 extern "C" {
@@ -1113,134 +1137,67 @@ int sat_libm_eval(int fn, const double* x, double* y, int64_t n, void* stream) {
     return launch_status();
 }
 
-int64_t sat_env_step_host_bytes(int64_t n) {
-    if (n <= 0) return 0;
-    // pa | ea (fp32 [n][3] each) | obs fp32 [n][18] | reward fp64 [n] | done u8 [n], each 256-byte aligned
-    auto al = [](int64_t b) { return (b + 255) / 256 * 256; };
-    // + one workspace per env range for up to 16 ranges
-    return al(n * 12) * 2 + al(n * 72) + al(n * 8) + al(n) + sat_workspace_bytes(n) + 16 * sat_workspace_bytes(64) + 16 * 4096;
-}
+int64_t sat_env_step_host_bytes(int64_t n) { return n > 0 ? host_io_carve(nullptr, n).bytes : 0; }
 
 int sat_env_step_host(const SatEnvState* st, const float* pa_host, const float* ea_host,
                       float* obs_host, double* reward_host, uint8_t* done_host, void* d_io,
-                      const SatEnvParams* p, void* stream, void* aux_stream, int chunks) {
+                      const SatEnvParams* p, void* stream, void* aux_stream) {
     int rc = check_state(st);
     if (rc) return rc;
     if (!pa_host || !ea_host || !obs_host || !reward_host || !done_host || !d_io || !p) return SAT_ERR_NULL;
     cudaStream_t s0 = (cudaStream_t)stream, s1 = (cudaStream_t)aux_stream;
     const int64_t n = st->n;
-    auto al = [](int64_t b) { return (b + 255) / 256 * 256; };
-    char* base = (char*)d_io;
-    float* d_pa = (float*)base;
-    float* d_ea = (float*)(base + al(n * 12));
-    float* d_obs = (float*)(base + 2 * al(n * 12));
-    double* d_rew = (double*)(base + 2 * al(n * 12) + al(n * 72));
-    uint8_t* d_done = (uint8_t*)(base + 2 * al(n * 12) + al(n * 72) + al(n * 8));
-    char* d_ws = base + 2 * al(n * 12) + al(n * 72) + al(n * 8) + al(n);
+    const HostIo io = host_io_carve(d_io, n);
     SatEnvParams q = *p;
     q.action_dtype = SAT_ACT_F32;
-    // error exits after work was forked onto the second stream: join both streams and release the fork event first
-    cudaEvent_t fork = nullptr;
-    auto leave = [&](int code) {
-        if (fork) {
-            cudaStreamSynchronize(s0);
-            if (s1) cudaStreamSynchronize(s1);
-            cudaEventDestroy(fork);
-            fork = nullptr;
-        }
-        return code;
-    };
-    if (chunks <= 0) {
-        // zero-copy form: pinned (UVA-mapped) host buffers are handed to the kernels directly: the action reads and the
-        // observation / reward / done stores cross PCIe from inside the kernels. With chunks < 0 the batch is additionally
-        // cut into -chunks env ranges alternating between the two streams. In rk4 mode with one range (chunks == 0) the
-        // observation instead leaves through a copy engine underneath kernel B (below).
-        cudaPointerAttributes at;
-        bool ok = true;
-        const void* ptrs[5] = {pa_host, ea_host, obs_host, reward_host, done_host};
-        void* dev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-        for (int i = 0; i < 5 && ok; ++i) {
-            ok = cudaPointerGetAttributes(&at, ptrs[i]) == cudaSuccess && at.type == cudaMemoryTypeHost && at.devicePointer != nullptr;
-            dev[i] = at.devicePointer;
-        }
-        cudaGetLastError();
-        int ranges = (chunks < 0 && s1) ? -chunks : 1;
-        if (ranges > 16) ranges = 16;
-        if (ok && ranges == 1 && s1 && q.mode == SAT_MODE_RK4) {
-            // rk4 mode, one range (the default): kernel A reads the actions from host memory (zero-copy), leaves a copy in
-            // device memory for kernel B and writes the step's next observation (88 % of the output bytes) to device
-            // memory; a copy engine moves the observation to the host on the second stream while kernel B (danger zone,
-            // reward) runs; kernel B writes reward / done straight to host memory. Kernel B must not READ host memory
-            // here: PCIe read requests may not pass the copy's posted writes, which stalled it by ~50 us.
-            // Measured at 65 536 envs: 241 us/step (all zero-copy: 287; two zero-copy ranges: 266; staged: 306).
-            static thread_local cudaEvent_t front_ev[64] = {};   // one event per device ordinal (events belong to a device)
-            int devid = 0;
-            cudaError_t ce0;
-            if ((ce0 = cudaGetDevice(&devid)) != cudaSuccess) return (int)ce0;
-            if (devid < 0 || devid >= 64) return SAT_ERR_SIZE;
-            cudaEvent_t& fe = front_ev[devid];
-            if (!fe && (ce0 = cudaEventCreateWithFlags(&fe, cudaEventDisableTiming)) != cudaSuccess) return (int)ce0;
-            rc = env_step_impl(st, dev[0], dev[1], nullptr, nullptr, nullptr, nullptr, (double*)dev[3], (uint8_t*)dev[4],
-                               nullptr, nullptr, nullptr, d_ws, &q, (void*)s0, nullptr, d_obs, fe, d_pa, d_ea);
-            if (rc) return rc;
-            if ((ce0 = cudaStreamWaitEvent(s1, fe, 0)) != cudaSuccess) return (int)ce0;
-            if ((ce0 = cudaMemcpyAsync(obs_host, d_obs, (size_t)n * 72, cudaMemcpyDeviceToHost, s1)) != cudaSuccess) return (int)ce0;
-            if ((ce0 = cudaStreamSynchronize(s0)) != cudaSuccess) return (int)ce0;
-            if ((ce0 = cudaStreamSynchronize(s1)) != cudaSuccess) return (int)ce0;
-            return SAT_OK;
-        }
-        if (ok) {
-            const int64_t per = ((n + ranges - 1) / ranges + 63) / 64 * 64;
-            const int64_t ws_per = sat_workspace_bytes(per);
-            cudaError_t ce0;
-            if (ranges > 1) {
-                if ((ce0 = cudaEventCreateWithFlags(&fork, cudaEventDisableTiming)) != cudaSuccess) return (int)ce0;
-                cudaEventRecord(fork, s0);
-                cudaStreamWaitEvent(s1, fork, 0);
-            }
-            int k = 0;
-            for (int64_t lo = 0; lo < n; lo += per, ++k) {
-                const int64_t m = (n - lo < per) ? n - lo : per;
-                SatEnvState sub = {st->state + lo, st->istate + lo, m, st->ld};
-                rc = sat_env_step(&sub, (const float*)dev[0] + lo * 3, (const float*)dev[1] + lo * 3, nullptr,
-                                  (float*)dev[2] + lo * 18, nullptr, nullptr, (double*)dev[3] + lo, (uint8_t*)dev[4] + lo,
-                                  nullptr, nullptr, nullptr, d_ws + (int64_t)k * ws_per, &q, (void*)((k & 1) ? s1 : s0));
-                if (rc) return leave(rc);
-            }
-            if ((ce0 = cudaStreamSynchronize(s0)) != cudaSuccess) return leave((int)ce0);
-            if (ranges > 1 && (ce0 = cudaStreamSynchronize(s1)) != cudaSuccess) return leave((int)ce0);
-            return leave(SAT_OK);
-        }
-        chunks = ranges;                                     // pageable memory: staged copies
+    // pinned (UVA-mapped) host buffers can be handed to the kernels directly (zero-copy)
+    cudaPointerAttributes at;
+    bool mapped = true;
+    const void* ptrs[5] = {pa_host, ea_host, obs_host, reward_host, done_host};
+    void* dev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+    for (int i = 0; i < 5 && mapped; ++i) {
+        mapped = cudaPointerGetAttributes(&at, ptrs[i]) == cudaSuccess && at.type == cudaMemoryTypeHost && at.devicePointer != nullptr;
+        dev[i] = at.devicePointer;
     }
-    // env ranges of a multiple of 64 envs (keeps every sub-column 16-byte aligned), alternating between the two
-    // streams so that the H2D of the actions, the kernels and the D2H of the results of different ranges overlap
-    if (chunks < 1 || !s1) chunks = 1;
-    int64_t per = ((n + chunks - 1) / chunks + 63) / 64 * 64;
+    cudaGetLastError();
     cudaError_t ce;
-    if (chunks > 1) {
-        if ((ce = cudaEventCreateWithFlags(&fork, cudaEventDisableTiming)) != cudaSuccess) return (int)ce;
-        cudaEventRecord(fork, s0);
-        cudaStreamWaitEvent(s1, fork, 0);
+    if (mapped && s1 && q.mode == SAT_MODE_RK4) {
+        // kernel A reads the actions from host memory (zero-copy), leaves a copy in device memory for kernel B and writes
+        // the step's next observation (88 % of the output bytes) to device memory; a copy engine moves the observation to
+        // the host on the second stream while kernel B (danger zone, reward) runs; kernel B writes reward / done straight
+        // to host memory. Kernel B must not READ host memory here: PCIe read requests may not pass the copy's posted
+        // writes, which stalled it by ~50 us. Measured at 65 536 envs: 241 us/step (all zero-copy: 287; staged: 333).
+        static thread_local cudaEvent_t front_ev[64] = {};   // one event per device ordinal (events belong to a device)
+        int devid = 0;
+        if ((ce = cudaGetDevice(&devid)) != cudaSuccess) return (int)ce;
+        if (devid < 0 || devid >= 64) return SAT_ERR_SIZE;
+        cudaEvent_t& fe = front_ev[devid];
+        if (!fe && (ce = cudaEventCreateWithFlags(&fe, cudaEventDisableTiming)) != cudaSuccess) return (int)ce;
+        rc = env_step_impl(st, dev[0], dev[1], nullptr, nullptr, nullptr, nullptr, (double*)dev[3], (uint8_t*)dev[4],
+                           nullptr, nullptr, nullptr, io.ws, &q, (void*)s0, nullptr, io.obs, fe, io.pa, io.ea);
+        if (rc) return rc;
+        if ((ce = cudaStreamWaitEvent(s1, fe, 0)) != cudaSuccess) return (int)ce;
+        if ((ce = cudaMemcpyAsync(obs_host, io.obs, (size_t)n * 72, cudaMemcpyDeviceToHost, s1)) != cudaSuccess) return (int)ce;
+        if ((ce = cudaStreamSynchronize(s0)) != cudaSuccess) return (int)ce;
+        return (int)cudaStreamSynchronize(s1);
     }
-    const int64_t ws_per = sat_workspace_bytes(per);
-    int k = 0;
-    for (int64_t lo = 0; lo < n; lo += per, ++k) {
-        const int64_t m = (n - lo < per) ? n - lo : per;
-        cudaStream_t s = (k & 1) ? s1 : s0;
-        SatEnvState sub = {st->state + lo, st->istate + lo, m, st->ld};
-        if ((ce = cudaMemcpyAsync(d_pa + lo * 3, pa_host + lo * 3, m * 12, cudaMemcpyHostToDevice, s)) != cudaSuccess) return leave((int)ce);
-        if ((ce = cudaMemcpyAsync(d_ea + lo * 3, ea_host + lo * 3, m * 12, cudaMemcpyHostToDevice, s)) != cudaSuccess) return leave((int)ce);
-        rc = sat_env_step(&sub, d_pa + lo * 3, d_ea + lo * 3, nullptr, d_obs + lo * 18, nullptr, nullptr, d_rew + lo,
-                          d_done + lo, nullptr, nullptr, nullptr, d_ws + (int64_t)k * ws_per, &q, (void*)s);
-        if (rc) return leave(rc);
-        if ((ce = cudaMemcpyAsync(obs_host + lo * 18, d_obs + lo * 18, m * 72, cudaMemcpyDeviceToHost, s)) != cudaSuccess) return leave((int)ce);
-        if ((ce = cudaMemcpyAsync(reward_host + lo, d_rew + lo, m * 8, cudaMemcpyDeviceToHost, s)) != cudaSuccess) return leave((int)ce);
-        if ((ce = cudaMemcpyAsync(done_host + lo, d_done + lo, m, cudaMemcpyDeviceToHost, s)) != cudaSuccess) return leave((int)ce);
+    if (mapped) {
+        // the action reads and the observation / reward / done stores cross PCIe from inside the kernels
+        rc = sat_env_step(st, dev[0], dev[1], nullptr, (float*)dev[2], nullptr, nullptr, (double*)dev[3], (uint8_t*)dev[4],
+                          nullptr, nullptr, nullptr, io.ws, &q, (void*)s0);
+        if (rc) return rc;
+        return (int)cudaStreamSynchronize(s0);
     }
-    if ((ce = cudaStreamSynchronize(s0)) != cudaSuccess) return leave((int)ce);
-    if (chunks > 1 && (ce = cudaStreamSynchronize(s1)) != cudaSuccess) return leave((int)ce);
-    return leave(SAT_OK);
+    // pageable host memory: staged copies through d_io
+    if ((ce = cudaMemcpyAsync(io.pa, pa_host, (size_t)n * 12, cudaMemcpyHostToDevice, s0)) != cudaSuccess) return (int)ce;
+    if ((ce = cudaMemcpyAsync(io.ea, ea_host, (size_t)n * 12, cudaMemcpyHostToDevice, s0)) != cudaSuccess) return (int)ce;
+    rc = sat_env_step(st, io.pa, io.ea, nullptr, io.obs, nullptr, nullptr, io.reward, io.done, nullptr, nullptr, nullptr, io.ws,
+                      &q, (void*)s0);
+    if (rc) return rc;
+    if ((ce = cudaMemcpyAsync(obs_host, io.obs, (size_t)n * 72, cudaMemcpyDeviceToHost, s0)) != cudaSuccess) return (int)ce;
+    if ((ce = cudaMemcpyAsync(reward_host, io.reward, (size_t)n * 8, cudaMemcpyDeviceToHost, s0)) != cudaSuccess) return (int)ce;
+    if ((ce = cudaMemcpyAsync(done_host, io.done, (size_t)n, cudaMemcpyDeviceToHost, s0)) != cudaSuccess) return (int)ce;
+    return (int)cudaStreamSynchronize(s0);
 }
 
 int sat_norm_update(double* stats, const double* x, int64_t n, int dim, int update,

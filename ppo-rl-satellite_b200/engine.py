@@ -301,44 +301,32 @@ class EnvBatch:
                 rew=torch.empty(n, dtype=torch.float64).pin_memory(),
                 done=torch.empty(n, dtype=torch.uint8).pin_memory(),
                 dio=torch.zeros(self.lib.sat_env_step_host_bytes(n), dtype=torch.uint8, device=self.device),
-                streams=[torch.cuda.Stream(device=self.device)])
+                aux_stream=torch.cuda.Stream(device=self.device))
             hb = self._host
             hb["np"] = tuple(hb[k].numpy() for k in ("pa", "ea", "obs", "rew", "done"))
         return self._host["np"]
 
-    def step_host(self, pa_np: np.ndarray, ea_np: np.ndarray, chunks: int = 0):
-        """step(pa, ea) with HOST arrays in and out: one sat_env_step_host call. chunks <= 0: the pinned host arrays are
-        handed to the kernels directly (UVA zero-copy). chunks = 0 (default): in rk4 mode the propagation kernel also emits
-        the next observation, which a copy engine moves to the host underneath the danger-zone kernel (241 us/step at
-        65 536 envs); -k cuts the batch into k all-zero-copy env ranges on two streams (-2: 266, -4: 291 us/step).
-        With chunks > 1 (staged copies) the batch is cut into env
-        ranges pipelined over two CUDA streams inside the library (H2D of the actions, the env-step kernels and the D2H of
-        obs fp32 / reward / done of different ranges overlap). Measured at 65 536 envs (rk4 mode, PCIe 54 GB/s): chunks
-        {1: 333, 2: 327, 4: 405, 8: 566} us/step -- the latency-bound finish kernel does not shrink linearly with the range,
-        so two ranges is the optimum of the staged form. Returns pinned numpy views (valid until the next call)."""
+    def step_host(self, pa_np: np.ndarray, ea_np: np.ndarray):
+        """step(pa, ea) with HOST arrays in and out: one sat_env_step_host call on the pinned host arrays, which the
+        kernels read and write directly (UVA zero-copy). In rk4 mode the propagation kernel also emits the next
+        observation, which a copy engine moves to the host on a second stream underneath the danger-zone kernel:
+        241 us/step at 65 536 envs on a B200 (DESIGN.md s6c has the forms measured before it). Returns pinned numpy views
+        (valid until the next call)."""
         pa_h, ea_h, obs_h, rew_h, done_h = self.host_buffers()
         hb = self._host
         if pa_np is not pa_h:
             pa_h[...] = pa_np
         if ea_np is not ea_h:
             ea_h[...] = ea_np
-        chunks = int(chunks)
-        chunks = max(-16, chunks) if chunks <= 0 else max(1, min(chunks, 16, self.n // 64 or 1))
-        if chunks < 0 and self.n < 128:
-            chunks = 0
         L.check(self.lib.sat_env_step_host(C.byref(self.st), hb["pa"].data_ptr(), hb["ea"].data_ptr(),
                                            hb["obs"].data_ptr(), hb["rew"].data_ptr(), hb["done"].data_ptr(),
                                            hb["dio"].data_ptr(), C.byref(self.params), L.stream_ptr(),
-                                           hb["streams"][0].cuda_stream, chunks),
+                                           hb["aux_stream"].cuda_stream),
                 "sat_env_step_host")
         if self.start_box is not None and self.params.auto_reset == L.RESET_STARTS:
             self.done.copy_(hb["done"])                      # the step synchronised: done_h is final
             self._redraw_after_step(self.done)
         return obs_h, rew_h, done_h
-
-    def step_host_single(self, pa_np: np.ndarray, ea_np: np.ndarray):
-        """unpipelined form (one env range, one stream)"""
-        return self.step_host(pa_np, ea_np, chunks=1)
 
     @property
     def h2d_bytes_per_step(self):

@@ -38,11 +38,11 @@ def test_header_symbols_are_exported(lib_path):
     assert not extra, f"exported but not declared: {extra}"
 
 
-def test_ctypes_binding_covers_header_and_loads(lib_path):
+def test_ctypes_binding_covers_header_and_checks_abi_version(lib_path):
     from ppo_rl_satellite_b200 import _lib
     assert sorted(_lib.SIGNATURES) == declared_symbols()
     lib = _lib.load()                      # dlopen + symbol lookup, no compute
-    assert lib.sat_abi_version() == 1
+    assert lib.sat_abi_version() == 2
     assert lib.sat_strerror(0) == b"ok" and b"NULL" in lib.sat_strerror(-1)
     assert lib.sat_workspace_bytes(65536) >= 65536 // 32 * 19 * 16
     p = _lib.default_params()

@@ -226,7 +226,7 @@ def test_degenerate_box_reproduces_the_default_batch(golden, eng):
 
 
 @gpu
-def test_rk4_starts_mode_vs_oracle_and_host_forms(oracle, eng):
+def test_rk4_starts_mode_vs_oracle_and_input_selected_host_forms(oracle, eng):
     """rk4 mode: the device step against the oracle's step_rk4 with the auto-reset to the starts emulated (tolerances of
     test_env_rk4_mode_vs_oracle); then every host-buffer form equals the device-resident starts-mode step"""
     n, T, S = 512, 16, 20
@@ -264,18 +264,22 @@ def test_rk4_starts_mode_vs_oracle_and_host_forms(oracle, eng):
     assert diverged.mean() < 0.02, diverged.mean()
     assert resets > n
 
+    from test_gpu_parity import step_host_call
     n = 1500
     hkw = dict(mode="rk4", substeps=5, h=1.0, d_capture=150000.0, max_episode_steps=6, start_box=box(60000.0, 3.0), start_seed=9)
-    for chunks in (0, -2, 1, 2):
+    for form in ("overlapped", "zero-copy", "staged"):
         a, b = eng.EnvBatch(n, **hkw), eng.EnvBatch(n, **hkw)
         obs_d = torch.empty((n, 18), dtype=torch.float32, device="cuda")
         dones = 0
         for t in range(9):
             pa, ea = _actions(rng, n)
             r, d = a.step(torch.from_numpy(pa).cuda(), torch.from_numpy(ea).cuda(), obs_f32=obs_d)
-            o, rh, dh = b.step_host(pa, ea, chunks=chunks)
-            assert np.array_equal(dh, d.cpu().numpy()) and np.array_equal(rh, r.cpu().numpy()), (chunks, t)
-            assert np.array_equal(o, obs_d.cpu().numpy()), (chunks, t)
+            if form == "overlapped":
+                o, rh, dh = b.step_host(pa, ea)
+            else:
+                o, rh, dh = step_host_call(b, pa, ea, pinned=form == "zero-copy")
+            assert np.array_equal(dh, d.cpu().numpy()) and np.array_equal(rh, r.cpu().numpy()), (form, t)
+            assert np.array_equal(o, obs_d.cpu().numpy()), (form, t)
             dones += int(dh.sum())
         assert dones > n
         assert torch.equal(a.state, b.state) and torch.equal(a.istate, b.istate) and a.start_draws == b.start_draws

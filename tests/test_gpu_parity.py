@@ -299,7 +299,25 @@ def test_env_ragged_and_tiny_batches(golden, oracle, eng):
             assert np.array_equal(obs.cpu().numpy(), o_obs.astype(np.float32))
 
 
-def test_env_step_host_buffers(golden, oracle, eng):
+def step_host_call(env, pa, ea, pinned):
+    """one direct sat_env_step_host call without an aux stream, on fresh pinned host buffers (the zero-copy form) or on
+    pageable numpy arrays (the staged form); redraws the starts of the finished envs as EnvBatch.step_host does.
+    Returns (obs, reward, done)."""
+    import ctypes as C
+    from ppo_rl_satellite_b200 import _lib as L
+    n = env.n
+    host = (lambda x: torch.from_numpy(x).pin_memory().numpy()) if pinned else (lambda x: x)
+    bufs = [host(x) for x in (np.ascontiguousarray(pa, np.float32), np.ascontiguousarray(ea, np.float32),
+                              np.empty((n, 18), np.float32), np.empty(n), np.empty(n, np.uint8))]
+    dio = torch.zeros(env.lib.sat_env_step_host_bytes(n), dtype=torch.uint8, device="cuda")
+    L.check(env.lib.sat_env_step_host(C.byref(env.st), *(x.ctypes.data for x in bufs), dio.data_ptr(), C.byref(env.params),
+                                      L.stream_ptr(), None), "sat_env_step_host")
+    env._redraw_after_step(torch.from_numpy(bufs[4]).cuda())
+    return bufs[2], bufs[3], bufs[4]
+
+
+def test_env_step_host_zero_copy_and_staged_vs_oracle(golden, oracle, eng):
+    """cw mode: the zero-copy form (EnvBatch.step_host) and the staged form (pageable arrays) against the oracle"""
     g = golden("env_golden.npz")
     n = 257
     env = eng.EnvBatch(n, mode="cw", d_capture=20000.0, max_episode_steps=7, stm=g["stm100_columns"])
@@ -308,18 +326,19 @@ def test_env_step_host_buffers(golden, oracle, eng):
     for t in range(10):
         pa = rng.uniform(-2, 2, (n, 3)).astype(np.float32)
         ea = rng.uniform(-2, 2, (n, 3)).astype(np.float32)
-        obs, r, d = env.step_host(pa, ea, chunks=(1, 2, 4, 0, -2)[t % 5])                # single-range / pipelined / zero-copy forms
+        obs, r, d = env.step_host(pa, ea) if t % 2 else step_host_call(env, pa, ea, pinned=False)
         o_obs, o_r, o_d = orc.step(pa.astype(np.float64), ea.astype(np.float64))
         assert np.array_equal(d, o_d) and np.array_equal(r, o_r) and np.array_equal(obs, o_obs.astype(np.float32))
 
 
-def test_env_step_host_rk4_forms_equal_device_step(eng):
-    """rk4 mode: every host-buffer form (overlapped observation copy = default, zero-copy ranges, staged) returns exactly
-    what the device-resident step returns, including the observation after an auto reset (captures and time-outs occur)"""
+def test_env_step_host_rk4_input_selected_forms_equal_device_step(eng):
+    """rk4 mode: every host-buffer form (overlapped observation copy through EnvBatch.step_host, zero-copy without an aux
+    stream, staged from pageable arrays) returns exactly what the device-resident step returns, including the observation
+    after an auto reset (captures and time-outs occur)"""
     n = 1500
     rng = np.random.default_rng(11)
     kw = dict(mode="rk4", substeps=5, h=1.0, d_capture=150000.0, max_episode_steps=6)
-    for chunks in (0, -2, -3, 1, 2):
+    for form in ("overlapped", "zero-copy", "staged"):
         a, b = eng.EnvBatch(n, **kw), eng.EnvBatch(n, **kw)
         P0 = np.array([200000.0, 0, 0]) + rng.normal(0, 6e4, (n, 3)); E0 = np.array([18000.0, 0, 0]) + rng.normal(0, 6e4, (n, 3))
         V0 = rng.normal(0, 3.0, (n, 3)); W0 = rng.normal(0, 3.0, (n, 3))
@@ -329,9 +348,12 @@ def test_env_step_host_rk4_forms_equal_device_step(eng):
         for t in range(9):
             pa = rng.uniform(-2, 2, (n, 3)).astype(np.float32); ea = rng.uniform(-2, 2, (n, 3)).astype(np.float32)
             r, d = a.step(torch.from_numpy(pa).cuda(), torch.from_numpy(ea).cuda(), obs_f32=obs_d)
-            obs, rh, dh = b.step_host(pa, ea, chunks=chunks)
-            assert np.array_equal(dh, d.cpu().numpy()) and np.array_equal(rh, r.cpu().numpy())
-            assert np.array_equal(obs, obs_d.cpu().numpy())
+            if form == "overlapped":
+                obs, rh, dh = b.step_host(pa, ea)
+            else:
+                obs, rh, dh = step_host_call(b, pa, ea, pinned=form == "zero-copy")
+            assert np.array_equal(dh, d.cpu().numpy()) and np.array_equal(rh, r.cpu().numpy()), (form, t)
+            assert np.array_equal(obs, obs_d.cpu().numpy()), (form, t)
             dones += int(dh.sum())
         assert dones > n                                       # every env timed out at least once, some were captured
         assert torch.equal(a.state, b.state) and torch.equal(a.istate, b.istate)
@@ -346,6 +368,11 @@ def test_env_argument_errors(eng):
     rc = lib.sat_env_step(C.byref(env.st), a.data_ptr(), a.data_ptr(), None, None, None, None, None, None,
                           None, None, None, None, C.byref(env.params), None)
     assert rc == -1                                         # reward/done missing
+    h = [np.zeros((4, 3), np.float32), np.zeros((4, 3), np.float32), np.zeros((4, 18), np.float32), np.zeros(4), np.zeros(4, np.uint8)]
+    dio = torch.zeros(lib.sat_env_step_host_bytes(4), dtype=torch.uint8, device="cuda")
+    for k in range(5):                                      # each host buffer missing in turn
+        ptrs = [None if i == k else x.ctypes.data for i, x in enumerate(h)]
+        assert lib.sat_env_step_host(C.byref(env.st), *ptrs, dio.data_ptr(), C.byref(env.params), None, None) == -1
     env.params.mode = 7
     rc = lib.sat_env_step(C.byref(env.st), a.data_ptr(), a.data_ptr(), None, None, None, None, env.reward.data_ptr(),
                           env.done.data_ptr(), None, None, None, None, C.byref(env.params), None)

@@ -202,6 +202,39 @@ int sat_norm_update(double* stats, const double* x, int64_t n, int dim, int upda
                     double* x_out_f64, float* x_out_f32, void* workspace, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Statistics shared across ranks. A batch sharded over G ranks keeps one set of running statistics: every rank computes
+ * its per-block (mean, M2) partials, the partials of all ranks are gathered rank-major, and every rank folds all of them
+ * into its own copy of the statistics. The fold is sat_env_step's / sat_norm_update's merge run over a block index that
+ * spans the ranks in rank order, so every rank ends with the same bits.
+ * Bit identity with the union batch: when every rank but the last holds a multiple of the rows per block (64 for the env
+ * step, 128 for sat_norm_partials), rank r's blocks are exactly the union batch's blocks, and the statistics after the
+ * fold are bit-identical to those one sat_env_step / sat_norm_update over the union batch leaves. Otherwise the blocks
+ * straddle ranks differently and the result agrees with the union batch to rounding only (still the same on every rank).
+ * ------------------------------------------------------------------------------------------------ */
+/* bytes of one rank's partials for n rows: dim == 0, the env step's [ceil(n/64)][19][2] doubles (18 observation dims, then
+ * the discounted return); 1 <= dim <= 32, sat_norm_partials' [ceil(n/128)][dim][2]. 0 for n <= 0 or another dim. */
+int64_t sat_stats_partials_bytes(int64_t n, int dim);
+/* sat_env_step with statistics on, except that the per-block partials are written to `partials`
+ * (sat_stats_partials_bytes(n, 0) bytes) instead of being folded; no statistics are touched. workspace:
+ * sat_workspace_bytes(n) bytes; the step zeroes its ticket (first 4 bytes), so it can be passed to sat_stats_fold next. */
+int sat_env_step_partials(const SatEnvState* st, const void* pa, const void* ea, const int32_t* count_override,
+                          float* obs_f32, double* obs_f64, double* term_obs_f64, double* reward, uint8_t* done,
+                          double* partials, void* workspace, const SatEnvParams* p, void* stream);
+/* the partials of a batch x [n][dim] fp64 (1 <= dim <= 32) into `partials` (sat_stats_partials_bytes(n, dim) bytes).
+ * workspace: >= 256 bytes; its ticket (first 4 bytes) is zeroed. */
+int sat_norm_partials(const double* x, int64_t n, int dim, double* partials, void* workspace, void* stream);
+/* Fold the gathered partials of `ranks` ranks into the running statistics. partials: device, rank-major, rank r's block j
+ * at ((r * rank_stride_blocks + j) * dims + d) * 2 (dims = 19 for dim == 0, else dim); rank_rows: device int64 [ranks],
+ * rank r's row count, 0 <= rank_rows[r] <= rank_stride_blocks * rows per block.
+ *   dim == 0: env-step partials into obs_stats (dim 18) / ret_stats (dim 1) / ret_std_out, each nullable, as sat_env_step.
+ *   dim >= 1: sat_norm_partials partials into obs_stats (dim `dim`); ret_stats and ret_std_out must be NULL.
+ * workspace: its first 4 bytes (the ticket) must be 0 on entry and are 0 again on exit; the workspace just given to
+ * sat_env_step_partials / sat_norm_partials on the same stream satisfies this. With ranks == 1 the fold produces the bits
+ * of sat_env_step's / sat_norm_update's own merge. Zero rows in total: the statistics are left unchanged. */
+int sat_stats_fold(const double* partials, int ranks, int64_t rank_stride_blocks, const int64_t* rank_rows, int dim,
+                   double* obs_stats, double* ret_stats, double* ret_std_out, void* workspace, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * K3  fused Gaussian actor. Replaces PPO_continuous.choose_action -> Actor_Gaussian.get_dist/forward
  * (ppo_continuous.py:83-95, 176-189) over n observations: mean = max_action*tanh(W3 tanh(W2 tanh(W1 s+b1)+b2)+b3),
  * a = clamp(mean + exp(log_std)*eps, +-max_action), logp = Normal(mean, std).log_prob(a) per dimension.

@@ -118,6 +118,11 @@ SIGNATURES = {
     "sat_env_step_host_bytes": (_I64, [_I64]),
     "sat_env_step_host": (C.c_int, [C.POINTER(SatEnvState), _P, _P, _P, _P, _P, _P, C.POINTER(SatEnvParams), _P, _P]),
     "sat_norm_update": (C.c_int, [_P, _P, _I64, _I32, _I32, _P, _P, _P, _P]),
+    "sat_stats_partials_bytes": (_I64, [_I64, _I32]),
+    "sat_env_step_partials": (C.c_int, [C.POINTER(SatEnvState), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,
+                                        C.POINTER(SatEnvParams), _P]),
+    "sat_norm_partials": (C.c_int, [_P, _I64, _I32, _P, _P, _P]),
+    "sat_stats_fold": (C.c_int, [_P, _I32, _I64, _P, _I32, _P, _P, _P, _P, _P]),
     "sat_actor_pack": (C.c_int, [C.POINTER(SatActorWeights), _P, _P]),
     "sat_actor_sample": (C.c_int, [C.POINTER(SatActorWeights), _P, C.POINTER(SatEnvState), _P, _I64, _I64,
                                    _U64, _U64, _P, _P, _P, _P, _P, _P, _P]),

@@ -658,26 +658,63 @@ SAT_DEV double block_sum_fixed(double v, double* sm) {
     return t;
 }
 
-__global__ void __launch_bounds__(kMergeThreads)
-stats_merge_kernel(const double* __restrict__ partials, int64_t nblocks, int64_t n_rows, int rows_per_block,
-                   int ndims_in_partials, double* obs_stats, int obs_dim, double* ret_stats, double* ret_std_out,
-                   unsigned int* ticket) {
-    __shared__ double sm[kMergeThreads / 32];
-    const int dim = blockIdx.x;                  // gridDim.x == ndims_in_partials
-    const double N = (double)n_rows;
-    double wsum = 0.0;
-    for (int64_t b = threadIdx.x; b < nblocks; b += kMergeThreads) {
+// Per-CTA partials as the merge reads them: at(b, dim, nb) is the (mean, M2) pair of block b and sets nb to its row count;
+// rewind() precedes each pass over b = threadIdx.x, threadIdx.x + kMergeThreads, ... (increasing).
+// One batch: n_rows rows cut into blocks of rows_per_block.
+struct OneBatch {
+    const double* partials;
+    int64_t n_rows;
+    int rows_per_block, ndims;
+    SAT_DEV void rewind() {}
+    SAT_DEV const double* at(int64_t b, int dim, double& nb) {
         const int64_t rem = n_rows - b * rows_per_block;
-        const double nb = (double)(rem < rows_per_block ? rem : rows_per_block);
-        wsum += nb * partials[(b * ndims_in_partials + dim) * 2 + 0];
+        nb = (double)(rem < rows_per_block ? rem : rows_per_block);
+        return partials + (b * ndims + dim) * 2;
+    }
+};
+
+// The batches of G ranks, gathered rank-major with a stride of `stride` blocks per rank; rank r holds rank_rows[r] rows.
+// Global block b runs over rank 0's blocks, then rank 1's, ...: the block order of the union batch whenever every rank
+// but the last holds a multiple of rows_per_block rows.
+struct RankMajor {
+    const double* partials;
+    const int64_t* rank_rows;
+    int64_t stride;
+    int rows_per_block, ndims;
+    int r;
+    int64_t b0, b1;                              // global blocks [b0, b1) are rank r's
+    SAT_DEV int64_t blocks_of(int64_t rows) const { return (rows + rows_per_block - 1) / rows_per_block; }
+    SAT_DEV void rewind() { r = 0; b0 = 0; b1 = blocks_of(rank_rows[0]); }
+    SAT_DEV const double* at(int64_t b, int dim, double& nb) {
+        while (b >= b1) { ++r; b0 = b1; b1 += blocks_of(rank_rows[r]); }
+        const int64_t j = b - b0;
+        const int64_t rem = rank_rows[r] - j * rows_per_block;
+        nb = (double)(rem < rows_per_block ? rem : rows_per_block);
+        return partials + ((r * stride + j) * ndims + dim) * 2;
+    }
+};
+
+// pass 1: grand mean of the block means weighted by their rows; pass 2: M2 about it. Each thread sums its blocks in
+// increasing b, then block_sum_fixed: the result depends only on the sequence of blocks.
+template <class Blocks>
+SAT_DEV void merge_fold(Blocks blocks, int64_t nblocks, double N, double* sm, double* obs_stats, int obs_dim,
+                        double* ret_stats, double* ret_std_out, unsigned int* ticket) {
+    const int dim = blockIdx.x;                  // gridDim.x == number of statistic dims in the partials
+    double wsum = 0.0;
+    blocks.rewind();
+    for (int64_t b = threadIdx.x; b < nblocks; b += kMergeThreads) {
+        double nb;
+        const double* q = blocks.at(b, dim, nb);
+        wsum += nb * q[0];
     }
     const double grand = block_sum_fixed(wsum, sm) / N;
     double m2 = 0.0;
+    blocks.rewind();
     for (int64_t b = threadIdx.x; b < nblocks; b += kMergeThreads) {
-        const int64_t rem = n_rows - b * rows_per_block;
-        const double nb = (double)(rem < rows_per_block ? rem : rows_per_block);
-        const double dm = partials[(b * ndims_in_partials + dim) * 2 + 0] - grand;
-        m2 += partials[(b * ndims_in_partials + dim) * 2 + 1] + nb * dm * dm;
+        double nb;
+        const double* q = blocks.at(b, dim, nb);
+        const double dm = q[0] - grand;
+        m2 += q[1] + nb * dm * dm;
     }
     m2 = block_sum_fixed(m2, sm);
     if (threadIdx.x == 0) {
@@ -692,6 +729,32 @@ stats_merge_kernel(const double* __restrict__ partials, int64_t nblocks, int64_t
             *ticket = 0u;
         }
     }
+}
+
+__global__ void __launch_bounds__(kMergeThreads)
+stats_merge_kernel(const double* __restrict__ partials, int64_t nblocks, int64_t n_rows, int rows_per_block,
+                   int ndims_in_partials, double* obs_stats, int obs_dim, double* ret_stats, double* ret_std_out,
+                   unsigned int* ticket) {
+    __shared__ double sm[kMergeThreads / 32];
+    merge_fold(OneBatch{partials, n_rows, rows_per_block, ndims_in_partials}, nblocks, (double)n_rows, sm, obs_stats,
+               obs_dim, ret_stats, ret_std_out, ticket);
+}
+
+// stats_merge_kernel over the gathered partials of G ranks (RankMajor); with G == 1 it is the same fold
+__global__ void __launch_bounds__(kMergeThreads)
+stats_fold_ranks_kernel(const double* __restrict__ partials, int G, int64_t stride, const int64_t* __restrict__ rank_rows,
+                        int rows_per_block, int ndims_in_partials, double* obs_stats, int obs_dim, double* ret_stats,
+                        double* ret_std_out, unsigned int* ticket) {
+    __shared__ double sm[kMergeThreads / 32];
+    int64_t n_rows = 0, nblocks = 0;
+    for (int r = 0; r < G; ++r) {
+        const int64_t m = rank_rows[r];
+        n_rows += m;
+        nblocks += (m + rows_per_block - 1) / rows_per_block;
+    }
+    if (n_rows == 0) return;                     // nothing to fold; the ticket stays 0
+    merge_fold(RankMajor{partials, rank_rows, stride, rows_per_block, ndims_in_partials, 0, 0, 0}, nblocks,
+               (double)n_rows, sm, obs_stats, obs_dim, ret_stats, ret_std_out, ticket);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -970,16 +1033,18 @@ int sat_env_observe(const SatEnvState* st, float* obs_f32, double* obs_f64, void
 }  // extern "C"
 
 namespace {
-// ev (nullable): 4 events recorded before the first launch and after the front / finish / merge launches
+// ev (nullable): 4 events recorded before the first launch and after the front / finish / merge launches.
+// partials_out (nullable): the finish kernel's per-CTA statistics partials go there and are not merged.
 int env_step_impl(const SatEnvState* st, const void* pa, const void* ea, const int32_t* count_override,
                   float* obs_f32, double* obs_f64, double* term_obs_f64, double* reward, uint8_t* done,
                   double* obs_stats, double* ret_stats, double* ret_std_out, void* workspace,
                   const SatEnvParams* p, void* stream, cudaEvent_t* ev, float* obs_early = nullptr,
-                  cudaEvent_t front_done = nullptr, float* pa_copy = nullptr, float* ea_copy = nullptr) {
+                  cudaEvent_t front_done = nullptr, float* pa_copy = nullptr, float* ea_copy = nullptr,
+                  double* partials_out = nullptr) {
     int rc = check_state(st);
     if (rc) return rc;
     if (!pa || !ea || !reward || !done || !p) return SAT_ERR_NULL;
-    const bool want_stats = obs_stats || ret_stats;
+    const bool want_stats = obs_stats || ret_stats || partials_out;
     if ((want_stats || p->mode == SAT_MODE_RK4) && !workspace) return SAT_ERR_NULL;
     if (p->mode != SAT_MODE_CW && p->mode != SAT_MODE_RK4) return SAT_ERR_MODE;
     if (p->action_dtype != SAT_ACT_F32 && p->action_dtype != SAT_ACT_F64) return SAT_ERR_MODE;
@@ -992,7 +1057,7 @@ int env_step_impl(const SatEnvState* st, const void* pa, const void* ea, const i
     char* ws = (char*)workspace;
     unsigned int* ticket = ws ? (unsigned int*)ws : nullptr;
     double* dis_prev = ws ? (double*)(ws + ws_disprev_offset()) : nullptr;
-    double* partials = want_stats ? (double*)(ws + ws_partials_offset(n)) : nullptr;
+    double* partials = partials_out ? partials_out : want_stats ? (double*)(ws + ws_partials_offset(n)) : nullptr;
     if (ev) cudaEventRecord(ev[0], s);
     // exact host-libm arithmetic in the danger-zone path (default) or libdevice (SatEnvParams.fast_libm); resets to the
     // reference's literals or (auto_reset == SAT_RESET_STARTS) to each env's start columns
@@ -1046,7 +1111,7 @@ int env_step_impl(const SatEnvState* st, const void* pa, const void* ea, const i
     rc = launch_status();
     if (rc) return rc;
     if (ev) cudaEventRecord(ev[2], s);
-    if (partials) {
+    if (partials && !partials_out) {
         stats_merge_kernel<<<kStatDims, kMergeThreads, 0, s>>>(partials, nblocks, n, kEnvsPerBlock, kStatDims,
                                                                obs_stats, kObs, ret_stats, ret_std_out, ticket);
         rc = launch_status();
@@ -1198,6 +1263,47 @@ int sat_env_step_host(const SatEnvState* st, const float* pa_host, const float* 
     if ((ce = cudaMemcpyAsync(reward_host, io.reward, (size_t)n * 8, cudaMemcpyDeviceToHost, s0)) != cudaSuccess) return (int)ce;
     if ((ce = cudaMemcpyAsync(done_host, io.done, (size_t)n, cudaMemcpyDeviceToHost, s0)) != cudaSuccess) return (int)ce;
     return (int)cudaStreamSynchronize(s0);
+}
+
+int64_t sat_stats_partials_bytes(int64_t n, int dim) {
+    if (n <= 0 || dim < 0 || dim > 32) return 0;
+    if (dim == 0) return (n + kEnvsPerBlock - 1) / kEnvsPerBlock * kStatDims * 2 * (int64_t)sizeof(double);
+    return (n + kNormRows - 1) / kNormRows * dim * 2 * (int64_t)sizeof(double);
+}
+
+int sat_env_step_partials(const SatEnvState* st, const void* pa, const void* ea, const int32_t* count_override,
+                          float* obs_f32, double* obs_f64, double* term_obs_f64, double* reward, uint8_t* done,
+                          double* partials, void* workspace, const SatEnvParams* p, void* stream) {
+    if (!partials) return SAT_ERR_NULL;
+    return env_step_impl(st, pa, ea, count_override, obs_f32, obs_f64, term_obs_f64, reward, done, nullptr, nullptr,
+                         nullptr, workspace, p, stream, nullptr, nullptr, nullptr, nullptr, nullptr, partials);
+}
+
+int sat_norm_partials(const double* x, int64_t n, int dim, double* partials, void* workspace, void* stream) {
+    if (!x || !partials || !workspace) return SAT_ERR_NULL;
+    if (n <= 0 || dim < 1 || dim > 32) return SAT_ERR_SIZE;
+    const int64_t nblocks = (n + kNormRows - 1) / kNormRows;
+    norm_partial_kernel<<<(unsigned)nblocks, kNormRows, 0, (cudaStream_t)stream>>>(x, n, dim, partials,
+                                                                                   (unsigned int*)workspace);
+    return launch_status();
+}
+
+int sat_stats_fold(const double* partials, int ranks, int64_t rank_stride_blocks, const int64_t* rank_rows, int dim,
+                   double* obs_stats, double* ret_stats, double* ret_std_out, void* workspace, void* stream) {
+    if (!partials || !rank_rows || !workspace) return SAT_ERR_NULL;
+    if (ranks < 1 || rank_stride_blocks < 1 || dim < 0 || dim > 32) return SAT_ERR_SIZE;
+    if (dim > 0 && (ret_stats || ret_std_out)) return SAT_ERR_SIZE;
+    if (!obs_stats && !ret_stats) return SAT_OK;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (dim == 0)
+        stats_fold_ranks_kernel<<<kStatDims, kMergeThreads, 0, s>>>(partials, ranks, rank_stride_blocks, rank_rows,
+                                                                    kEnvsPerBlock, kStatDims, obs_stats, kObs, ret_stats,
+                                                                    ret_std_out, (unsigned int*)workspace);
+    else
+        stats_fold_ranks_kernel<<<dim, kMergeThreads, 0, s>>>(partials, ranks, rank_stride_blocks, rank_rows, kNormRows,
+                                                              dim, obs_stats, dim, nullptr, nullptr,
+                                                              (unsigned int*)workspace);
+    return launch_status();
 }
 
 int sat_norm_update(double* stats, const double* x, int64_t n, int dim, int update,

@@ -116,18 +116,83 @@ class RunningStats:
         self.buf.copy_(sd["buf"].to(self.buf.device))
         return self
 
-    def update_normalize(self, x, update=True, out_dtype=None):
-        """x: CUDA fp64 [n, dim]. Merges the batch (update=True) then returns (x-mean)/(std+1e-8)."""
+    def update_normalize(self, x, update=True, out_dtype=None, group=None):
+        """x: CUDA fp64 [n, dim]. Merges the batch (update=True) then returns (x-mean)/(std+1e-8).
+        group (a torch.distributed process group): x is this rank's shard of a batch sharded over the group, and the
+        merge folds every rank's shard (sat_stats_fold), so every rank's statistics become those of the union batch - bit
+        for bit when every rank but the last brings a multiple of 128 rows. Collective: every rank of the group calls it."""
         torch = L.require_cuda()
+        lib = L.load()
         x = x.contiguous()
         n = x.shape[0]
-        ws = torch.empty(L.load().sat_workspace_bytes(n), dtype=torch.uint8, device=x.device)
+        ws = torch.empty(lib.sat_workspace_bytes(n), dtype=torch.uint8, device=x.device)
+        if update and group is not None:
+            ex = StatsExchange(group, n, self.dim, x.device)
+            L.check(lib.sat_norm_partials(L.ptr(x), n, self.dim, L.ptr(ex.send), ws.data_ptr(), L.stream_ptr()),
+                    "sat_norm_partials")
+            ex.fold(self, None, None, ws)
+            update = False
         out64 = torch.empty_like(x) if out_dtype in (None, torch.float64) else None
         out32 = torch.empty(x.shape, dtype=torch.float32, device=x.device) if out_dtype == torch.float32 else None
-        L.check(L.load().sat_norm_update(self.buf.data_ptr(), x.data_ptr(), n, self.dim, int(bool(update)),
-                                         L.ptr(out64), L.ptr(out32), ws.data_ptr(), L.stream_ptr()),
+        L.check(lib.sat_norm_update(self.buf.data_ptr(), x.data_ptr(), n, self.dim, int(bool(update)),
+                                    L.ptr(out64), L.ptr(out32), ws.data_ptr(), L.stream_ptr()),
                 "sat_norm_update")
         return out64 if out64 is not None else out32
+
+
+def fold_stats(partials, rank_rows, dim: int, obs_stats: RunningStats | None = None, ret_stats: RunningStats | None = None,
+               ret_std_out=None, workspace=None):
+    """sat_stats_fold: fold the gathered per-block partials of G ranks into the statistics.
+    partials: CUDA fp64 [G, stride] rank-major, each row one rank's partials padded to a common length; rank_rows: CUDA
+    int64 [G] row counts. dim 0: env-step partials (EnvBatch.step_partials) into obs_stats (18) / ret_stats (1) /
+    ret_std_out; dim >= 1: sat_norm_partials of a [n, dim] batch into obs_stats. workspace: the workspace the partials were
+    just computed with on this stream (its ticket is zero)."""
+    torch = L.require_cuda()
+    dims = 19 if dim == 0 else dim
+    if partials.dtype != torch.float64 or partials.dim() != 2 or partials.shape[1] % (2 * dims):
+        raise L.SatError(f"partials must be float64 [ranks, blocks * {2 * dims}]")
+    if rank_rows.dtype != torch.int64 or rank_rows.numel() != partials.shape[0]:
+        raise L.SatError("rank_rows must be int64 with one row count per rank")
+    L.check(L.load().sat_stats_fold(L.ptr(partials), partials.shape[0], partials.shape[1] // (2 * dims), L.ptr(rank_rows),
+                                    int(dim), L.ptr(obs_stats.buf) if obs_stats is not None else None,
+                                    L.ptr(ret_stats.buf) if ret_stats is not None else None, L.ptr(ret_std_out),
+                                    L.ptr(workspace), L.stream_ptr()), "sat_stats_fold")
+
+
+class StatsExchange:
+    """Per-block statistics partials exchanged across the ranks of a process group: `send` takes this rank's partials,
+    fold() gathers every rank's (torch.distributed.all_gather_into_tensor on the current stream; NCCL or gloo) into one
+    rank-major buffer and folds them all into this rank's statistics (sat_stats_fold), so every rank holds the same bits.
+    dim 0: the env step's partials (64 rows per block, 19 dims); dim >= 1: a [rows, dim] batch's (128 rows per block).
+
+    Construction is collective: every rank's (rows, dim) are gathered once and checked by every rank on the same data, so
+    either every rank proceeds or every rank raises."""
+
+    def __init__(self, group, rows: int, dim: int, device):
+        torch = L.require_cuda()
+        dist = torch.distributed
+        self.group, self.dim = group, int(dim)
+        world = dist.get_world_size(group)
+        mine = torch.tensor([int(rows), int(dim)], dtype=torch.int64, device=device)
+        every = torch.empty(world * 2, dtype=torch.int64, device=device)
+        dist.all_gather_into_tensor(every, mine, group=group)
+        every = every.view(world, 2).cpu()
+        rows_all, dims_all = every[:, 0].tolist(), every[:, 1].tolist()
+        if len(set(dims_all)) != 1 or min(rows_all) < 1:
+            raise L.SatError(f"shared statistics need the same dim and at least one row on every rank; got rows {rows_all}, "
+                             f"dims {dims_all}")
+        rpb = 64 if dim == 0 else 128
+        dims = 19 if dim == 0 else dim
+        stride = max((r + rpb - 1) // rpb for r in rows_all)
+        self.rank_rows = every[:, 0].to(device).contiguous()
+        self.send = torch.zeros(stride * dims * 2, dtype=torch.float64, device=device)
+        self.gathered = torch.zeros((world, stride * dims * 2), dtype=torch.float64, device=device)
+
+    def fold(self, obs_stats: RunningStats | None, ret_stats: RunningStats | None, ret_std_out, workspace):
+        """gather every rank's `send` and fold them all; workspace as for fold_stats"""
+        import torch.distributed as dist
+        dist.all_gather_into_tensor(self.gathered.view(-1), self.send, group=self.group)
+        fold_stats(self.gathered, self.rank_rows, self.dim, obs_stats, ret_stats, ret_std_out, workspace)
 
 
 # --------------------------------------------------------------------------------------------- K2
@@ -144,6 +209,9 @@ class EnvBatch:
     env, manual or automatic, puts its kinematics at its start (count 0, int_state 0; fuel / dis / dangerous_zone persist)
     and then draws its next one. `starts` is the [12, n] view of the next starts. start_box=None: the reference's reset
     literals for every env.
+
+    share_stats(group): the batch is one rank's shard of a batch sharded over a process group, and step() updates its
+    running statistics with every rank's shard (see share_stats).
     """
 
     def __init__(self, n: int, mode: str = "cw", flag: int = 0, d_capture: float = 100000.0,
@@ -186,6 +254,7 @@ class EnvBatch:
         self.reward = torch.empty(self.n, dtype=torch.float64, device=self.device)
         self.done = torch.empty(self.n, dtype=torch.uint8, device=self.device)
         self._host = None
+        self._shared = None
         self.init()
 
     # -- parameters that the reference lets the driver patch after construction (CPPO_main.py:98)
@@ -254,8 +323,14 @@ class EnvBatch:
     def step(self, pa, ea, count=None, obs_f32=None, obs_f64=None, term_obs_f64=None, reward=None, done=None,
              obs_stats: RunningStats | None = None, ret_stats: RunningStats | None = None, ret_std_out=None):
         """One step() of every env. pa/ea: CUDA [n,3] float32 or float64. Outputs are written into the
-        given tensors (allocated by the caller to keep the hot loop allocation-free)."""
+        given tensors (allocated by the caller to keep the hot loop allocation-free). After share_stats(group), the
+        statistics are updated with every rank's step (collective)."""
         torch = self.torch
+        if self._shared is not None and (obs_stats is not None or ret_stats is not None):
+            reward, done = self.step_partials(pa, ea, self._shared.send, count, obs_f32, obs_f64, term_obs_f64, reward,
+                                              done)
+            self._shared.fold(obs_stats, ret_stats, ret_std_out, self.workspace)
+            return reward, done
         L.guard_device(self.device)
         if pa.dtype != ea.dtype or pa.dtype not in (torch.float32, torch.float64):
             raise L.SatError("actions must both be float32 or both float64")
@@ -268,6 +343,38 @@ class EnvBatch:
                                       L.ptr(ret_stats.buf) if ret_stats is not None else None,
                                       L.ptr(ret_std_out), self.workspace.data_ptr(), C.byref(self.params),
                                       L.stream_ptr()), "sat_env_step")
+        self._redraw_after_step(done)
+        return reward, done
+
+    def share_stats(self, group):
+        """Shared-statistics mode: from now on step() with obs_stats / ret_stats folds the statistics partials of every
+        rank of `group` (a torch.distributed process group, each rank holding its shard of the envs) into this rank's
+        statistics: step with the partials out (sat_env_step_partials), all_gather them, fold them all (sat_stats_fold).
+        Every rank then holds the same statistics, bit-identical to one batch of the union of the shards stepping the
+        union of the actions whenever every rank but the last holds a multiple of 64 envs (and row_offset / start_seed
+        key each env by its global index). Collective: every rank calls it, and every rank's step() must then pass the
+        same set of statistics. group=None switches back to per-rank statistics (not collective)."""
+        self._shared = None if group is None else StatsExchange(group, self.n, 0, self.device)
+        return self
+
+    def step_partials(self, pa, ea, partials, count=None, obs_f32=None, obs_f64=None, term_obs_f64=None, reward=None,
+                      done=None):
+        """step() with statistics on, but the per-block partials go to `partials` (CUDA fp64, at least
+        sat_stats_partials_bytes(n, 0) bytes) instead of into any statistics; fold_stats() folds them. The workspace
+        of this batch is then ready for fold_stats()."""
+        torch = self.torch
+        L.guard_device(self.device)
+        if pa.dtype != ea.dtype or pa.dtype not in (torch.float32, torch.float64):
+            raise L.SatError("actions must both be float32 or both float64")
+        if partials.dtype != torch.float64 or partials.numel() * 8 < self.lib.sat_stats_partials_bytes(self.n, 0):
+            raise L.SatError("partials must be float64 of at least sat_stats_partials_bytes(n, 0) bytes")
+        self.params.action_dtype = L.ACT_F32 if pa.dtype == torch.float32 else L.ACT_F64
+        reward = self.reward if reward is None else reward
+        done = self.done if done is None else done
+        L.check(self.lib.sat_env_step_partials(C.byref(self.st), L.ptr(pa), L.ptr(ea), L.ptr(count), L.ptr(obs_f32),
+                                               L.ptr(obs_f64), L.ptr(term_obs_f64), L.ptr(reward), L.ptr(done),
+                                               L.ptr(partials), self.workspace.data_ptr(), C.byref(self.params),
+                                               L.stream_ptr()), "sat_env_step_partials")
         self._redraw_after_step(done)
         return reward, done
 

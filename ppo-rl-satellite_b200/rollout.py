@@ -35,21 +35,31 @@ class RolloutBuffer:
 
 
 class VectorTrainer:
-    """Drives `agent` (learner: pursuer for flag 0, evader for flag 1) against `opponent` on an EnvBatch."""
+    """Drives `agent` (learner: pursuer for flag 0, evader for flag 1) against `opponent` on an EnvBatch.
+
+    stats_group (a torch.distributed process group, default None): the ranks of the group each drive their shard of one
+    env batch, and the running statistics (observation normaliser, return statistics behind the reward scaling) are
+    shared: the initial observations' statistics and every collect() step fold every rank's shard (EnvBatch.share_stats,
+    RunningStats.update_normalize with group). Every rank then holds the same statistics, those of the union batch, bit
+    for bit when every rank but the last holds a multiple of 128 envs (the initial observations are folded in blocks of
+    128 rows, the steps in blocks of 64) and the env batches key their starts by global env index (row_offset). Collective: every rank of the group builds its trainer
+    with the same stats_group. None: each rank's statistics see its own shard only."""
 
     def __init__(self, env: eng.EnvBatch, agent, opponent, T: int, use_state_norm=True, use_reward_scaling=True,
-                 rank: int = 0, seed: int = 0, strict_errors: bool = False):
+                 rank: int = 0, seed: int = 0, strict_errors: bool = False, stats_group=None):
         self.env, self.agent, self.opponent, self.T = env, agent, opponent, T
         self.strict_errors = strict_errors
         self.buf = RolloutBuffer(T, env.n, env.device)
         self.obs_stats = eng.RunningStats(18, env.device) if use_state_norm else None
         self.ret_stats = eng.RunningStats(1, env.device) if use_reward_scaling else None
-        self.row_offset = rank * env.n
+        self.row_offset = rank * env.n            # the global row id of env 0 only when every shard holds env.n envs
         self.seed = seed
         self.t_global = 0
         self.explained_variance = None
+        if stats_group is not None:
+            env.share_stats(stats_group)
         if self.obs_stats is not None:
-            self.obs_stats.update_normalize(env.observe())          # statistics of the initial observations
+            self.obs_stats.update_normalize(env.observe(), group=stats_group)   # statistics of the initial observations
         self.learner_is_pursuer = env.params.flag == 0
 
     def collect(self):
@@ -129,6 +139,8 @@ class VectorTrainer:
 
     # ---- full-run checkpoint: env SoA state, running normalisers, Philox counter, networks + optimisers
     def state_dict(self):
+        """With stats_group set, every rank holds the same obs_stats / ret_stats, so the statistics of a state_dict() saved
+        on any rank are valid for every rank; the "env" entry is the saving rank's shard."""
         ag = self.agent
         return {"env": self.env.state_dict(), "t_global": self.t_global, "seed": self.seed,
                 "obs_stats": self.obs_stats.state_dict() if self.obs_stats is not None else None,

@@ -288,6 +288,32 @@ int sat_actor_sample_pair_tc(const SatActorWeights* wa, const SatActorWeights* w
                              const float* obs_f32, const SatEnvState* st, const double* obs_stats, int64_t n, int64_t row_offset,
                              uint64_t seed, uint64_t step_a, uint64_t step_b, float* act_a, float* logp_a, float* obs_out,
                              float* act_b, float* logp_b, void* stream);
+/* Opponent pool (self-play against past snapshots): the learner wa on all n rows and, on contiguous groups of rows, frozen
+ * snapshots of earlier networks, all in ONE persistent launch (the learner's tiles, then every group's tiles).
+ * sat_actor_tc_snapshot builds a snapshot of w once: its tensor-core weight image (tc_image, SAT_ACTOR_TC_IMAGE_FLOATS
+ * floats) and its bias / head tables (tc_tables, SAT_ACTOR_TC_TABLE_FLOATS floats), both from w->packed, and fills *snap
+ * (host memory) with the pointers, w's activation and max_action; row_end is left 0. w->packed, tc_image and tc_tables must
+ * stay unchanged while the snapshot is in use (copy the packed weights first if the network trains on).
+ * sat_actor_sample_pool_tc: group k covers rows [groups_host[k - 1].row_end, groups_host[k].row_end) (0 for k = 0); its
+ * outputs act_b / logp_b are exactly those of sat_actor_sample_tc of that snapshot on those rows with row offset
+ * row_offset + groups_host[k - 1].row_end and step step_b; act_a / logp_a / obs_out are exactly sat_actor_sample_pair_tc's
+ * net-a outputs. 1 <= groups <= SAT_ACTOR_POOL_MAX_GROUPS, row_end strictly increasing, every row_end but the last a multiple
+ * of 128 (the row tile) and the last = n (SAT_ERR_SIZE); every snapshot built with wa's activation (SAT_ERR_MODE). */
+#define SAT_ACTOR_POOL_MAX_GROUPS 16
+#define SAT_ACTOR_TC_TABLE_FLOATS (5 * 256)   /* per column pair two float4 (b2, head weights), then b1 in accumulator order */
+typedef struct {
+    const float* packed;      /* the snapshot's SAT_ACTOR_PACKED_FLOATS weights (b3 and log_std are read from here) */
+    const float* tc_image;    /* its tensor-core weight image */
+    const float* tc_tables;   /* its bias / head tables */
+    int64_t row_end;          /* exclusive end of the group's rows (set by the caller before sampling) */
+    int32_t use_tanh;         /* activation the snapshot was built with */
+    float   max_action;
+} SatActorPoolGroup;
+int sat_actor_tc_snapshot(const SatActorWeights* w, float* tc_image, float* tc_tables, SatActorPoolGroup* snap, void* stream);
+int sat_actor_sample_pool_tc(const SatActorWeights* wa, float* tc_image_a, const SatActorPoolGroup* groups_host, int groups,
+                             const float* obs_f32, const SatEnvState* st, const double* obs_stats, int64_t n,
+                             int64_t row_offset, uint64_t seed, uint64_t step_a, uint64_t step_b, float* act_a, float* logp_a,
+                             float* obs_out, float* act_b, float* logp_b, void* stream);
 int sat_critic_forward(const SatActorWeights* w, const float* obs_f32, int64_t n, float* v, void* stream);
 /* Two Gaussian actors on the same observations in ONE launch (pursuer and evader of a rollout step, CPPO_main.py:122-123):
  * exactly the results of two sat_actor_sample calls with steps step_a / step_b; obs_out (nullable) receives the fp32

@@ -23,6 +23,8 @@ MODE_CW, MODE_RK4 = 0, 1
 ACT_F32, ACT_F64 = 0, 1
 ACTOR_PACKED_FLOATS = 18 * 256 + 256 + 256 * 256 + 256 + 4 * 256 + 4 + 4
 ACTOR_TC_IMAGE_FLOATS = 2 * 256 * 256
+ACTOR_TC_TABLE_FLOATS = 5 * 256
+ACTOR_POOL_MAX_GROUPS = 16
 
 
 class SatEnvState(C.Structure):
@@ -44,6 +46,11 @@ class SatActorWeights(C.Structure):
     _fields_ = [("w1", C.c_void_p), ("b1", C.c_void_p), ("w2", C.c_void_p), ("b2", C.c_void_p),
                 ("w3", C.c_void_p), ("b3", C.c_void_p), ("log_std", C.c_void_p), ("packed", C.c_void_p),
                 ("in_dim", C.c_int32), ("hidden", C.c_int32), ("act_dim", C.c_int32),
+                ("use_tanh", C.c_int32), ("max_action", C.c_float)]
+
+
+class SatActorPoolGroup(C.Structure):
+    _fields_ = [("packed", C.c_void_p), ("tc_image", C.c_void_p), ("tc_tables", C.c_void_p), ("row_end", C.c_int64),
                 ("use_tanh", C.c_int32), ("max_action", C.c_float)]
 
 
@@ -129,6 +136,9 @@ SIGNATURES = {
     "sat_actor_sample_tc": (C.c_int, [C.POINTER(SatActorWeights), _P, _P, C.POINTER(SatEnvState), _P, _I64, _I64,
                                       _U64, _U64, _P, _P, _P, _P, _P, _P, _P]),
     "sat_actor_sample_pair_tc": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _I64, _I64, _U64, _U64, _U64, _P, _P, _P, _P, _P, _P]),
+    "sat_actor_tc_snapshot": (C.c_int, [C.POINTER(SatActorWeights), _P, _P, C.POINTER(SatActorPoolGroup), _P]),
+    "sat_actor_sample_pool_tc": (C.c_int, [C.POINTER(SatActorWeights), _P, C.POINTER(SatActorPoolGroup), _I32, _P,
+                                           C.POINTER(SatEnvState), _P, _I64, _I64, _U64, _U64, _U64, _P, _P, _P, _P, _P, _P]),
     "sat_critic_forward": (C.c_int, [C.POINTER(SatActorWeights), _P, _I64, _P, _P]),
     "sat_actor_sample_pair": (C.c_int, [_P, _P, _P, _P, _P, _I64, _I64, _U64, _U64, _U64, _P, _P, _P, _P, _P, _P]),
     "sat_gae": (C.c_int, [_P, _P, _P, _P, _I64, _I64, _F, _F, _P, _P, _P]),

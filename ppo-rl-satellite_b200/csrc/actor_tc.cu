@@ -36,6 +36,7 @@
 // chunks are on the tensor core, and its layer-1 MMAs start as soon as the epilogue has the accumulators in registers.
 // Shared memory: A 2 x 24 KB, X 24 KB, B 3 x 48 KB, head table 4 KB, bias 1 KB = 222 KB -> one CTA per SM.
 #include <cstdint>
+#include <type_traits>
 #include <cuda_runtime.h>
 #include "sat_math.cuh"
 #include "tc_mlp.cuh"
@@ -83,6 +84,41 @@ __global__ void actor_tc_pack_kernel(const float* __restrict__ packed0, unsigned
     *reinterpret_cast<uint4*>(base) = H;
     *reinterpret_cast<uint4*>(base + B_WORD) = M;
     *reinterpret_cast<uint4*>(base + 2 * B_WORD) = L;
+}
+
+// A frozen snapshot's bias / head tables in global memory, in exactly the layout of the kernel's shared-memory tables (one
+// network): w3p[HID] float4 (per column pair (b2a', b2b', w0a, w0b), (w1a, w1b, w2a, w2b)), then b1p[HID] in layer-1
+// accumulator column order; tanh networks carry b1 and b2 pre-multiplied by 2 log2(e) like the kernel's own tables.
+constexpr int TAB_W3P = 0, TAB_B1P = 4 * HID;
+static_assert(TAB_B1P + HID == SAT_ACTOR_TC_TABLE_FLOATS, "header constant out of sync");
+__global__ void actor_tc_table_kernel(const float* __restrict__ pk, float* __restrict__ tables, int use_tanh) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= HID) return;
+    const float bs = use_tanh ? kTwoLog2e : 1.0f;
+    tables[TAB_B1P + c] = pk[OFF_B1 + l1_unit(c)] * bs;
+    const int pr = c >> 1, hb = c & 1;
+    float* q0 = tables + TAB_W3P + 8 * pr;
+    q0[hb] = pk[OFF_B2 + c] * bs;
+    q0[2 + hb] = pk[OFF_W3 + c];
+    q0[4 + hb] = pk[OFF_W3 + HID + c];
+    q0[6 + hb] = pk[OFF_W3 + 2 * HID + c];
+}
+
+// the opponent groups of a pool launch (kernel parameter space): group k covers rows [row_end[k - 1], row_end[k])
+struct TcPool {
+    const float* packed[SAT_ACTOR_POOL_MAX_GROUPS];
+    const unsigned char* image[SAT_ACTOR_POOL_MAX_GROUPS];
+    const float* tables[SAT_ACTOR_POOL_MAX_GROUPS];
+    int64_t row_end[SAT_ACTOR_POOL_MAX_GROUPS];
+    float max_action[SAT_ACTOR_POOL_MAX_GROUPS];
+    int groups;
+};
+struct TcNoPool {};
+// the group holding row row0 (a row tile never straddles two groups: every interior bound is a multiple of TM)
+__device__ __forceinline__ int pool_group(const TcPool& p, int64_t row0) {
+    int k = 0;
+    while (k + 1 < p.groups && row0 >= p.row_end[k]) ++k;
+    return k;
 }
 
 #ifdef SAT_TC_TRACE
@@ -179,11 +215,15 @@ struct TcNet {
     float max_action;
 };
 
-template <bool TANH>
+// POOL: network 1 is an opponent pool (nnet = 2, net1 holds only the outputs and the step): an opponent tile streams the
+// image of the group holding its rows, reads that group's bias / head tables from global memory (the shared-memory tables
+// hold network 0's only) and its b3 / log_std / max_action from the group; the learner's tiles are network 0's as above.
+template <bool TANH, bool POOL>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 actor_tc_kernel(const __grid_constant__ TcNet net0, const __grid_constant__ TcNet net1, const int nnet,
                 const float* __restrict__ obs_f32, const SatEnvState st, const double* __restrict__ obs_stats, int64_t n,
-                int64_t row_offset, uint64_t seed, float* __restrict__ obs_out) {
+                int64_t row_offset, uint64_t seed, float* __restrict__ obs_out,
+                const __grid_constant__ std::conditional_t<POOL, TcPool, TcNoPool> pool) {
     extern __shared__ unsigned char smem_dyn[];
     // 1024-byte alignment for the swizzled tiles by pointer arithmetic on the shared array (an integer round trip would turn
     // every access into a generic-space LD/ST)
@@ -216,7 +256,7 @@ actor_tc_kernel(const __grid_constant__ TcNet net0, const __grid_constant__ TcNe
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(kTmemCols) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
-    for (int i = tid; i < HID * nnet; i += TC_THREADS) {
+    for (int i = tid; i < HID * (POOL ? 1 : nnet); i += TC_THREADS) {
         // biases pre-multiplied by 2 log2(e) for the tanh networks (the activation takes its argument in that scale)
         const int nt = i / HID, c = i % HID;
         const float* pk = nt ? net1.packed : net0.packed;
@@ -287,6 +327,7 @@ actor_tc_kernel(const __grid_constant__ TcNet net0, const __grid_constant__ TcNe
             for (int t = 0; t < my_tiles; ++t) {
                 const int u = (int)blockIdx.x + t * (int)gridDim.x;
                 const unsigned char* img = (u >= ntiles) ? net1.image : net0.image;
+                if constexpr (POOL) { if (u >= ntiles) img = pool.image[pool_group(pool, (int64_t)(u - ntiles) * TM)]; }
 #pragma unroll 1
                 for (int idx = 0; idx < SUBS; ++idx, ++pq) {
                     if (pq >= NSB) mbar_wait(&b_empty[sb], bphase ^ 1);  // the MMAs of sub-chunk pq - NSB have read this stage
@@ -326,7 +367,10 @@ actor_tc_kernel(const __grid_constant__ TcNet net0, const __grid_constant__ TcNe
             const float* __restrict__ packed = nt.packed;
             const float* __restrict__ eps_in = nt.eps_in;
             const uint64_t step = nt.step;
-            const float max_action = nt.max_action;
+            float max_action = nt.max_action;
+            if constexpr (POOL) {
+                if (tile_net(tt)) { const int k = pool_group(pool, tile_row0(tt)); packed = pool.packed[k]; max_action = pool.max_action[k]; }
+            }
             const float* rd = red + (tt & 1) * (NPART * TM * 4);
             const float pre_a = ((rd[(0 * TM + r) * 4 + a] + rd[(1 * TM + r) * 4 + a]) + rd[(2 * TM + r) * 4 + a]) + rd[(3 * TM + r) * 4 + a];
             float eps;
@@ -355,7 +399,15 @@ actor_tc_kernel(const __grid_constant__ TcNet net0, const __grid_constant__ TcNe
         };
 #pragma unroll 1
         for (int t = 0; t < my_tiles; ++t) {
-            const int tab = tile_net(t) * HID;                          // this tile's bias / head tables
+            int tab = tile_net(t) * HID;                                // this tile's bias / head tables
+            const float* b1t = b1p;
+            const float4* w3t = w3p;
+            if constexpr (POOL) {
+                if (tile_net(t)) {                                      // an opponent's tables: global, broadcast loads
+                    const float* tg = pool.tables[pool_group(pool, tile_row0(t))];
+                    b1t = tg + TAB_B1P; w3t = reinterpret_cast<const float4*>(tg + TAB_W3P); tab = 0;
+                }
+            }
             if (t + 1 < my_tiles) prefetch_x(part, tile_row0(t + 1) + r, n, obs_f32, st);
             // ---- layer-1 pre-activations of the thread's 64 hidden units (columns [64 part, +64) of both accumulators)
             float pre1[CPT];
@@ -379,7 +431,7 @@ actor_tc_kernel(const __grid_constant__ TcNet net0, const __grid_constant__ TcNe
                 float h[UPT];
 #pragma unroll
                 for (int j = 0; j < UPT; j += 2) {
-                    const float2 bb = *reinterpret_cast<const float2*>(b1p + tab + part * CPT + kc * UPT + j);
+                    const float2 bb = *reinterpret_cast<const float2*>(b1t + tab + part * CPT + kc * UPT + j);
                     const float2 hh = act2_scaled<TANH>(__ffma2_rn(make_float2(pre1[kc * UPT + j], pre1[kc * UPT + j + 1]), make_float2(sc, sc), bb));
                     h[j] = hh.x; h[j + 1] = hh.y;
                 }
@@ -423,7 +475,7 @@ actor_tc_kernel(const __grid_constant__ TcNet net0, const __grid_constant__ TcNe
             float2 p0 = make_float2(0.0f, 0.0f), p1 = p0, p2 = p0;
 #pragma unroll
             for (int j = 0; j < CPT; j += 2) {
-                const float4 qa4 = w3p[tab + part * CPT + j], qb4 = w3p[tab + part * CPT + j + 1];   // pair (j, j + 1): two broadcast loads
+                const float4 qa4 = w3t[tab + part * CPT + j], qb4 = w3t[tab + part * CPT + j + 1];   // pair (j, j + 1): two broadcast loads
                 const float2 h2 = act2_scaled_fma<TANH>(__ffma2_rn(make_float2(acc2[j], acc2[j + 1]), make_float2(sc, sc), make_float2(qa4.x, qa4.y)));
                 p0 = __ffma2_rn(h2, make_float2(qa4.z, qa4.w), p0);
                 p1 = __ffma2_rn(h2, make_float2(qb4.x, qb4.y), p1);
@@ -456,6 +508,35 @@ extern "C" int sat_debug_actor_tc_trace(unsigned long long* out) { return (int)c
 #endif
 
 namespace {
+// once per device: the kernels' shared-memory opt-in; the SM count (cached)
+int tc_setup(int* sms_out) {
+    static unsigned char done[64] = {0};
+    static int sm_count[64] = {0};
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return (int)e;
+    const bool cached = dev >= 0 && dev < 64;
+    if (!cached || !done[dev]) {
+        e = cudaFuncSetAttribute(actor_tc_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM);
+        if (e != cudaSuccess) return (int)e;
+        e = cudaFuncSetAttribute(actor_tc_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM);
+        if (e != cudaSuccess) return (int)e;
+        e = cudaFuncSetAttribute(actor_tc_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM);
+        if (e != cudaSuccess) return (int)e;
+        e = cudaFuncSetAttribute(actor_tc_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM);
+        if (e != cudaSuccess) return (int)e;
+        if (cached) done[dev] = 1;
+    }
+    int sms = cached ? sm_count[dev] : 0;
+    if (sms <= 0) {
+        e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+        if (e != cudaSuccess) return (int)e;
+        if (cached) sm_count[dev] = sms;
+    }
+    *sms_out = sms;
+    return SAT_OK;
+}
+
 // launches the persistent kernel for one network (b == nullptr) or two networks on the same observations
 int launch_tc(const SatActorWeights* wa, float* image_a, const SatActorWeights* wb, float* image_b, const float* obs_f32,
               const SatEnvState* st, const double* obs_stats, int64_t n, int64_t row_offset, uint64_t seed, uint64_t step_a,
@@ -470,25 +551,9 @@ int launch_tc(const SatActorWeights* wa, float* image_a, const SatActorWeights* 
     if (n <= 0 || ((uintptr_t)wa->packed & 15) || ((uintptr_t)image_a & 15)) return SAT_ERR_SIZE;
     if (wb && (((uintptr_t)wb->packed & 15) || ((uintptr_t)image_b & 15))) return SAT_ERR_SIZE;
     if (!obs_f32 && (st->n < n || st->ld < st->n)) return SAT_ERR_SIZE;
-    static unsigned char done[64] = {0};
-    static int sm_count[64] = {0};
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
+    int sms = 0;
+    cudaError_t e = (cudaError_t)tc_setup(&sms);
     if (e != cudaSuccess) return (int)e;
-    const bool cached = dev >= 0 && dev < 64;
-    if (!cached || !done[dev]) {
-        e = cudaFuncSetAttribute(actor_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM);
-        if (e != cudaSuccess) return (int)e;
-        e = cudaFuncSetAttribute(actor_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM);
-        if (e != cudaSuccess) return (int)e;
-        if (cached) done[dev] = 1;
-    }
-    int sms = cached ? sm_count[dev] : 0;
-    if (sms <= 0) {
-        e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (e != cudaSuccess) return (int)e;
-        if (cached) sm_count[dev] = sms;
-    }
     cudaStream_t s = (cudaStream_t)stream;
     // the images are rebuilt from the live weights on every call (a few microseconds): they can never be stale
     TcNet n0 = {wa->packed, reinterpret_cast<unsigned char*>(image_a), eps_in, act_a, logp_a, mean_out, eps_out, step_a, wa->max_action};
@@ -508,8 +573,61 @@ int launch_tc(const SatActorWeights* wa, float* image_a, const SatActorWeights* 
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;     // overlap this kernel's prologue with the pack kernel
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
-    e = wa->use_tanh ? cudaLaunchKernelEx(&cfg, actor_tc_kernel<true>, n0, n1, nnet, obs_f32, s0, obs_stats, n, row_offset, seed, obs_out)
-                     : cudaLaunchKernelEx(&cfg, actor_tc_kernel<false>, n0, n1, nnet, obs_f32, s0, obs_stats, n, row_offset, seed, obs_out);
+    e = wa->use_tanh ? cudaLaunchKernelEx(&cfg, actor_tc_kernel<true, false>, n0, n1, nnet, obs_f32, s0, obs_stats, n, row_offset, seed, obs_out, TcNoPool{})
+                     : cudaLaunchKernelEx(&cfg, actor_tc_kernel<false, false>, n0, n1, nnet, obs_f32, s0, obs_stats, n, row_offset, seed, obs_out, TcNoPool{});
+    return e == cudaSuccess ? launch_status() : (int)e;
+}
+
+// the learner on all rows and the snapshot of every group on its rows, in one persistent grid: the learner's image is rebuilt
+// from its live weights (the snapshots' images are frozen, built once by sat_actor_tc_snapshot)
+int launch_pool(const SatActorWeights* wa, float* image_a, const SatActorPoolGroup* groups, int ngroups, const float* obs_f32,
+                const SatEnvState* st, const double* obs_stats, int64_t n, int64_t row_offset, uint64_t seed, uint64_t step_a,
+                uint64_t step_b, float* act_a, float* logp_a, float* obs_out, float* act_b, float* logp_b, void* stream) {
+    if (!wa || !wa->packed || !image_a || !groups || !act_a || !logp_a || !act_b || !logp_b || (!obs_f32 && !st)) return SAT_ERR_NULL;
+    if (ngroups < 1 || ngroups > SAT_ACTOR_POOL_MAX_GROUPS) return SAT_ERR_SIZE;
+    for (int k = 0; k < ngroups; ++k)
+        if (!groups[k].packed || !groups[k].tc_image || !groups[k].tc_tables) return SAT_ERR_NULL;
+    if (wa->in_dim != IN || wa->hidden != HID || wa->act_dim != 3) return SAT_ERR_SIZE;
+    if (n <= 0 || ((uintptr_t)wa->packed & 15) || ((uintptr_t)image_a & 15)) return SAT_ERR_SIZE;
+    if (!obs_f32 && (st->n < n || st->ld < st->n)) return SAT_ERR_SIZE;
+    TcPool pool = {};
+    pool.groups = ngroups;
+    int64_t lo = 0;
+    for (int k = 0; k < ngroups; ++k) {
+        const SatActorPoolGroup& g = groups[k];
+        const int64_t hi = g.row_end;
+        if (hi <= lo || (k + 1 < ngroups && hi % TM) || (k + 1 == ngroups && hi != n)) return SAT_ERR_SIZE;
+        if (((uintptr_t)g.packed | (uintptr_t)g.tc_image | (uintptr_t)g.tc_tables) & 15) return SAT_ERR_SIZE;
+        if ((g.use_tanh != 0) != (wa->use_tanh != 0)) return SAT_ERR_MODE;      // one activation per launch
+        pool.packed[k] = g.packed;
+        pool.image[k] = reinterpret_cast<const unsigned char*>(g.tc_image);
+        pool.tables[k] = g.tc_tables;
+        pool.row_end[k] = hi;
+        pool.max_action[k] = g.max_action;
+        lo = hi;
+    }
+    int sms = 0;
+    cudaError_t e = (cudaError_t)tc_setup(&sms);
+    if (e != cudaSuccess) return (int)e;
+    cudaStream_t s = (cudaStream_t)stream;
+    TcNet n0 = {wa->packed, reinterpret_cast<unsigned char*>(image_a), nullptr, act_a, logp_a, nullptr, nullptr, step_a, wa->max_action};
+    TcNet n1 = {nullptr, nullptr, nullptr, act_b, logp_b, nullptr, nullptr, step_b, 0.0f};
+    actor_tc_pack_kernel<<<dim3((NCHUNK * 4 * HID + 255) / 256, 1), 256, 0, s>>>(n0.packed, const_cast<unsigned char*>(n0.image),
+                                                                             nullptr, nullptr);
+    int rc = launch_status();
+    if (rc) return rc;
+    SatEnvState s0 = {};
+    if (!obs_f32) s0 = *st;
+    const int64_t work = ((n + TM - 1) / TM) * 2;
+    const unsigned blocks = (unsigned)(work < sms ? work : sms);
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(blocks); cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = TC_SMEM; cfg.stream = s;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;     // overlap this kernel's prologue with the pack kernel
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr; cfg.numAttrs = 1;
+    e = wa->use_tanh ? cudaLaunchKernelEx(&cfg, actor_tc_kernel<true, true>, n0, n1, 2, obs_f32, s0, obs_stats, n, row_offset, seed, obs_out, pool)
+                     : cudaLaunchKernelEx(&cfg, actor_tc_kernel<false, true>, n0, n1, 2, obs_f32, s0, obs_stats, n, row_offset, seed, obs_out, pool);
     return e == cudaSuccess ? launch_status() : (int)e;
 }
 }  // namespace
@@ -531,6 +649,30 @@ int sat_actor_sample_pair_tc(const SatActorWeights* wa, const SatActorWeights* w
     if (!wb) return SAT_ERR_NULL;
     return launch_tc(wa, tc_image_a, wb, tc_image_b, obs_f32, st, obs_stats, n, row_offset, seed, step_a, step_b, nullptr, act_a,
                      logp_a, nullptr, nullptr, obs_out, act_b, logp_b, stream);
+}
+
+int sat_actor_tc_snapshot(const SatActorWeights* w, float* tc_image, float* tc_tables, SatActorPoolGroup* snap, void* stream) {
+    if (!w || !w->packed || !tc_image || !tc_tables || !snap) return SAT_ERR_NULL;
+    if (w->in_dim != IN || w->hidden != HID || w->act_dim != 3) return SAT_ERR_SIZE;
+    if (((uintptr_t)w->packed | (uintptr_t)tc_image | (uintptr_t)tc_tables) & 15) return SAT_ERR_SIZE;
+    cudaStream_t s = (cudaStream_t)stream;
+    actor_tc_pack_kernel<<<dim3((NCHUNK * 4 * HID + 255) / 256, 1), 256, 0, s>>>(w->packed, reinterpret_cast<unsigned char*>(tc_image),
+                                                                             nullptr, nullptr);
+    int rc = launch_status();
+    if (rc) return rc;
+    actor_tc_table_kernel<<<1, HID, 0, s>>>(w->packed, tc_tables, w->use_tanh);
+    rc = launch_status();
+    if (rc) return rc;
+    *snap = SatActorPoolGroup{w->packed, tc_image, tc_tables, 0, w->use_tanh != 0, w->max_action};
+    return SAT_OK;
+}
+
+int sat_actor_sample_pool_tc(const SatActorWeights* wa, float* tc_image_a, const SatActorPoolGroup* groups_host, int groups,
+                             const float* obs_f32, const SatEnvState* st, const double* obs_stats, int64_t n,
+                             int64_t row_offset, uint64_t seed, uint64_t step_a, uint64_t step_b, float* act_a, float* logp_a,
+                             float* obs_out, float* act_b, float* logp_b, void* stream) {
+    return launch_pool(wa, tc_image_a, groups_host, groups, obs_f32, st, obs_stats, n, row_offset, seed, step_a, step_b, act_a,
+                       logp_a, obs_out, act_b, logp_b, stream);
 }
 
 }  // extern "C"

@@ -718,6 +718,63 @@ class GaussianActorKernel:
                 "sat_actor_sample_pair")
         return act, logp, other_act, other_logp
 
+    def sample_vs_pool(self, pool: "OpponentPool", slots, group_row_end, obs=None, env: EnvBatch | None = None,
+                       obs_stats: RunningStats | None = None, seed: int = 0, step: int = 0, other_step: int = 1,
+                       row_offset: int = 0, act=None, logp=None, obs_out=None, other_act=None, other_logp=None,
+                       tc: bool | None = None):
+        """the pool counterpart of sample_pair: this actor on all rows (exactly sample_pair's own outputs) and, on rows
+        [group_row_end[k - 1], group_row_end[k]), the snapshot in pool slot slots[k] (exactly that snapshot's sample() on
+        those rows with row_offset + group_row_end[k - 1] and step other_step) -> (act, logp, other_act, other_logp).
+        Tensor-core path (default): every group's tiles and the learner's go through ONE persistent grid
+        (sat_actor_sample_pool_tc); every bound but the last a multiple of 128, the last = the row count. FFMA2 path
+        (tc=False): one sample() per group."""
+        torch = self.torch
+        L.guard_device(self.device)
+        if self.w is None:
+            raise L.SatError("weights not loaded")
+        slots, ends = [int(s) for s in slots], [int(e) for e in group_row_end]
+        if len(slots) != len(ends):
+            raise L.SatError(f"{len(slots)} slots for {len(ends)} groups")
+        groups = [pool.group(s) for s in slots]                    # IndexError on a slot the pool does not hold
+        n = obs.shape[0] if obs is not None else env.n
+        use_tc = (self.use_tc if tc is None else tc) and not self.critic
+        new = lambda: torch.empty((n, ACT_DIM), dtype=torch.float32, device=self.device)
+        act = new() if act is None else act
+        logp = new() if logp is None else logp
+        other_act = new() if other_act is None else other_act
+        other_logp = new() if other_logp is None else other_logp
+        if obs is None:
+            # the fp32 (normalised) observation, materialised once (sat_env_observe_norm: the fused path's arithmetic)
+            obs, env, obs_stats, obs_out = self._tc_obs(env, obs_stats, obs_out), None, None, None
+        m64 = 2 ** 64 - 1
+        if use_tc:
+            arr = (L.SatActorPoolGroup * max(1, len(groups)))()
+            for k, (g, e) in enumerate(zip(groups, ends)):
+                arr[k] = g
+                arr[k].row_end = e
+            L.check(self.lib.sat_actor_sample_pool_tc(C.byref(self.w), self._image().data_ptr(), arr, len(groups), L.ptr(obs),
+                                                      None, None, n, int(row_offset), int(seed) & m64, int(step) & m64,
+                                                      int(other_step) & m64, L.ptr(act), L.ptr(logp), L.ptr(obs_out),
+                                                      L.ptr(other_act), L.ptr(other_logp), L.stream_ptr()),
+                    "sat_actor_sample_pool_tc")
+            return act, logp, other_act, other_logp
+        if not 1 <= len(ends) <= L.ACTOR_POOL_MAX_GROUPS:
+            raise L.SatError(f"{len(ends)} groups: 1 .. {L.ACTOR_POOL_MAX_GROUPS} supported")
+        lo = 0
+        for k, e in enumerate(ends):
+            if e <= lo or (k + 1 < len(ends) and e % 128) or (k + 1 == len(ends) and e != n):
+                raise L.SatError(f"group bounds {ends}: strictly increasing, multiples of 128 but the last, the last = {n}")
+            lo = e
+        if any(g.use_tanh != self.use_tanh for g in groups):
+            raise L.SatError("a snapshot was built with another activation than this actor")
+        self.sample(obs=obs, seed=seed, step=step, row_offset=row_offset, act=act, logp=logp, obs_out=obs_out, tc=False)
+        lo = 0
+        for s, e in zip(slots, ends):
+            pool.kernel(s).sample(obs=obs[lo:e], seed=seed, step=other_step, row_offset=int(row_offset) + lo,
+                                  act=other_act[lo:e], logp=other_logp[lo:e], tc=False)
+            lo = e
+        return act, logp, other_act, other_logp
+
     def value(self, obs, out=None):
         torch = self.torch
         if not self.critic:
@@ -727,6 +784,97 @@ class GaussianActorKernel:
         L.check(self.lib.sat_critic_forward(C.byref(self.w), L.ptr(obs), n, L.ptr(out), L.stream_ptr()),
                 "sat_critic_forward")
         return out
+
+
+class OpponentPool:
+    """A FIFO ring of up to `capacity` frozen snapshots of an actor, for self-play against past opponents (fictitious
+    self-play / league training instead of pure alternating best response). add(actor_kernel) copies the actor's packed
+    weights and builds their tensor-core weight image and bias / head tables once (sat_actor_tc_snapshot, about 0.8 MB of
+    device memory per snapshot); when the ring is full the oldest snapshot goes. Every snapshot gets the next id of a
+    counter that never goes back. Slot k is the k-th oldest snapshot held (ids[k]). GaussianActorKernel.sample_vs_pool
+    samples any of them on groups of rows in the learner's launch."""
+
+    def __init__(self, capacity: int, use_tanh: bool = True, max_action: float = 1.6, device="cuda"):
+        if not 1 <= int(capacity) <= L.ACTOR_POOL_MAX_GROUPS:
+            raise L.SatError(f"pool capacity {capacity}: 1 .. {L.ACTOR_POOL_MAX_GROUPS} supported")
+        torch = L.require_cuda()
+        self.torch, self.lib = torch, L.load()
+        self.capacity, self.use_tanh, self.max_action = int(capacity), int(bool(use_tanh)), float(max_action)
+        self.device = torch.device(device)
+        self._snaps = []                  # oldest first: {"id", "packed", "image", "tables", "group", "kernel"}
+        self._next_id = 0
+
+    def __len__(self):
+        return len(self._snaps)
+
+    @property
+    def ids(self):
+        return [s["id"] for s in self._snaps]
+
+    def add(self, actor_kernel: GaussianActorKernel) -> int:
+        """snapshot the actor's current weights; returns the snapshot's id"""
+        if actor_kernel.w is None or actor_kernel.critic:
+            raise L.SatError("the pool takes loaded actor kernels")
+        if actor_kernel.use_tanh != self.use_tanh or actor_kernel.max_action != self.max_action:
+            raise L.SatError("the actor's activation / max_action differ from the pool's")
+        L.guard_device(self.device)
+        s = self._snaps.pop(0) if len(self._snaps) == self.capacity else self._alloc()
+        s["packed"].copy_(actor_kernel.packed)
+        self._build(s)
+        s["id"] = self._next_id
+        self._next_id += 1
+        self._snaps.append(s)
+        return s["id"]
+
+    def _alloc(self):
+        torch = self.torch
+        f32 = dict(dtype=torch.float32, device=self.device)
+        s = {"packed": torch.empty(L.ACTOR_PACKED_FLOATS, **f32), "image": torch.empty(L.ACTOR_TC_IMAGE_FLOATS, **f32),
+             "tables": torch.empty(L.ACTOR_TC_TABLE_FLOATS, **f32)}
+        # the snapshot as a GaussianActorKernel (FFMA2 path and references): its own image scratch, so sample(tc=True)
+        # never writes into the frozen image
+        k = GaussianActorKernel(self.max_action, bool(self.use_tanh), self.device)
+        k.packed = s["packed"]
+        k.w = L.SatActorWeights(None, None, None, None, None, None, None, s["packed"].data_ptr(), OBS_DIM, 256, ACT_DIM,
+                                self.use_tanh, self.max_action)
+        s["kernel"] = k
+        return s
+
+    def _build(self, s):
+        g = L.SatActorPoolGroup()
+        L.check(self.lib.sat_actor_tc_snapshot(C.byref(s["kernel"].w), s["image"].data_ptr(), s["tables"].data_ptr(),
+                                               C.byref(g), L.stream_ptr()), "sat_actor_tc_snapshot")
+        s["group"] = g
+
+    def group(self, slot: int):
+        """the SatActorPoolGroup of slot `slot` (row_end 0)"""
+        return self._snaps[slot]["group"]
+
+    def kernel(self, slot: int) -> GaussianActorKernel:
+        """the snapshot in slot `slot` as an actor kernel (do not train it)"""
+        return self._snaps[slot]["kernel"]
+
+    def state_dict(self):
+        """packed weights and ids; the images and tables are rebuilt on load"""
+        return {"capacity": self.capacity, "use_tanh": self.use_tanh, "max_action": self.max_action,
+                "next_id": self._next_id, "ids": self.ids, "packed": [s["packed"].clone() for s in self._snaps]}
+
+    def load_state_dict(self, sd):
+        if int(sd["use_tanh"]) != self.use_tanh or float(sd["max_action"]) != self.max_action:
+            raise L.SatError("the saved pool's activation / max_action differ from this pool's")
+        if len(sd["packed"]) > self.capacity:
+            raise L.SatError(f"the saved pool holds {len(sd['packed'])} snapshots, more than this pool's capacity {self.capacity}")
+        L.guard_device(self.device)
+        snaps = self._snaps
+        self._snaps = []
+        for i, (sid, packed) in enumerate(zip(sd["ids"], sd["packed"])):
+            s = snaps[i] if i < len(snaps) else self._alloc()
+            s["packed"].copy_(packed)
+            self._build(s)
+            s["id"] = int(sid)
+            self._snaps.append(s)
+        self._next_id = int(sd["next_id"])
+        return self
 
 
 # --------------------------------------------------------------------------------------------- fused PPO step

@@ -6,9 +6,39 @@ advantage normalisation with all-reduced moments, then the K-epoch minibatch upd
 or the PyTorch step, + NCCL gradient all-reduce). Envs shard across ranks with no traffic during the rollout (SURVEY.md s8e)."""
 from __future__ import annotations
 
+import numpy as np
 import torch
 
 from . import engine as eng
+
+POOL_TILE = 128            # rows per tile of the pool launch: every group bound but the last is a multiple of it
+
+
+def pool_group_bounds(n_total: int, groups: int):
+    """exclusive ends of `groups` contiguous groups over n_total global rows: 128 floor(tiles k / groups) for k = 1 ..
+    groups with tiles = ceil(n_total / 128), the last = n_total (a group may be empty when there are fewer tiles than
+    groups)"""
+    tiles = -(-int(n_total) // POOL_TILE)
+    ends = [min(POOL_TILE * (tiles * k // groups), int(n_total)) for k in range(1, groups + 1)]
+    ends[-1] = int(n_total)
+    return ends
+
+
+def shard_groups(ends, lo: int, hi: int):
+    """the groups (global bounds `ends`) that hold rows of the shard [lo, hi): [(group index, group end in shard rows)]"""
+    out, start = [], 0
+    for k, e in enumerate(ends):
+        a, b = max(start, lo), min(e, hi)
+        if b > a:
+            out.append((k, b - lo))
+        start = e
+    return out
+
+
+def pool_permutation(seed: int, collect_index: int, size: int):
+    """which pool slot plays group k: a permutation drawn from (seed, collect index) only, the same on every rank"""
+    rng = np.random.default_rng([int(seed) & (2 ** 64 - 1), int(collect_index)])
+    return [int(v) for v in rng.permutation(size)]
 
 
 class RolloutBuffer:
@@ -43,10 +73,21 @@ class VectorTrainer:
     RunningStats.update_normalize with group). Every rank then holds the same statistics, those of the union batch, bit
     for bit when every rank but the last holds a multiple of 128 envs (the initial observations are folded in blocks of
     128 rows, the steps in blocks of 64) and the env batches key their starts by global env index (row_offset). Collective: every rank of the group builds its trainer
-    with the same stats_group. None: each rank's statistics see its own shard only."""
+    with the same stats_group. None: each rank's statistics see its own shard only.
+
+    opponent_pool (engine.OpponentPool, default None): the learner plays past snapshots of the opponent instead of its
+    current weights. Every collect() splits the global rows (world shards of env.n) into len(pool) groups with
+    pool_group_bounds, gives group k the snapshot in slot pool_permutation(seed, collect index)[k] and samples this
+    shard's groups in the learner's launch (sample_vs_pool); it then sets opponent_stats, per group of the shard: the
+    snapshot id, the rows, the learner's mean reward and the episodes finished. With world > 1 every shard must start on a
+    128-row boundary. None: the opponent's current weights on every row (sample_pair)."""
 
     def __init__(self, env: eng.EnvBatch, agent, opponent, T: int, use_state_norm=True, use_reward_scaling=True,
-                 rank: int = 0, seed: int = 0, strict_errors: bool = False, stats_group=None):
+                 rank: int = 0, seed: int = 0, strict_errors: bool = False, stats_group=None, opponent_pool=None,
+                 world: int = 1):
+        if opponent_pool is not None and int(world) > 1 and (rank * env.n) % POOL_TILE:
+            raise eng.L.SatError(f"an opponent pool over {world} shards needs every shard to start on a {POOL_TILE}-row "
+                                 f"boundary (row offset {rank * env.n})")
         self.env, self.agent, self.opponent, self.T = env, agent, opponent, T
         self.strict_errors = strict_errors
         self.buf = RolloutBuffer(T, env.n, env.device)
@@ -55,6 +96,7 @@ class VectorTrainer:
         self.row_offset = rank * env.n            # the global row id of env 0 only when every shard holds env.n envs
         self.seed = seed
         self.t_global = 0
+        self.world, self.opponent_pool, self.collects, self.opponent_stats = int(world), opponent_pool, 0, None
         self.explained_variance = None
         if stats_group is not None:
             env.share_stats(stats_group)
@@ -68,17 +110,39 @@ class VectorTrainer:
             self.agent.sync_kernels()
         if self.opponent._dirty:
             self.opponent.sync_kernels()
+        pool = self.opponent_pool
+        if pool is not None:
+            if len(pool) == 0:
+                raise eng.L.SatError("the opponent pool is empty")
+            local = shard_groups(pool_group_bounds(self.world * env.n, len(pool)), self.row_offset, self.row_offset + env.n)
+            perm = pool_permutation(self.seed, self.collects, len(pool))
+            slots, ends = [perm[k] for k, _ in local], [e for _, e in local]
         for t in range(self.T):
             g = self.t_global
             # learner and opponent act on the same observation (CPPO_main.py:122-123): one launch for both networks
-            self.agent.actor_kernel.sample_pair(self.opponent.actor_kernel, env=env, obs_stats=self.obs_stats, seed=self.seed,
-                                                step=2 * g, other_step=2 * g + 1, row_offset=self.row_offset, act=buf.act[t],
-                                                logp=buf.logp[t], obs_out=buf.obs[t], other_act=buf.opp_act[t],
-                                                other_logp=buf.opp_logp[t])
+            if pool is None:
+                self.agent.actor_kernel.sample_pair(self.opponent.actor_kernel, env=env, obs_stats=self.obs_stats,
+                                                    seed=self.seed, step=2 * g, other_step=2 * g + 1, row_offset=self.row_offset,
+                                                    act=buf.act[t], logp=buf.logp[t], obs_out=buf.obs[t],
+                                                    other_act=buf.opp_act[t], other_logp=buf.opp_logp[t])
+            else:
+                self.agent.actor_kernel.sample_vs_pool(pool, slots, ends, env=env, obs_stats=self.obs_stats, seed=self.seed,
+                                                       step=2 * g, other_step=2 * g + 1, row_offset=self.row_offset,
+                                                       act=buf.act[t], logp=buf.logp[t], obs_out=buf.obs[t],
+                                                       other_act=buf.opp_act[t], other_logp=buf.opp_logp[t])
             pa, ea = (buf.act[t], buf.opp_act[t]) if self.learner_is_pursuer else (buf.opp_act[t], buf.act[t])
             env.step(pa, ea, reward=buf.rew64[t], done=buf.done[t], obs_stats=self.obs_stats, ret_stats=self.ret_stats,
                      ret_std_out=buf.ret_std[t:t + 1] if self.ret_stats is not None else None)
             self.t_global += 1
+        self.collects += 1
+        if pool is not None:
+            # per group: the learner's reward summed over the rollout and the episodes finished, summed over the group's
+            # contiguous rows (no atomics: the same bits on every run), one copy to the host
+            per_row = torch.stack([buf.rew64.sum(0), buf.done.sum(0, dtype=torch.float64)])
+            rew, eps = torch.stack([per_row[:, lo:e].sum(1) for lo, e in zip([0] + ends, ends)], 1).tolist()
+            rows = np.diff([0] + ends)
+            self.opponent_stats = [{"snapshot_id": pool.ids[s], "rows": int(r), "mean_reward": rw / (int(r) * self.T),
+                                    "episodes_finished": int(ep)} for s, r, rw, ep in zip(slots, rows, rew, eps)]
         # The reference raises where an element set is circular / parabolic (satellite_function.py:40-42 via :52-58); the
         # kernel flags the env (err = 1, dz = 0) and goes on. One reduced flag per collect() makes that visible.
         n_err = int(env.err.sum().item())
@@ -148,7 +212,8 @@ class VectorTrainer:
                 "actor": ag.actor.state_dict(), "critic": ag.critic.state_dict(),
                 "opt_actor": ag.optimizer_actor.state_dict(), "opt_critic": ag.optimizer_critic.state_dict(),
                 "fused_adam": [n.state_dict() for n in ag._fused["nets"]] if ag._fused is not None else None,
-                "opponent_actor": self.opponent.actor.state_dict()}
+                "opponent_actor": self.opponent.actor.state_dict(), "collects": self.collects,
+                "opponent_pool": self.opponent_pool.state_dict() if self.opponent_pool is not None else None}
 
     def load_state_dict(self, sd):
         ag = self.agent
@@ -161,6 +226,9 @@ class VectorTrainer:
         ag.actor.load_state_dict(sd["actor"]); ag.critic.load_state_dict(sd["critic"])
         ag.optimizer_actor.load_state_dict(sd["opt_actor"]); ag.optimizer_critic.load_state_dict(sd["opt_critic"])
         self.opponent.actor.load_state_dict(sd["opponent_actor"])
+        self.collects = int(sd.get("collects", 0))
+        if self.opponent_pool is not None and sd.get("opponent_pool") is not None:
+            self.opponent_pool.load_state_dict(sd["opponent_pool"])
         if sd.get("fused_adam") is not None:
             for n, st in zip(ag._fused_for(1)["nets"], sd["fused_adam"]):
                 n.load_state_dict(st)
@@ -172,12 +240,28 @@ class SelfPlay:
     """Alternating pursuer / evader training on one device-resident env batch: the batched counterpart of CPPO_main.py's
     `Sign == 0` branch (train_pursuer_network with reset(0), :94-161, then train_evader_network with reset(1), :163-230).
     The upstream evader trainer updates the *pursuer* agent with the evader's buffer (CPPO_main.py:215); here the evader
-    learns from its own rollouts, which is the evident intent."""
+    learns from its own rollouts, which is the evident intent.
 
-    def __init__(self, env: eng.EnvBatch, pursuer, evader, T: int, mini_batch_size: int, rank: int = 0, seed: int = 0, **kw):
+    opponent_pool=P: each role keeps a pool of up to P snapshots of its actor (engine.OpponentPool), seeded with its initial
+    actor; the end of a phase adds the learner's actor to its role's pool, and each trainer plays the other role's pool
+    (VectorTrainer opponent_pool), so a learner faces a mixture of the opponent's past snapshots. Each record then carries
+    "opponents": the trainer's opponent_stats."""
+
+    def __init__(self, env: eng.EnvBatch, pursuer, evader, T: int, mini_batch_size: int, rank: int = 0, seed: int = 0,
+                 opponent_pool: int | None = None, **kw):
         self.env, self.mb = env, mini_batch_size
-        self.trainers = {0: VectorTrainer(env, pursuer, evader, T, rank=rank, seed=seed, **kw),
-                         1: VectorTrainer(env, evader, pursuer, T, rank=rank, seed=seed + 1, **kw)}
+        self.pools = None
+        if opponent_pool:
+            self.pools = {}
+            for flag, ag in ((0, pursuer), (1, evader)):
+                if ag._dirty:
+                    ag.sync_kernels()
+                k = ag.actor_kernel
+                self.pools[flag] = eng.OpponentPool(int(opponent_pool), bool(k.use_tanh), k.max_action, k.device)
+                self.pools[flag].add(k)
+        p0, p1 = (self.pools[0], self.pools[1]) if self.pools else (None, None)
+        self.trainers = {0: VectorTrainer(env, pursuer, evader, T, rank=rank, seed=seed, opponent_pool=p1, **kw),
+                         1: VectorTrainer(env, evader, pursuer, T, rank=rank, seed=seed + 1, opponent_pool=p0, **kw)}
 
     def run_phase(self, flag: int, iterations: int, group=None, use_graph: bool = True, fused: bool = True, callback=None,
                   stats: bool = False):
@@ -193,9 +277,15 @@ class SelfPlay:
                       "episodes_finished": int(tr.buf.done.sum())}
             upd = tr.update(self.mb, total_steps=it, group=group, use_graph=use_graph, fused=fused, stats=stats)
             record = dict(record, **upd.as_dict()) if stats else record
+            if tr.opponent_pool is not None:
+                record["opponents"] = tr.opponent_stats
             out.append(record)
             if callback is not None:
                 callback(record)
+        if self.pools:
+            if tr.agent._dirty:
+                tr.agent.sync_kernels()
+            self.pools[flag].add(tr.agent.actor_kernel)          # the other role's trainer draws from this pool
         return out
 
     def run(self, rounds: int, iterations_per_phase: int, **kw):

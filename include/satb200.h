@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define SATB200_ABI_VERSION 2
+#define SATB200_ABI_VERSION 3
 
 #define SAT_OK          0
 #define SAT_ERR_NULL   -1   /* required pointer is NULL */
@@ -328,15 +328,17 @@ int sat_actor_sample_pair(const SatActorWeights* wa, const SatActorWeights* wb, 
  * K4  GAE reverse scan. Replaces the block at ppo_continuous.py:198-210.
  * time-major form: r, done [T][N]; v [T+1][N] with v[t+1] = V(s') of step t (dw == done, SURVEY Q8);
  * r_scale nullable [T]: per-step reward scale (1/(std_R+1e-8)) applied on the fly.
+ * gamma, lamda are the reference's python floats: the recursion coefficient is their double product rounded to fp32
+ * (gamma*lamda*gae under numpy 2), the delta uses gamma rounded to fp32 (torch's fp32 tensor times a python float).
  * flat form: the reference's (B,1) buffers of one env in time order, with separate vs_next and dw.
  * Outputs adv / v_target share the input layout. sat_adv_normalize applies
  * (adv - mean)/(std_unbiased + 1e-5) (ppo_continuous.py:210); sums[3] (nullable in/out) lets the caller
  * all-reduce (sum, sum of squares, count) across ranks between the two phases.
  * ------------------------------------------------------------------------------------------------ */
 int sat_gae(const float* r, const float* v, const uint8_t* done, const float* r_scale, int64_t T, int64_t N,
-            float gamma, float lamda, float* adv, float* v_target, void* stream);
+            double gamma, double lamda, float* adv, float* v_target, void* stream);
 int sat_gae_flat(const float* r, const float* vs, const float* vs_next, const float* dw, const float* done,
-                 int64_t B, float gamma, float lamda, float* adv, float* v_target, void* stream);
+                 int64_t B, double gamma, double lamda, float* adv, float* v_target, void* stream);
 int sat_adv_moments(const float* adv, int64_t count, double* sums /*[3] device*/, void* workspace, void* stream);
 int sat_adv_normalize(float* adv, int64_t count, const double* sums /*[3] device*/, void* stream);
 

@@ -79,7 +79,7 @@ def lib():
         L.orc_env_step_rk4_batch.argtypes = [C.POINTER(OrcEnv), C.POINTER(C.c_int32), i64, C.c_double, i32,
                                              C.c_double, C.c_double, C.c_double, dp, dp, dp, dp,
                                              C.POINTER(C.c_uint8), i32, i32]
-        L.orc_gae.argtypes = [fp, fp, fp, fp, fp, i64, C.c_float, C.c_float, fp, fp]
+        L.orc_gae.argtypes = [fp, fp, fp, fp, fp, i64, C.c_double, C.c_double, fp, fp]
         L.orc_adv_normalize.argtypes = [fp, i64]
         L.orc_actor_forward.argtypes = [fp] * 6 + [i32, i32, i32, C.c_float, fp, i64, fp]
         L.orc_critic_forward.argtypes = [fp] * 6 + [i32, i32, fp, i64, fp]

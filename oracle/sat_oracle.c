@@ -624,14 +624,16 @@ double orc_reward_scaling(orc_rms* r, double* R, double gamma, double x) {   /* 
 /* ------------------------------------------------------------------------------------------
  * GAE, ppo_continuous.py:198-210. Under numpy 2 (NEP 50) the recursion runs in float32:
  * delta and d are np.float32, gamma*lamda is a python float (weak) -> float32 arithmetic.
+ * gamma and lamda are the python floats: their product is formed in double and rounded once.
  * ------------------------------------------------------------------------------------------ */
 void orc_gae(const float* r, const float* vs, const float* vs_next, const float* dw, const float* done,
-             int64_t B, float gamma, float lamda, float* adv, float* v_target) {
+             int64_t B, double gamma, double lamda, float* adv, float* v_target) {
     int64_t t;
     float gae = 0.0f;
-    float gl = (float)((double)gamma * (double)lamda);      /* python float product, then weak-cast */
+    const float gl = (float)(gamma * lamda);                 /* python float product, then weak-cast */
+    const float g32 = (float)gamma;                          /* torch rounds the scalar to the tensor's fp32 */
     for (t = B - 1; t >= 0; --t) {
-        float delta = r[t] + gamma * (1.0f - dw[t]) * vs_next[t] - vs[t];               /* :203 (torch fp32) */
+        float delta = r[t] + g32 * (1.0f - dw[t]) * vs_next[t] - vs[t];                 /* :203 (torch fp32) */
         gae = delta + gl * gae * (1.0f - done[t]);                                      /* :205 */
         adv[t] = gae;                                                                   /* :206 */
         v_target[t] = gae + vs[t];                                                      /* :208 */

@@ -110,7 +110,7 @@ double orc_reward_scaling(orc_rms* r, double* R, double gamma, double x);  /* :5
 
 /* ---- GAE (ppo_continuous.py:198-210); fp32 recursion as executed under numpy 2 ---- */
 void orc_gae(const float* r, const float* vs, const float* vs_next, const float* dw, const float* done,
-             int64_t B, float gamma, float lamda, float* adv, float* v_target);
+             int64_t B, double gamma, double lamda, float* adv, float* v_target);
 void orc_adv_normalize(float* adv, int64_t B); /* (adv-mean)/(std_unbiased+1e-5), torch semantics */
 
 /* ---- Gaussian actor (ppo_continuous.py:83-95, 176-189), fp32 ---- */

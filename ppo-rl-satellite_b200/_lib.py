@@ -12,6 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libsatb200.so")
 
+ABI_VERSION = 3                   # SATB200_ABI_VERSION of the header this binding mirrors
 SAT_STATE_COLS = 16
 SAT_ISTATE_COLS = 4
 COL_P, COL_PV, COL_E, COL_EV, COL_FUEL_C, COL_FUEL_T, COL_DIS, COL_RET = 0, 3, 6, 9, 12, 13, 14, 15
@@ -141,8 +142,8 @@ SIGNATURES = {
                                            C.POINTER(SatEnvState), _P, _I64, _I64, _U64, _U64, _U64, _P, _P, _P, _P, _P, _P]),
     "sat_critic_forward": (C.c_int, [C.POINTER(SatActorWeights), _P, _I64, _P, _P]),
     "sat_actor_sample_pair": (C.c_int, [_P, _P, _P, _P, _P, _I64, _I64, _U64, _U64, _U64, _P, _P, _P, _P, _P, _P]),
-    "sat_gae": (C.c_int, [_P, _P, _P, _P, _I64, _I64, _F, _F, _P, _P, _P]),
-    "sat_gae_flat": (C.c_int, [_P, _P, _P, _P, _P, _I64, _F, _F, _P, _P, _P]),
+    "sat_gae": (C.c_int, [_P, _P, _P, _P, _I64, _I64, _D, _D, _P, _P, _P]),
+    "sat_gae_flat": (C.c_int, [_P, _P, _P, _P, _P, _I64, _D, _D, _P, _P, _P]),
     "sat_adv_moments": (C.c_int, [_P, _I64, _P, _P, _P]),
     "sat_adv_normalize": (C.c_int, [_P, _I64, _P, _P]),
     "sat_peak_fp64": (C.c_int, [_P, _I32, _I32, _I32, C.POINTER(C.c_double), _P]),
@@ -169,8 +170,8 @@ def load():
             fn = getattr(lib, name)     # AttributeError if the .so does not export a declared symbol
             fn.restype = res
             fn.argtypes = args
-        if lib.sat_abi_version() != 2:
-            raise ImportError("libsatb200.so ABI version mismatch")
+        if lib.sat_abi_version() != ABI_VERSION:
+            raise ImportError(f"libsatb200.so ABI version {lib.sat_abi_version()}, this binding expects {ABI_VERSION}: rebuild it")
         _lib = lib
     return _lib
 

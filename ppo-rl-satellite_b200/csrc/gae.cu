@@ -262,23 +262,25 @@ constexpr int kMomBlocks = 148 * 8;   // 8 per SM
 extern "C" {
 
 int sat_gae(const float* r, const float* v, const uint8_t* done, const float* r_scale, int64_t T, int64_t N,
-            float gamma, float lamda, float* adv, float* v_target, void* stream) {
+            double gamma, double lamda, float* adv, float* v_target, void* stream) {
     if (!r || !v || !done || !adv || !v_target) return SAT_ERR_NULL;
     if (T <= 0 || N <= 0) return SAT_ERR_SIZE;
-    const float gl = (float)((double)gamma * (double)lamda);   // python float product, weak-cast to fp32
+    // :205 multiplies the python floats first and weak-casts the double product to fp32; :203 multiplies an fp32 tensor
+    // by gamma, which torch rounds to fp32 first
+    const float gl = (float)(gamma * lamda), g32 = (float)gamma;
     // at least ~6 CTAs per SM (148 SMs) where the env count allows it
-    if (N >= 32 * 888) gae_time_major_kernel<32><<<(unsigned)((N + 31) / 32), kGaeThreads, 0, (cudaStream_t)stream>>>(r, v, done, r_scale, T, N, gamma, gl, adv, v_target);
-    else if (N >= 16 * 296) gae_time_major_kernel<16><<<(unsigned)((N + 15) / 16), kGaeThreads, 0, (cudaStream_t)stream>>>(r, v, done, r_scale, T, N, gamma, gl, adv, v_target);
-    else gae_time_major_kernel<8><<<(unsigned)((N + 7) / 8), kGaeThreads, 0, (cudaStream_t)stream>>>(r, v, done, r_scale, T, N, gamma, gl, adv, v_target);
+    if (N >= 32 * 888) gae_time_major_kernel<32><<<(unsigned)((N + 31) / 32), kGaeThreads, 0, (cudaStream_t)stream>>>(r, v, done, r_scale, T, N, g32, gl, adv, v_target);
+    else if (N >= 16 * 296) gae_time_major_kernel<16><<<(unsigned)((N + 15) / 16), kGaeThreads, 0, (cudaStream_t)stream>>>(r, v, done, r_scale, T, N, g32, gl, adv, v_target);
+    else gae_time_major_kernel<8><<<(unsigned)((N + 7) / 8), kGaeThreads, 0, (cudaStream_t)stream>>>(r, v, done, r_scale, T, N, g32, gl, adv, v_target);
     return launch_status();
 }
 
 int sat_gae_flat(const float* r, const float* vs, const float* vs_next, const float* dw, const float* done,
-                 int64_t B, float gamma, float lamda, float* adv, float* v_target, void* stream) {
+                 int64_t B, double gamma, double lamda, float* adv, float* v_target, void* stream) {
     if (!r || !vs || !vs_next || !dw || !done || !adv || !v_target) return SAT_ERR_NULL;
     if (B <= 0) return SAT_ERR_SIZE;
-    const float gl = (float)((double)gamma * (double)lamda);
-    gae_flat_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(r, vs, vs_next, dw, done, B, gamma, gl, adv, v_target);
+    const float gl = (float)(gamma * lamda), g32 = (float)gamma;          // as in sat_gae
+    gae_flat_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(r, vs, vs_next, dw, done, B, g32, gl, adv, v_target);
     return launch_status();
 }
 

@@ -776,11 +776,19 @@ class GaussianActorKernel:
         return act, logp, other_act, other_logp
 
     def value(self, obs, out=None):
+        """V(s) for obs [n, 18] fp32 into out [n] fp32 (new if None), both on this kernel's device."""
         torch = self.torch
         if not self.critic:
             raise L.SatError("not a critic kernel")
+        if obs.dim() != 2 or obs.shape[1] != 18 or obs.dtype != torch.float32:
+            raise L.SatError(f"obs must be [n, 18] fp32, got {list(obs.shape)} {obs.dtype}")
         n = obs.shape[0]
         out = torch.empty(n, dtype=torch.float32, device=self.device) if out is None else out
+        if tuple(out.shape) != (n,) or out.dtype != torch.float32:
+            raise L.SatError(f"out must be [{n}] fp32, got {list(out.shape)} {out.dtype}")
+        if (obs.device != out.device or obs.device.type != "cuda"
+                or self.device.index is not None and obs.device.index != self.device.index):
+            raise L.SatError(f"obs and out must be on {self.device}, got {obs.device} and {out.device}")
         L.check(self.lib.sat_critic_forward(C.byref(self.w), L.ptr(obs), n, L.ptr(out), L.stream_ptr()),
                 "sat_critic_forward")
         return out
@@ -1038,11 +1046,26 @@ def ppo_workspace(mb: int, device):
 
 # --------------------------------------------------------------------------------------------- K4
 def gae_time_major(r, v, done, gamma=0.99, lamda=0.95, r_scale=None, adv=None, v_target=None):
-    """r [T,N] fp32, v [T+1,N] fp32, done [T,N] uint8 (CUDA). ppo_continuous.py:198-208 per env column."""
+    """r [T,N] fp32, v [T+1,N] fp32, done [T,N] uint8 or bool, r_scale [T] fp32 or None, adv / v_target [T,N] fp32 or
+    None (new), all on one CUDA device. ppo_continuous.py:198-208 per env column; gamma and lamda are taken as python
+    floats, as the reference holds them."""
     torch = L.require_cuda()
+    if r.dim() != 2:
+        raise L.SatError(f"r must be [T, N], got {list(r.shape)}")
     T, N = r.shape
     adv = torch.empty_like(r) if adv is None else adv
     v_target = torch.empty_like(r) if v_target is None else v_target
+    want = {"r": (r, (T, N)), "v": (v, (T + 1, N)), "adv": (adv, (T, N)), "v_target": (v_target, (T, N))}
+    if r_scale is not None:
+        want["r_scale"] = (r_scale, (T,))
+    for name, (t, shape) in want.items():
+        if tuple(t.shape) != shape or t.dtype != torch.float32:
+            raise L.SatError(f"{name} must be {list(shape)} fp32, got {list(t.shape)} {t.dtype}")
+    if tuple(done.shape) != (T, N) or done.dtype not in (torch.uint8, torch.bool):
+        raise L.SatError(f"done must be [{T}, {N}] uint8 or bool, got {list(done.shape)} {done.dtype}")
+    devs = {t.device for t in (r, v, done, adv, v_target) + ((r_scale,) if r_scale is not None else ())}
+    if len(devs) != 1 or r.device.type != "cuda":
+        raise L.SatError(f"every tensor must be on one CUDA device, got {sorted(map(str, devs))}")
     L.check(L.load().sat_gae(L.ptr(r), L.ptr(v), L.ptr(done), L.ptr(r_scale), T, N, float(gamma), float(lamda),
                              L.ptr(adv), L.ptr(v_target), L.stream_ptr()), "sat_gae")
     return adv, v_target

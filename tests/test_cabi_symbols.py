@@ -38,11 +38,19 @@ def test_header_symbols_are_exported(lib_path):
     assert not extra, f"exported but not declared: {extra}"
 
 
-def test_ctypes_binding_covers_header_and_checks_abi_version(lib_path):
+def header_abi_version():
+    m = re.search(r"^#define\s+SATB200_ABI_VERSION\s+(\d+)\s*$", open(HEADER, encoding="utf-8").read(), flags=re.M)
+    assert m, "SATB200_ABI_VERSION not found in satb200.h"
+    return int(m.group(1))
+
+
+def test_ctypes_binding_covers_header_and_matches_header_abi_version(lib_path):
+    """the binding declares every header symbol, and the header, the library and the binding agree on the ABI version
+    (the version changes with any signature change, e.g. 3: sat_gae / sat_gae_flat take double gamma, lamda)"""
     from ppo_rl_satellite_b200 import _lib
     assert sorted(_lib.SIGNATURES) == declared_symbols()
     lib = _lib.load()                      # dlopen + symbol lookup, no compute
-    assert lib.sat_abi_version() == 2
+    assert lib.sat_abi_version() == header_abi_version() == _lib.ABI_VERSION >= 3
     assert lib.sat_strerror(0) == b"ok" and b"NULL" in lib.sat_strerror(-1)
     assert lib.sat_workspace_bytes(65536) >= 65536 // 32 * 19 * 16
     p = _lib.default_params()
